@@ -540,6 +540,8 @@ def run_gpu(args):
     ms_total = t0.elapsed_time(t1)
     sweep_kernel_ms = float(np.mean([a.elapsed_time(b) for a, b in sweep_evs]))
     resident_counts = o.read_counters(host_cnt)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pkg, torch, frames, power, host_cnt)
 
     # the HBM-bound kernel of the path, one SNR point per launch (stage API): steps x 21 launches, events around each
     # (after one second of idle: the first sweep of the loop then shows the kernel at full clocks, the mean over the whole loop
@@ -661,6 +663,26 @@ def run_gpu(args):
     return 0
 
 
+DUMP_SAMPLE_FRAMES = 8192
+
+
+def dump_outputs(out_dir, pkg, torch, frames, power, counters):
+    """Write what the last timed step returned to its caller, so that two builds can be compared output for output:
+    counters.npy (one row per SNR point, columns as ofdm_counters, float64: the integer totals stay exact) and, for a
+    fixed, seeded sample of frames, the TX IQ and frame power (sample_*.npy; about 21 MB at any frame count)."""
+    os.makedirs(out_dir, exist_ok=True)
+    n_frames = frames.shape[0]
+    idx = np.sort(np.random.default_rng(0).choice(n_frames, min(DUMP_SAMPLE_FRAMES, n_frames), replace=False))
+    sel = torch.from_numpy(idx).to(frames.device)
+    raw = counters.cpu().numpy()
+    n_int = pkg.sweep.N_INT_FIELDS
+    cnt = np.concatenate([raw[:, :n_int].astype(np.float64), raw[:, n_int:].copy().view(np.float64)], axis=1)
+    arrays = {"counters": cnt, "sample_frame_index": idx.astype(np.float64),
+              "sample_tx_frames": frames.index_select(0, sel).cpu().numpy(), "sample_tx_power": power.index_select(0, sel).cpu().numpy()}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def emit(line):
     """print the one JSON line on the real stdout (libraries such as NCCL may write to fd 1 meanwhile)"""
     os.write(_REAL_STDOUT, (json.dumps(line) + "\n").encode())
@@ -687,7 +709,12 @@ def main():
     ap.add_argument("--mc-frames", type=int, default=2_000_000, help="frames per GPU of the configs[3] / configs[4] Monte-Carlo sweeps")
     ap.add_argument("--until-round-frames", type=int, default=1 << 20, help="frames per round and GPU of the until-rule sweep")
     ap.add_argument("--no-configs", action="store_true", help="skip configs[2] / [3] / [4] (A/B runs of the headline only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 path")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)

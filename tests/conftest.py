@@ -57,8 +57,11 @@ def ofdm(pkg, lib):
 
 @pytest.fixture(scope="session")
 def golden():
-    path = os.path.join(ROOT, "tests", "golden", "stage_vectors.npz")
-    return np.load(path)
+    out = {}
+    for name in ("stage_vectors.npz", "chain_totals.npz"):
+        with np.load(os.path.join(ROOT, "tests", "golden", name)) as z:
+            out.update({k: z[k] for k in z.files})
+    return out
 
 
 def bits_and_noise(seed, n_frames, n_sym):

@@ -1,13 +1,14 @@
-"""Generates tests/golden/stage_vectors.npz from the COMPILED, UNMODIFIED reference
-(oracle/_ref/libofdm_ref.so, built from /root/reference/src/OFDM.c by oracle/Makefile).
-Run in the build container (the reference tree is not on the GPU box):
+"""Generates tests/golden/stage_vectors.npz and tests/golden/chain_totals.npz from the COMPILED, UNMODIFIED
+reference (oracle/_ref/libofdm_ref.so, built by oracle/Makefile from $REF_ROOT/src/OFDM.c, REF_ROOT being a
+checkout of the original simulator):
 
-    python tests/golden/make_golden.py
+    REF_ROOT=<checkout of the original> python tests/golden/make_golden.py
 
 Contents: per-stage vectors of the reference stage chain for a few frames (bits, QPSK points, grid,
 TX IQ, the noise draw g_keep captured from the reference's rand()/Box-Muller stream, OTA IQ, H_est,
 equalised points, slicer output, demodulated bits, per-frame EVM / bit errors) at several SNRs and
-two frame lengths, plus whole-chain totals for a 256-frame batch per SNR.
+two frame lengths; in chain_totals.npz, whole-chain totals for a 256-frame batch per SNR.  Two files keep
+each well under 1 MB.
 """
 import os
 import sys
@@ -20,7 +21,10 @@ import pyoracle as po  # noqa: E402
 
 
 def main():
-    po.build()
+    ref_root = os.environ.get("REF_ROOT")
+    if not ref_root or not os.path.isfile(os.path.join(ref_root, "src", "OFDM.c")):
+        raise SystemExit("set REF_ROOT to a checkout of the original simulator (it must contain src/OFDM.c)")
+    po.build(force=True)                # oracle/Makefile takes REF_ROOT from the environment
     ref = po.Ref()
     out = {}
     out["lts_freq"] = ref.lts_freq()
@@ -36,12 +40,11 @@ def main():
         bits = rng.integers(0, 2, (n_frames, 96 * n_sym), dtype=np.uint8)
         # frame 0 of the n_sym=2 set carries the reference repo's own golden bits (data/Matlab_Output.txt) as symbol 0
         if n_sym == 2:
-            mo = os.path.join("/root/reference", "data", "Matlab_Output.txt")
-            if os.path.exists(mo):
-                b96 = np.array(open(mo).read().split(), dtype=np.float64).astype(np.uint8)
-                assert b96.size == 96
-                bits[0, :96] = b96
-                out["matlab_output_bits"] = b96
+            mo = os.path.join(ref_root, "data", "Matlab_Output.txt")
+            b96 = np.array(open(mo).read().split(), dtype=np.float64).astype(np.uint8)
+            assert b96.size == 96
+            bits[0, :96] = b96
+            out["matlab_output_bits"] = b96
         out[tag + "bits"] = bits
         mod = ref.qpsk_mod(bits)
         out[tag + "mod"] = mod
@@ -78,9 +81,11 @@ def main():
         a = ref.chain(bits, g, n_sym, float(s))
         tot.append([a.bit_errors, a.bits, a.frames_in_error, a.rail_errors, a.frames, a.sum_err2, a.sum_ref2, a.sum_evm_lin])
     out["chain_totals"] = np.array(tot, np.float64)
-    path = os.path.join(ROOT, "tests", "golden", "stage_vectors.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, os.path.getsize(path), "bytes,", len(out), "arrays")
+    chain = {k: out.pop(k) for k in [k for k in out if k.startswith("chain_")]}
+    for name, arrays in (("stage_vectors.npz", out), ("chain_totals.npz", chain)):
+        path = os.path.join(ROOT, "tests", "golden", name)
+        np.savez_compressed(path, **arrays)
+        print("wrote", path, os.path.getsize(path), "bytes,", len(arrays), "arrays")
 
 
 if __name__ == "__main__":

@@ -13,7 +13,8 @@ import pytest
 
 from conftest import ROOT
 
-REF_SCRIPTS = "/root/reference/scripts"
+REF_ROOT = os.environ.get("REF_ROOT", "")          # a checkout of the original simulator, as for oracle/Makefile
+REF_SCRIPTS = os.path.join(REF_ROOT, "scripts")
 
 
 def declared_symbols():
@@ -77,7 +78,7 @@ def test_writers_match_reference_writers(pkg, lib, ref, tmp_path):
     assert open(tmp_path / "rc.txt").read() == open(tmp_path / "mc.txt").read()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SCRIPTS), reason="reference scripts not present on this box")
+@pytest.mark.skipif(not REF_ROOT or not os.path.isdir(REF_SCRIPTS), reason="REF_ROOT (the original simulator's scripts) not set")
 def test_reference_scripts_consume_outputs_unchanged(pkg, lib, port, golden, tmp_path):
     # compare_double.py: demodulated bits of the golden payload, dumped in the live (real-part) format, vs data/Matlab_Output.txt
     b96 = golden["matlab_output_bits"]
@@ -86,7 +87,7 @@ def test_reference_scripts_consume_outputs_unchanged(pkg, lib, port, golden, tmp
     iq = np.stack([rx.astype(np.float32), np.zeros(96, np.float32)], axis=1)
     assert pkg.write_complex_array_to_file(lib, iq, str(tmp_path / "Code_Output.txt"), 0) == 0
     with open(tmp_path / "Matlab_Output.txt", "w") as f:
-        f.write(open("/root/reference/data/Matlab_Output.txt").read())
+        f.write(open(os.path.join(REF_ROOT, "data", "Matlab_Output.txt")).read())
     out = subprocess.run([sys.executable, os.path.join(REF_SCRIPTS, "compare_double.py")], cwd=tmp_path, capture_output=True, text=True)
     assert out.returncode == 0 and "Extracted 96 numbers" in out.stdout and "Max Error: 0.000000e+00" in out.stdout, out.stdout + out.stderr
     # compare_complex.py: IQ in the "re + imi" triple format on both sides
