@@ -45,6 +45,25 @@ class RxDump(C.Structure):
                 ("frame_bit_errors", C.c_void_p), ("frame_evm_lin", C.c_void_p)]
 
 
+class Channel(C.Structure):
+    """ofdm_channel"""
+    _fields_ = [("noise", C.c_int), ("snr_def", C.c_int), ("n_taps", C.c_int)]
+
+
+# ofdm_channel's enums under the names the Python methods take; ("real", "frame_power") is the reference's channel
+NOISE = {"real": 0, "complex": 1}
+SNR_DEF = {"frame_power": 0, "esn0": 1, "ebn0": 2}
+
+
+def channel(noise="real", snr_def="frame_power", n_taps=0):
+    """Channel from names: noise "real" | "complex", snr_def "frame_power" | "esn0" | "ebn0" (include/ofdm_b200.h)."""
+    if noise not in NOISE:
+        raise ValueError("noise must be one of %s, not %r" % (sorted(NOISE), noise))
+    if snr_def not in SNR_DEF:
+        raise ValueError("snr_def must be one of %s, not %r" % (sorted(SNR_DEF), snr_def))
+    return Channel(NOISE[noise], SNR_DEF[snr_def], int(n_taps))
+
+
 class OfdmError(RuntimeError):
     pass
 
@@ -84,6 +103,7 @@ SIGNATURES = {
     "ofdm_frame_power": (_I, [_VP, _VP, _VP, _L, _I, _I]),
     "ofdm_awgn_inject": (_I, [_VP, _VP, _VP, _VP, _F, _VP, _L, _I, _I]),
     "ofdm_awgn_philox": (_I, [_VP, _VP, _VP, _F, _U32, _U32, _U64, _VP, _L, _I, _I]),
+    "ofdm_awgn_philox_ex": (_I, [_VP, _I, _I, _VP, _VP, _F, _U32, _U32, _U64, _VP, _L, _I, _I]),
     "ofdm_rx_frames": (_I, [_VP, _VP, _VP, _L, _I, _I, _VP, C.POINTER(RxDump)]),
     "ofdm_awgn_rx_inject": (_I, [_VP, _VP, _VP, _VP, _VP, _F, _L, _I, _I, _VP, C.POINTER(RxDump)]),
     "ofdm_awgn_rx_philox": (_I, [_VP, _VP, _VP, _VP, _F, _U32, _U32, _U64, _L, _I, _I, _VP, C.POINTER(RxDump)]),
@@ -100,6 +120,9 @@ SIGNATURES = {
     "ofdm_mc_sweep_philox_dev": (_I, [_VP, _U32, _U64, _L, _I, _VP, _I, _I, _VP]),
     "ofdm_mc_sweep_points_dev": (_I, [_VP, _U32, _U64, _L, _I, _I, _VP, _VP, _I, _I, _VP]),
     "ofdm_mc_sweep_until": (_I, [_VP, _U32, _U64, _I, _I, _VP, _I, _I, _U64, _U64, _L, C.POINTER(Counters), C.POINTER(_I)]),
+    "ofdm_mc_sweep_channel_dev": (_I, [_VP, C.POINTER(Channel), _U32, _U64, _L, _I, _VP, _VP, _I, _I, _VP]),
+    "ofdm_mc_sweep_channel_until": (_I, [_VP, C.POINTER(Channel), _U32, _U64, _I, _VP, _I, _I, _U64, _U64, _L, C.POINTER(Counters),
+                                         C.POINTER(_I)]),
     "ofdm_mc_sweep_philox": (_I, [_VP, _U32, _U64, _L, _I, _VP, _I, _I, C.POINTER(Counters)]),
     "ofdm_multipath_taps": (_I, [_VP, _VP, _VP, _I, _VP, _L, _I]),
     "ofdm_multipath_philox": (_I, [_VP, _VP, _U32, _U64, _I, _VP, _VP, _L, _I]),
@@ -310,6 +333,14 @@ class Ofdm:
                                               n_frames, n_sym, mode))
         return ota
 
+    def awgn_philox_ex(self, tx, snr_db, seed, stream, frame0, n_sym, mode, noise="real", snr_def="frame_power", power=None):
+        """the channel (noise, snr_def) on LTS||data frames with on-chip draws; ("real", "frame_power") is awgn_philox"""
+        ch = channel(noise, snr_def)
+        ota = self.empty(tuple(tx.shape), self.torch.float32)
+        self._check(self.lib.ofdm_awgn_philox_ex(self.h, ch.noise, ch.snr_def, _ptr(tx), _ptr(power), snr_db, seed, stream, frame0,
+                                                 _ptr(ota), tx.shape[0], n_sym, mode))
+        return ota
+
     def rx_frames(self, ota, tx_packed, n_sym, mode, want=()):
         n_frames = ota.shape[0]
         cnt = self.new_counters()
@@ -430,6 +461,29 @@ class Ofdm:
         rounds = _I(0)
         self._check(self.lib.ofdm_mc_sweep_until(self.h, seed, frame0, n_sym, n_taps, snr.ctypes.data, len(snr), mode, target_errors, max_bits,
                                                  round_frames, out, C.byref(rounds)))
+        return list(out), int(rounds.value)
+
+    def mc_sweep_channel(self, seed, frame0, n_frames, n_sym, snr_db, mode, noise="real", snr_def="frame_power", n_taps=0, streams=None,
+                         counters=None):
+        """Monte-Carlo sweep through the channel (noise, snr_def, n_taps); ("real", "frame_power") is mc_sweep_points.
+        counters=None: returns host totals (synchronises); else accumulates into the device counters tensor."""
+        ch = channel(noise, snr_def, n_taps)
+        snr = np.ascontiguousarray(snr_db, dtype=np.float32)
+        st = None if streams is None else np.ascontiguousarray(streams, dtype=np.uint32)
+        cnt = counters if counters is not None else self.new_counters(len(snr))
+        self._check(self.lib.ofdm_mc_sweep_channel_dev(self.h, C.byref(ch), seed, frame0, n_frames, n_sym, snr.ctypes.data,
+                                                       None if st is None else st.ctypes.data, len(snr), mode, _ptr(cnt)))
+        return None if counters is not None else self.read_counters(cnt)
+
+    def mc_sweep_channel_until(self, seed, frame0, n_sym, snr_db, mode, noise="real", snr_def="frame_power", n_taps=0, target_errors=100,
+                               max_bits=10 ** 9, round_frames=1 << 20):
+        """configs[3]'s stop rule through the channel (noise, snr_def, n_taps) on one GPU: returns (host totals, rounds)"""
+        ch = channel(noise, snr_def, n_taps)
+        snr = np.ascontiguousarray(snr_db, dtype=np.float32)
+        out = (Counters * len(snr))()
+        rounds = _I(0)
+        self._check(self.lib.ofdm_mc_sweep_channel_until(self.h, C.byref(ch), seed, frame0, n_sym, snr.ctypes.data, len(snr), mode,
+                                                         target_errors, max_bits, round_frames, out, C.byref(rounds)))
         return list(out), int(rounds.value)
 
     def multipath_taps(self, tx, taps, n_sym):

@@ -42,8 +42,8 @@ struct ofdm_ctx {
     unsigned long long *replayed_dev = nullptr;  // frames / points the speculating kernels replayed exactly (this context)
     float lts_power_prefix = 0.0f;
     // cached scratch (grown on demand, released with the context)
-    void *scratch[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    size_t scratch_bytes[6] = {0, 0, 0, 0, 0, 0};
+    void *scratch[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    size_t scratch_bytes[7] = {0, 0, 0, 0, 0, 0, 0};
 };
 
 namespace {
@@ -374,6 +374,34 @@ int sweep_points(ofdm_ctx *ctx, const float *frames, const float *g, const float
 
 bool mode_ok(int mode) { return mode == OFDM_MODE_EXACT || mode == OFDM_MODE_FAST; }
 bool nsym_ok(int n_sym) { return n_sym >= 1 && n_sym <= OFDM_MAX_SYM; }
+bool noise_ok(int noise) { return noise == OFDM_NOISE_REAL_RAIL || noise == OFDM_NOISE_COMPLEX; }
+bool snr_def_ok(int snr_def) { return snr_def >= OFDM_SNR_FRAME_POWER && snr_def <= OFDM_SNR_EBN0; }
+bool is_reference_channel(int noise, int snr_def) { return noise == OFDM_NOISE_REAL_RAIL && snr_def == OFDM_SNR_FRAME_POWER; }
+
+// noise power of an Es/N0 or Eb/N0 point: a data bin carries X (|X| = 1) and, through the transmitter's 1/64 IFFT and the
+// receiver's unscaled FFT, noise of variance 64 np, so Es/N0 = 1 / (64 np); Eb/N0 = Es/N0 / 2 (two bits per QPSK point).
+// In double, rounded to float once.
+float fixed_noise_power(int snr_def, float snr_db)
+{
+    const double per_point = snr_def == OFDM_SNR_EBN0 ? 128.0 : 64.0;
+    return (float)(1.0 / (per_point * pow(10.0, (double)snr_db / 10.0)));
+}
+
+// k_awgn_channel over n_frames frames of len samples: power != NULL -> np = power[f] / snr_lin, else np = np_fixed
+int launch_awgn_channel(ofdm_ctx *ctx, int noise, const float *tx, const float *power, float snr_lin, float np_fixed, uint32_t seed,
+                        uint32_t stream, uint64_t frame0, float *ota, long n_frames, int len, int mode)
+{
+    const float2 *x = reinterpret_cast<const float2 *>(tx);
+    float2 *y = reinterpret_cast<float2 *>(ota);
+    auto launch = [&](auto k) -> int {
+        int grid = grid_for(ctx, k, 0, kWarpsPerBlock, n_frames);
+        k<<<grid, kThreads, 0, ctx->stream>>>(x, power, snr_lin, np_fixed, seed, stream, frame0, y, n_frames, len);
+        return check_launch(ctx, "k_awgn_channel");
+    };
+    const bool cx = noise == OFDM_NOISE_COMPLEX;
+    if (mode == OFDM_MODE_EXACT) return cx ? launch(k_awgn_channel<true, true>) : launch(k_awgn_channel<true, false>);
+    return cx ? launch(k_awgn_channel<false, true>) : launch(k_awgn_channel<false, false>);
+}
 
 
 }  // namespace
@@ -489,7 +517,7 @@ int ofdm_ctx_destroy(ofdm_ctx *ctx)
     if (!ctx) return OFDM_ERR_INVALID;
     cudaSetDevice(ctx->device);
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-    for (int i = 0; i < 6; ++i) if (ctx->scratch[i]) cudaFree(ctx->scratch[i]);
+    for (int i = 0; i < 7; ++i) if (ctx->scratch[i]) cudaFree(ctx->scratch[i]);
     if (ctx->sts_dev) cudaFree(ctx->sts_dev);
     if (ctx->replayed_dev) cudaFree(ctx->replayed_dev);
     if (ctx->copy_stream) {
@@ -759,6 +787,23 @@ int ofdm_awgn_philox(ofdm_ctx *ctx, const float *tx, const float *power, float s
                      uint64_t frame0, float *ota, long n_frames, int n_sym, int mode)
 {
     return awgn_common(ctx, kNoisePhilox, tx, nullptr, power, snr_db, seed, stream, frame0, ota, n_frames, n_sym, mode);
+}
+int ofdm_awgn_philox_ex(ofdm_ctx *ctx, int noise, int snr_def, const float *tx, const float *power, float snr_db, uint32_t seed,
+                        uint32_t stream, uint64_t frame0, float *ota, long n_frames, int n_sym, int mode)
+{
+    if (int st = bind(ctx)) return st;
+    OFDM_REQUIRE(ctx, noise_ok(noise) && snr_def_ok(snr_def));
+    if (is_reference_channel(noise, snr_def))
+        return awgn_common(ctx, kNoisePhilox, tx, nullptr, power, snr_db, seed, stream, frame0, ota, n_frames, n_sym, mode);
+    OFDM_REQUIRE(ctx, n_frames >= 0 && nsym_ok(n_sym) && mode_ok(mode));
+    if (n_frames == 0) return OFDM_OK;
+    OFDM_REQUIRE(ctx, tx != nullptr && ota != nullptr);
+    const int len = OFDM_FRAME_LEN(n_sym);
+    if (snr_def != OFDM_SNR_FRAME_POWER)
+        return launch_awgn_channel(ctx, noise, tx, nullptr, 1.f, fixed_noise_power(snr_def, snr_db), seed, stream, frame0, ota, n_frames, len, mode);
+    const float *pw = nullptr;
+    if (int st = resolve_power(ctx, tx, power, n_frames, len, mode, &pw)) return st;
+    return launch_awgn_channel(ctx, noise, tx, pw, snr_linear(snr_db), 0.f, seed, stream, frame0, ota, n_frames, len, mode);
 }
 
 static int rx_common(ofdm_ctx *ctx, int noise, const float *in, const float *g, const float *power, const uint32_t *tx_bits,
@@ -1104,6 +1149,84 @@ int mc_awgn_core(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, long n_frames, i
 }
 int mc_multipath_core(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, long n_frames, int n_sym, int n_taps, const float *snr_db,
                       const uint32_t *streams, int n_snr, int mode, ofdm_counters *counters);
+
+// Channels other than the reference's, fp32, two-symbol frames: k_mc_quad<fast, MP, CH>, the frame built once on chip and the
+// channel + receiver run per point from shared memory.  The noise scale goes through McParams::inv_sqrt_snr: sigma / sqrt(P)
+// for the frame-power definition, sigma itself for Es/N0 and Eb/N0 (kChFixedSigma).
+int mc_channel_fused(ofdm_ctx *ctx, const ofdm_channel &ch, uint32_t seed, uint64_t frame0, long n_frames, const float *snr_db,
+                     const uint32_t *streams, int n_snr, ofdm_counters *counters)
+{
+    const bool cx = ch.noise == OFDM_NOISE_COMPLEX, fixed = ch.snr_def != OFDM_SNR_FRAME_POWER, mp = ch.n_taps > 0;
+    const double rail_share = cx ? 0.5 : 1.0;               // complex noise: half of the noise power per rail
+    const long max_frames = 1L << 30;                      // per launch: the per-lane totals are 32-bit
+    for (long f0 = 0; f0 < n_frames; f0 += max_frames) {
+        McParams p;
+        memset(&p, 0, sizeof p);
+        p.seed = seed; p.frame0 = frame0 + (uint64_t)f0; p.n_frames = n_frames - f0 < max_frames ? n_frames - f0 : max_frames;
+        p.n_snr = n_snr; p.counters = counters; p.n_taps = ch.n_taps;
+        for (int i = 0; i < n_snr; ++i) {
+            if (fixed) p.inv_sqrt_snr[i] = (float)sqrt(rail_share * (double)fixed_noise_power(ch.snr_def, snr_db[i]));
+            else { p.snr_lin[i] = snr_linear(snr_db[i]); p.inv_sqrt_snr[i] = (float)sqrt(rail_share / (double)p.snr_lin[i]); }
+            p.stream[i] = streams ? streams[i] : (uint32_t)i;
+        }
+        auto launch = [&](auto k) -> int {
+            const size_t smem = mp ? mc_quad_mp_smem_bytes() : mc_quad_smem_bytes();
+            OFDM_CUDA(ctx, allow_smem(ctx, k, smem));
+            int per_sm = 1;
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, kMcQuadWarps * 32, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
+            const long full = (long)per_sm * ctx->sm_count, need = (p.n_frames + kMcQuadWarps * 4 - 1) / (kMcQuadWarps * 4);
+            const long grid = need < full ? need : full;
+            k<<<(int)(grid < 1 ? 1 : grid), kMcQuadWarps * 32, smem, ctx->stream>>>(p);
+            return check_launch(ctx, "k_mc_quad<channel>");
+        };
+        constexpr int C = kChComplex, F = kChFixedSigma;
+        int st;
+        if (mp) st = cx ? (fixed ? launch(k_mc_quad<kArithFast, true, C | F>) : launch(k_mc_quad<kArithFast, true, C>)) : launch(k_mc_quad<kArithFast, true, F>);
+        else st = cx ? (fixed ? launch(k_mc_quad<kArithFast, false, C | F>) : launch(k_mc_quad<kArithFast, false, C>)) : launch(k_mc_quad<kArithFast, false, F>);
+        if (st) return st;
+    }
+    return OFDM_OK;
+}
+
+// Every other shape and EXACT: frames staged in HBM per chunk -- Philox bits, transmitter, [taps], [frame power], then per point
+// the channel (k_awgn_channel) into an OTA buffer and the verified receiver of ofdm_rx_frames on it
+int mc_channel_staged(ofdm_ctx *ctx, const ofdm_channel &ch, uint32_t seed, uint64_t frame0, long n_frames, int n_sym, const float *snr_db,
+                      const uint32_t *streams, int n_snr, int mode, ofdm_counters *counters)
+{
+    const int len = OFDM_FRAME_LEN(n_sym);
+    const bool per_frame = ch.snr_def == OFDM_SNR_FRAME_POWER;
+    long chunk = (2L << 30) / ((long)len * 8);
+    if (chunk < 1024) chunk = 1024;
+    for (long f0 = 0; f0 < n_frames; f0 += chunk) {
+        const long n = n_frames - f0 < chunk ? n_frames - f0 : chunk;
+        const size_t frame_bytes = (size_t)n * len * 2 * sizeof(float);
+        void *bits = nullptr, *frames = nullptr, *power = nullptr, *faded = nullptr, *ota = nullptr;
+        if (int st = ensure_scratch(ctx, 4, (size_t)n * n_sym * 3 * sizeof(uint32_t), &bits)) return st;
+        if (int st = ensure_scratch(ctx, 1, frame_bytes, &frames)) return st;
+        if (int st = ensure_scratch(ctx, 6, frame_bytes, &ota)) return st;
+        if (per_frame) if (int st = ensure_scratch(ctx, 2, (size_t)n * sizeof(float), &power)) return st;
+        const uint64_t fr0 = frame0 + (uint64_t)f0;
+        if (int st = ofdm_random_bits(ctx, seed, fr0, n, n_sym, (uint32_t *)bits)) return st;
+        if (int st = ofdm_tx_frames(ctx, (const uint32_t *)bits, (float *)frames, ch.n_taps > 0 ? nullptr : (float *)power, n, n_sym, mode)) return st;
+        const float *air = (const float *)frames;
+        if (ch.n_taps > 0) {
+            if (int st = ensure_scratch(ctx, 5, frame_bytes, &faded)) return st;
+            if (int st = ofdm_multipath_philox(ctx, air, seed, fr0, ch.n_taps, (float *)faded, nullptr, n, n_sym)) return st;
+            air = (const float *)faded;
+            if (per_frame) if (int st = frame_power(ctx, air, (float *)power, n, len, mode)) return st;     // power of what goes on the air
+        }
+        for (int i = 0; i < n_snr; ++i) {
+            const uint32_t stream = streams ? streams[i] : (uint32_t)i;
+            const int st = per_frame ? launch_awgn_channel(ctx, ch.noise, air, (const float *)power, snr_linear(snr_db[i]), 0.f, seed, stream, fr0,
+                                                           (float *)ota, n, len, mode)
+                                     : launch_awgn_channel(ctx, ch.noise, air, nullptr, 1.f, fixed_noise_power(ch.snr_def, snr_db[i]), seed, stream,
+                                                           fr0, (float *)ota, n, len, mode);
+            if (st) return st;
+            if (int st2 = ofdm_rx_frames(ctx, (const float *)ota, (const uint32_t *)bits, n, n_sym, mode, counters + i, nullptr)) return st2;
+        }
+    }
+    return OFDM_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -1121,19 +1244,42 @@ int ofdm_mc_sweep_philox_dev(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, long
 int ofdm_mc_sweep_points_dev(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, long n_frames, int n_sym, int n_taps, const float *snr_db,
                              const uint32_t *streams, int n_points, int mode, ofdm_counters *counters)
 {
+    const ofdm_channel ch = {OFDM_NOISE_REAL_RAIL, OFDM_SNR_FRAME_POWER, n_taps};
+    return ofdm_mc_sweep_channel_dev(ctx, &ch, seed, frame0, n_frames, n_sym, snr_db, streams, n_points, mode, counters);
+}
+
+int ofdm_mc_sweep_channel_dev(ofdm_ctx *ctx, const ofdm_channel *ch, uint32_t seed, uint64_t frame0, long n_frames, int n_sym,
+                              const float *snr_db, const uint32_t *streams, int n_points, int mode, ofdm_counters *counters)
+{
     if (int st = bind(ctx)) return st;
-    OFDM_REQUIRE(ctx, n_frames >= 0 && nsym_ok(n_sym) && mode_ok(mode) && n_points >= 0 && n_points <= kMaxSnr && n_taps >= 0 && n_taps <= kMaxTaps);
+    OFDM_REQUIRE(ctx, ch != nullptr && noise_ok(ch->noise) && snr_def_ok(ch->snr_def) && ch->n_taps >= 0 && ch->n_taps <= kMaxTaps);
+    OFDM_REQUIRE(ctx, n_frames >= 0 && nsym_ok(n_sym) && mode_ok(mode) && n_points >= 0 && n_points <= kMaxSnr);
     if (n_frames == 0 || n_points == 0) return OFDM_OK;
     OFDM_REQUIRE(ctx, snr_db != nullptr && counters != nullptr);
-    if (n_taps > 0) return mc_multipath_core(ctx, seed, frame0, n_frames, n_sym, n_taps, snr_db, streams, n_points, mode, counters);
-    return mc_awgn_core(ctx, seed, frame0, n_frames, n_sym, snr_db, streams, n_points, mode, counters);
+    if (is_reference_channel(ch->noise, ch->snr_def)) {
+        if (ch->n_taps > 0) return mc_multipath_core(ctx, seed, frame0, n_frames, n_sym, ch->n_taps, snr_db, streams, n_points, mode, counters);
+        return mc_awgn_core(ctx, seed, frame0, n_frames, n_sym, snr_db, streams, n_points, mode, counters);
+    }
+    if (mode != OFDM_MODE_EXACT && n_sym == 2 && !ctx->force_generic)
+        return mc_channel_fused(ctx, *ch, seed, frame0, n_frames, snr_db, streams, n_points, counters);
+    return mc_channel_staged(ctx, *ch, seed, frame0, n_frames, n_sym, snr_db, streams, n_points, mode, counters);
 }
 
 int ofdm_mc_sweep_until(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, int n_sym, int n_taps, const float *snr_db, int n_snr, int mode,
                         uint64_t target_errors, uint64_t max_bits, long round_frames, ofdm_counters *out_host, int *rounds_out)
 {
+    const ofdm_channel ch = {OFDM_NOISE_REAL_RAIL, OFDM_SNR_FRAME_POWER, n_taps};
+    return ofdm_mc_sweep_channel_until(ctx, &ch, seed, frame0, n_sym, snr_db, n_snr, mode, target_errors, max_bits, round_frames, out_host,
+                                       rounds_out);
+}
+
+int ofdm_mc_sweep_channel_until(ofdm_ctx *ctx, const ofdm_channel *ch, uint32_t seed, uint64_t frame0, int n_sym, const float *snr_db,
+                                int n_snr, int mode, uint64_t target_errors, uint64_t max_bits, long round_frames, ofdm_counters *out_host,
+                                int *rounds_out)
+{
     if (int st = bind(ctx)) return st;
-    OFDM_REQUIRE(ctx, nsym_ok(n_sym) && mode_ok(mode) && n_snr >= 0 && n_snr <= kMaxSnr && n_taps >= 0 && n_taps <= kMaxTaps);
+    OFDM_REQUIRE(ctx, ch != nullptr && noise_ok(ch->noise) && snr_def_ok(ch->snr_def) && ch->n_taps >= 0 && ch->n_taps <= kMaxTaps);
+    OFDM_REQUIRE(ctx, nsym_ok(n_sym) && mode_ok(mode) && n_snr >= 0 && n_snr <= kMaxSnr);
     OFDM_REQUIRE(ctx, round_frames >= 1 && max_bits >= 1 && (n_snr == 0 || (snr_db != nullptr && out_host != nullptr)));
     if (rounds_out) *rounds_out = 0;
     if (n_snr == 0) return OFDM_OK;
@@ -1148,8 +1294,8 @@ int ofdm_mc_sweep_until(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, int n_sym
         uint32_t stream_a[kMaxSnr];
         for (int j = 0; j < n_active; ++j) { snr_a[j] = snr_db[active[j]]; stream_a[j] = (uint32_t)active[j]; }
         OFDM_CUDA(ctx, cudaMemsetAsync(cnt, 0, sizeof(ofdm_counters) * (size_t)n_active, ctx->stream));
-        if (int st = ofdm_mc_sweep_points_dev(ctx, seed, frame0 + (uint64_t)rounds * (uint64_t)round_frames, round_frames, n_sym, n_taps, snr_a, stream_a,
-                                              n_active, mode, (ofdm_counters *)cnt))
+        if (int st = ofdm_mc_sweep_channel_dev(ctx, ch, seed, frame0 + (uint64_t)rounds * (uint64_t)round_frames, round_frames, n_sym, snr_a, stream_a,
+                                               n_active, mode, (ofdm_counters *)cnt))
             return st;
         OFDM_CUDA(ctx, cudaMemcpyAsync(part, cnt, sizeof(ofdm_counters) * (size_t)n_active, cudaMemcpyDeviceToHost, ctx->stream));
         OFDM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));

@@ -282,7 +282,9 @@ struct Philox {
         return c;
     }
 };
-enum { kDomainNoise = 0, kDomainBits = 1, kDomainTaps = 2 };
+// domain 3 is the flat noise layout of k_awgn_philox_flat; domain 4 holds the Q-rail draws of complex noise, in the block
+// layout of domain 0 (noise_slot), so that a complex channel's I-rail draws are exactly those of the real-rail channel
+enum { kDomainNoise = 0, kDomainBits = 1, kDomainTaps = 2, kDomainNoiseQ = 4 };
 
 // one Box-Muller pair from two words (both branches used); fast intrinsics
 __device__ __forceinline__ float2 box_muller(uint32_t r0, uint32_t r1)

@@ -385,6 +385,41 @@ __global__ void __launch_bounds__(kThreads) k_awgn(const float2 *__restrict__ tx
     }
 }
 
+// z[j] without indexing a local array (selects stay in registers)
+__device__ __forceinline__ float pick4(const float (&z)[4], int j) { return j == 0 ? z[0] : (j == 1 ? z[1] : (j == 2 ? z[2] : z[3])); }
+
+// The channel of ofdm_awgn_philox_ex on LTS||data frames (include/ofdm_b200.h, DESIGN.md "Channels").  Noise power per frame:
+// power[f] / snr_lin (the reference's definition), or np_fixed for every frame when power is NULL (Es/N0, Eb/N0).  Real rail:
+// all of it on I, sigma = sqrt(np); COMPLEX: half per rail, sigma = sqrt(np / 2), the Q-rail draw is the normal in the same
+// slot of domain 4.  EXACT: x + (float)(sigma_d * (double)g) per rail; fast: fmaf with sigma in fp32.  One warp per frame.
+template <bool EXACT, bool COMPLEX>
+__global__ void __launch_bounds__(kThreads) k_awgn_channel(const float2 *__restrict__ tx, const float *__restrict__ power,
+                                                           float snr_lin, float np_fixed, uint32_t seed, uint32_t stream,
+                                                           uint64_t frame0, float2 *__restrict__ ota, long n_frames, int len)
+{
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (long f = (long)blockIdx.x * kWarpsPerBlock + warp; f < n_frames; f += (long)gridDim.x * kWarpsPerBlock) {
+        const float np = power ? __fdiv_rn(power[f], snr_lin) : np_fixed;
+        const double sigma_d = __dsqrt_rn(COMPLEX ? __dmul_rn(0.5, (double)np) : (double)np);
+        const float sigma_f = (float)sigma_d;
+        const uint64_t fr = frame0 + (uint64_t)f;
+        const float2 *x = tx + f * len;
+        float2 *y = ota + f * len;
+        for (int n = lane; n < len; n += 32) {
+            float2 s = x[n];
+            int blk, j; noise_slot(n, blk, j);
+            float z[4];
+            philox_normals4(seed, stream, fr, (uint32_t)blk, kDomainNoise, z);
+            s.x = add_noise<EXACT>(s.x, pick4(z, j), sigma_d, sigma_f);
+            if (COMPLEX) {
+                philox_normals4(seed, stream, fr, (uint32_t)blk, kDomainNoiseQ, z);
+                s.y = add_noise<EXACT>(s.y, pick4(z, j), sigma_d, sigma_f);
+            }
+            y[n] = s;
+        }
+    }
+}
+
 // ------------------------------------------------------------------ receiver (optionally fused with the channel)
 struct RxParams {
     const float2 *in;           // OTA frames (NOISE == none) or TX frames (noise added in registers)

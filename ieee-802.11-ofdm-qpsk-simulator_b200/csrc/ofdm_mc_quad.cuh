@@ -47,11 +47,18 @@ inline size_t mc_quad_mp_smem_bytes() { return sizeof(McQuadWarpMp) * kMcQuadWar
 template <bool MP> struct McQuadSmem { using type = McQuadWarp; };
 template <> struct McQuadSmem<true> { using type = McQuadWarpMp; };
 
-template <int ARITH, bool MP = false>
+// CH, the channel (DESIGN.md "Channels"; 0 = the reference's): kChComplex = circular complex noise, the Q-rail draws from
+// domain 4 in the blocks of the I-rail ones; kChFixedSigma = the noise scale does not depend on the frame (Es/N0, Eb/N0): no
+// frame power is measured and p.inv_sqrt_snr[i] holds point i's sigma itself.  Otherwise sigma = sqrt(P) * p.inv_sqrt_snr[i].
+enum { kChComplex = 1, kChFixedSigma = 2 };
+
+template <int ARITH, bool MP = false, int CH = 0>
 __global__ void __launch_bounds__(kMcQuadWarps * 32, 2) k_mc_quad(McParams p)
 {
     static_assert(ARITH == kArithFast || ARITH == kArithChecked, "the all-exact arithmetic runs in k_mc_philox");
     static_assert(!MP || ARITH == kArithFast, "the fused multipath variant is fp32 only");
+    static_assert(CH == 0 || ARITH == kArithFast, "the fused channel variants are fp32 only (EXACT runs staged)");
+    constexpr bool COMPLEX = (CH & kChComplex) != 0, FIXED = (CH & kChFixedSigma) != 0;
     constexpr bool CHECKED = ARITH == kArithChecked;
     constexpr int LEVEL = CHECKED ? 2 : 0;                        // fast: plain fp32 (statistical results, no EVM guard: as k_mc_philox)
     constexpr int WARPS = kMcQuadWarps;
@@ -118,7 +125,7 @@ __global__ void __launch_bounds__(kMcQuadWarps * 32, 2) k_mc_quad(McParams p)
             }
         }
         __syncwarp();
-        float P;
+        float P = 0.f;
         if constexpr (MP) {
             // taps of this frame (k_multipath<true>): i.i.d. complex Gaussian, E|h_l|^2 = 1 / n_taps
             const int n_taps = p.n_taps;
@@ -150,7 +157,7 @@ __global__ void __launch_bounds__(kMcQuadWarps * 32, 2) k_mc_quad(McParams p)
             float pm = 0.f;
             for (int n = u; n < 160; n += 8) {                      // the LTS slot: guard interval (power only), then the two halves
                 const float2 y = fir(s_ltsx + n, n_taps - 1 < n ? n_taps - 1 : n);
-                pm = fmaf(y.x, y.x, fmaf(y.y, y.y, pm));
+                if constexpr (!FIXED) pm = fmaf(y.x, y.x, fmaf(y.y, y.y, pm));
                 if (n >= 32) ws.fwl[grp][((n - 32) >> 6) * kWin + ((n - 32) & 63)] = y;
             }
             // symbol 1 first: its cyclic prefix still needs the clean tail of symbol 0 (the taps reach 15 samples back), while
@@ -164,7 +171,7 @@ __global__ void __launch_bounds__(kMcQuadWarps * 32, 2) k_mc_quad(McParams p)
 #pragma unroll 1
                 for (int m = 0; m < 10; ++m) {
                     const float2 y = fir(st + 15 + u + 8 * m, n_taps - 1);
-                    pm = fmaf(y.x, y.x, fmaf(y.y, y.y, pm));
+                    if constexpr (!FIXED) pm = fmaf(y.x, y.x, fmaf(y.y, y.y, pm));
                     if (m >= 2) ws.body[grp][s * kWin + u + 8 * (m - 2)] = y;
                 }
                 __syncwarp();
@@ -208,14 +215,14 @@ __global__ void __launch_bounds__(kMcQuadWarps * 32, 2) k_mc_quad(McParams p)
             // float square root, tests/test_sigma_rounding.py), spread over the group's lanes
             for (int si = u; si < p.n_snr; si += 8) ws.sig[grp][si] = __fsqrt_rn(__fdiv_rn(P, p.snr_lin[si]));
             __syncwarp();
-        } else {
+        } else if constexpr (!FIXED) {
             pw += __shfl_xor_sync(0xffffffffu, pw, 1);
             pw += __shfl_xor_sync(0xffffffffu, pw, 2);
             pw += __shfl_xor_sync(0xffffffffu, pw, 4);
             P = (pw + c_tab.lts_power_sum) * (1.f / 320.f);
         }
-        float sqrtP;
-        asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(sqrtP) : "f"(P));
+        float sqrtP = 1.f;
+        if constexpr (!FIXED) asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(sqrtP) : "f"(P));
         const float chan = CHECKED ? p.radius_chan * sqrtP : 0.f;
         // the lane's payload words, bit a of every data bin with L < 0 flipped (quad_slot)
         const uint32_t fw[2][3] = {{b0.x ^ ql.flip0, b0.y ^ ql.flip1, b0.z ^ ql.flip2}, {b1.x ^ ql.flip0, b1.y ^ ql.flip1, b1.z ^ ql.flip2}};
@@ -235,7 +242,8 @@ __global__ void __launch_bounds__(kMcQuadWarps * 32, 2) k_mc_quad(McParams p)
             float sigma_f;
             if constexpr (CHECKED) sigma_f = ws.sig[grp][si]; else sigma_f = sqrtP * p.inv_sqrt_snr[si];
             const uint32_t stream = p.stream[si];
-            // noisy samples of the window whose Philox blocks start at blk (v[m] = x[u + 8m] + sigma z, real rail only: SURVEY Q1)
+            // noisy samples of the window whose Philox blocks start at blk (v[m] = x[u + 8m] + sigma z, real rail only: SURVEY Q1;
+            // kChComplex: + i sigma z' with z' the normal in the same slot of domain 4)
             auto window = [&](const float2 *src, int blk, float2 (&v)[8], float2 &n2) {
                 float za[4], zb[4];
                 philox_normals4(p.seed, stream, fr, (uint32_t)(blk + u), kDomainNoise, za);
@@ -246,6 +254,12 @@ __global__ void __launch_bounds__(kMcQuadWarps * 32, 2) k_mc_quad(McParams p)
                     smp.x = fmaf(sigma_f, m < 4 ? za[m] : zb[m - 4], smp.x);               // speculated channel (kChanRadius)
                     if (CHECKED) n2 = __ffma2_rn(smp, smp, n2);
                     v[m] = smp;
+                }
+                if constexpr (COMPLEX) {
+                    philox_normals4(p.seed, stream, fr, (uint32_t)(blk + u), kDomainNoiseQ, za);
+                    philox_normals4(p.seed, stream, fr, (uint32_t)(blk + u + 8), kDomainNoiseQ, zb);
+#pragma unroll
+                    for (int m = 0; m < 8; ++m) v[m].y = fmaf(sigma_f, m < 4 ? za[m] : zb[m - 4], v[m].y);
                 }
             };
             // ---- Channel_Estimation :830-850: the two noisy halves added in time, one transform; G = A + B at bins u + 8j

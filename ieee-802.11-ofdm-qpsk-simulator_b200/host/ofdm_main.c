@@ -25,6 +25,11 @@
  *   --draws FILE [--bits FILE]: configs[1] from C -- injected-noise sweep (ofdm_sweep_inject_host): FILE holds one float32
  *       standard-normal draw per sample, [frames][160 + 80 nsym] (e.g. the reference's captured g_keep stream); the payload is
  *       the Philox bit stream of --seed, or packed uint32 words [frames][3 nsym] from --bits;
+ *   --noise real|complex, --snr-def frame_power|esn0|ebn0 (with --frames N or --target-errors E, also with --taps and --gpus): the
+ *       channel of the Monte-Carlo sweep (ofdm_channel, include/ofdm_b200.h).  The default, real / frame_power, is the reference's:
+ *       noise on the I rail only, SNR = measured frame power / noise power.  complex = circular complex noise, half of the noise
+ *       power per rail; esn0 / ebn0 = Es/N0 per data subcarrier / Eb/N0, the SNR axis of textbook QPSK curves.  Not available
+ *       with --message or --draws, whose channels are the reference's by definition;
  *   --gpus N: the frames of the Monte-Carlo sweep are sharded across N GPUs of this node by global frame index
  *       (one context per GPU, all driven from this thread) and the counters are summed with ONE NCCL all-reduce
  *       per buffer type (built with -DOFDM_WITH_NCCL; link -lnccl).
@@ -104,9 +109,10 @@ static void report_rate(const char *what, int n_gpus, long frames, int n_sym, in
     } while (0)
 
 /* SURVEY 8(e): shard (frame range) across GPUs, counter-based RNG keyed on the global frame index, one all-reduce */
-static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, int n_taps, const float *SNR, int n_snr, int mode, ofdm_counters *totals,
-                           unsigned long long target_errors, unsigned long long max_bits, long round_frames, int round_reduce_host)
+static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, const ofdm_channel *ch, const float *SNR, int n_snr, int mode,
+                           ofdm_counters *totals, unsigned long long target_errors, unsigned long long max_bits, long round_frames, int round_reduce_host)
 {
+    const int n_taps = ch->n_taps, reference = ch->noise == OFDM_NOISE_REAL_RAIL && ch->snr_def == OFDM_SNR_FRAME_POWER;
     ofdm_ctx *ctxs[8] = {0};
     ofdm_ctx *ctx = NULL;
     void *cnt[8], *ints[8], *dbls[8];
@@ -125,7 +131,8 @@ static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, in
     NCHECK(ncclCommInitAll(comms, n_gpus, devs));
     for (int d = 0; d < n_gpus; ++d) {                      /* first use of a kernel on a device loads it: keep that out of the timing */
         ctx = ctxs[d];
-        if (n_taps > 0) CHECK(ofdm_mc_sweep_multipath_dev(ctx, seed, 0, 256, n_sym, n_taps, SNR, n_snr, mode, (ofdm_counters *)cnt[d]));
+        if (!reference) CHECK(ofdm_mc_sweep_channel_dev(ctx, ch, seed, 0, 256, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)cnt[d]));
+        else if (n_taps > 0) CHECK(ofdm_mc_sweep_multipath_dev(ctx, seed, 0, 256, n_sym, n_taps, SNR, n_snr, mode, (ofdm_counters *)cnt[d]));
         else CHECK(ofdm_mc_sweep_philox_dev(ctx, seed, 0, 256, n_sym, SNR, n_snr, mode, (ofdm_counters *)cnt[d]));
         CHECK(ofdm_memset_dev(ctx, cnt[d], 0, sizeof(ofdm_counters) * (size_t)n_snr));
         CHECK(ofdm_counters_pack(ctx, (const ofdm_counters *)cnt[d], n_snr, (uint64_t *)ints[d], (double *)dbls[d]));
@@ -157,8 +164,8 @@ static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, in
                 long lo = d * base + (d < rem ? d : rem), n = base + (d < rem ? 1 : 0);
                 ctx = ctxs[d];
                 CHECK(ofdm_memset_dev(ctx, cnt[d], 0, sizeof(ofdm_counters) * (size_t)n_active));
-                CHECK(ofdm_mc_sweep_points_dev(ctx, seed, (uint64_t)rounds * (uint64_t)round_frames + (uint64_t)lo, n, n_sym, n_taps, snr_a, stream_a,
-                                               n_active, mode, (ofdm_counters *)cnt[d]));
+                CHECK(ofdm_mc_sweep_channel_dev(ctx, ch, seed, (uint64_t)rounds * (uint64_t)round_frames + (uint64_t)lo, n, n_sym, snr_a, stream_a,
+                                                n_active, mode, (ofdm_counters *)cnt[d]));
                 if (!round_reduce_host) CHECK(ofdm_counters_pack(ctx, (const ofdm_counters *)cnt[d], n_active, (uint64_t *)ints[d], (double *)dbls[d]));
             }
             if (round_reduce_host) {
@@ -212,7 +219,8 @@ static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, in
         long base = frames / n_gpus, rem = frames % n_gpus;
         long lo = d * base + (d < rem ? d : rem), n = base + (d < rem ? 1 : 0);
         ctx = ctxs[d];
-        if (n_taps > 0) CHECK(ofdm_mc_sweep_multipath_dev(ctx, seed, (uint64_t)lo, n, n_sym, n_taps, SNR, n_snr, mode, (ofdm_counters *)cnt[d]));
+        if (!reference) CHECK(ofdm_mc_sweep_channel_dev(ctx, ch, seed, (uint64_t)lo, n, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)cnt[d]));
+        else if (n_taps > 0) CHECK(ofdm_mc_sweep_multipath_dev(ctx, seed, (uint64_t)lo, n, n_sym, n_taps, SNR, n_snr, mode, (ofdm_counters *)cnt[d]));
         else CHECK(ofdm_mc_sweep_philox_dev(ctx, seed, (uint64_t)lo, n, n_sym, SNR, n_snr, mode, (ofdm_counters *)cnt[d]));
         CHECK(ofdm_counters_pack(ctx, (const ofdm_counters *)cnt[d], n_snr, (uint64_t *)ints[d], (double *)dbls[d]));
     }
@@ -250,6 +258,8 @@ int main(int argc, char **argv)
     unsigned long long target_errors = 0, max_bits = 0;
     long round_frames = 1L << 22;
     const char *draws_file = NULL, *bits_file = NULL;
+    ofdm_channel ch = {OFDM_NOISE_REAL_RAIL, OFDM_SNR_FRAME_POWER, 0};
+    int channel_set = 0;                 /* --noise / --snr-def given */
     int round_reduce_host = 1;           /* until rule: per-round totals summed on the host (measured 8 GPUs, 13 rounds: 0.033 s against 0.294 s with two
                                             single-process NCCL group all-reduces per round, profiles/r2_c_driver_until_8gpu.txt) */
     for (int i = 1; i < argc; ++i) {
@@ -278,12 +288,31 @@ int main(int argc, char **argv)
         else if (!strcmp(a, "--outdir")) outdir = v;
         else if (!strcmp(a, "--dump")) dump = v;
         else if (!strcmp(a, "--mode")) mode = !strcmp(v, "fast") ? OFDM_MODE_FAST : OFDM_MODE_EXACT;
+        else if (!strcmp(a, "--noise")) {
+            if (!strcmp(v, "real")) ch.noise = OFDM_NOISE_REAL_RAIL;
+            else if (!strcmp(v, "complex")) ch.noise = OFDM_NOISE_COMPLEX;
+            else { fprintf(stderr, "--noise must be real or complex\n"); return 2; }
+            channel_set = 1;
+        } else if (!strcmp(a, "--snr-def")) {
+            if (!strcmp(v, "frame_power")) ch.snr_def = OFDM_SNR_FRAME_POWER;
+            else if (!strcmp(v, "esn0")) ch.snr_def = OFDM_SNR_ESN0;
+            else if (!strcmp(v, "ebn0")) ch.snr_def = OFDM_SNR_EBN0;
+            else { fprintf(stderr, "--snr-def must be frame_power, esn0 or ebn0\n"); return 2; }
+            channel_set = 1;
+        }
         else { fprintf(stderr, "unknown option %s\n", a); return 2; }
         ++i;
     }
     if (n_snr < 1 || n_snr > 64 || frames < 1) { fprintf(stderr, "need 1 <= snr-count <= 64 and frames >= 1\n"); return 2; }
     if (target_errors > 0 && max_bits == 0) max_bits = target_errors * 10000000ULL;        /* the BER-1e-7 budget */
     if (round_frames < 1) { fprintf(stderr, "--round-frames must be >= 1\n"); return 2; }
+    if (channel_set && (draws_file || (frames < 2 && target_errors == 0))) {
+        fprintf(stderr, "--noise / --snr-def choose the channel of the Monte-Carlo sweeps (--frames N > 1 or --target-errors E); "
+                        "--message and --draws run the reference's channel\n");
+        return 2;
+    }
+    ch.n_taps = n_taps;
+    const int reference_channel = ch.noise == OFDM_NOISE_REAL_RAIL && ch.snr_def == OFDM_SNR_FRAME_POWER;
 
     ofdm_ctx *ctx = NULL;
     float SNR[64], EVM_dB[64], EVM_AGC_dB[64], BER[64];
@@ -293,7 +322,7 @@ int main(int argc, char **argv)
     if (n_gpus > 1) {
 #ifdef OFDM_WITH_NCCL
         if (frames < 2 && target_errors == 0) { fprintf(stderr, "--gpus needs --frames N > 1 or --target-errors E\n"); return 2; }
-        int rc = sweep_multi_gpu(n_gpus, seed, frames, n_sym, n_taps, SNR, n_snr, mode, totals, target_errors, max_bits, round_frames, round_reduce_host);
+        int rc = sweep_multi_gpu(n_gpus, seed, frames, n_sym, &ch, SNR, n_snr, mode, totals, target_errors, max_bits, round_frames, round_reduce_host);
         if (rc) return rc;
 #else
         fprintf(stderr, "built without NCCL (make ofdm_sweep NCCL=1)\n");
@@ -338,12 +367,22 @@ int main(int argc, char **argv)
     } else if (target_errors > 0) {                    /* configs[3]: until >= E errors or the bit budget, one GPU */
         int rounds = 0;
         const double t0 = now_s();
-        CHECK(ofdm_mc_sweep_until(ctx, seed, 0, n_sym, n_taps, SNR, n_snr, mode, target_errors, max_bits, round_frames, totals, &rounds));
+        CHECK(ofdm_mc_sweep_channel_until(ctx, &ch, seed, 0, n_sym, SNR, n_snr, mode, target_errors, max_bits, round_frames, totals, &rounds));
         unsigned long long fp = 0;
         for (int i = 0; i < n_snr; ++i) fp += totals[i].frames;
         const double dt = now_s() - t0;
         fprintf(stderr, "until-sweep: %d rounds of %ld frames, %llu frame-points x %d symbols on 1 GPU(s) in %.3f s = %.3e data symbols/s\n", rounds, round_frames,
                 fp, n_sym, dt, (double)fp * n_sym / dt);
+    } else if (frames > 1 && !reference_channel) {     /* another channel, with or without taps */
+        void *d_cnt = NULL;
+        CHECK(ofdm_dev_alloc(ctx, &d_cnt, sizeof(ofdm_counters) * (size_t)n_snr));
+        CHECK(ofdm_memset_dev(ctx, d_cnt, 0, sizeof(ofdm_counters) * (size_t)n_snr));
+        const double t0 = now_s();
+        CHECK(ofdm_mc_sweep_channel_dev(ctx, &ch, seed, 0, frames, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)d_cnt));
+        CHECK(ofdm_memcpy_d2h(ctx, totals, d_cnt, sizeof(ofdm_counters) * (size_t)n_snr));
+        CHECK(ofdm_ctx_sync(ctx));
+        report_rate("channel sweep", 1, frames, n_sym, n_snr, now_s() - t0);
+        ofdm_dev_free(ctx, d_cnt);
     } else if (frames > 1 && n_taps > 0) {             /* configs[4]: per-frame random multipath taps */
         void *d_cnt = NULL;
         CHECK(ofdm_dev_alloc(ctx, &d_cnt, sizeof(ofdm_counters) * (size_t)n_snr));

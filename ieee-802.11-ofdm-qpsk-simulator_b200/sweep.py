@@ -2,6 +2,7 @@
 one all-reduce of the per-SNR counters (the only exchange the path has -- SURVEY.md section 8(e)).
 Works with any torch.distributed backend: nccl on the GPUs, gloo in the CPU tests."""
 import ctypes as C
+import math
 
 import numpy as np
 
@@ -102,10 +103,11 @@ def until_loop(run_round, n_points, target_errors, max_bits, round_frames, rank=
 
 
 def mc_sweep_until(ofdm, seed, n_sym, snr_db, mode, target_errors=100, max_bits=10 ** 9, round_frames=1 << 22, n_taps=0, rank=0, world=1,
-                   group=None, frame0=0):
+                   group=None, frame0=0, noise="real", snr_def="frame_power"):
     """configs[3] as stated, on ``world`` GPUs: SNR points x frame ranges are sharded by rounds (every rank works on every
     still-active point, on its own slice of the round's frames -- so the slow high-SNR points use all GPUs), one all-reduce
-    of the counters per round.  Returns (list of global Counters, rounds) on every rank."""
+    of the counters per round.  ``noise`` / ``snr_def`` choose the channel (binding.channel; the default is the reference's).
+    Returns (list of global Counters, rounds) on every rank."""
     import torch
     import torch.distributed as dist
     snr = np.asarray(snr_db, dtype=np.float32)
@@ -115,7 +117,7 @@ def mc_sweep_until(ofdm, seed, n_sym, snr_db, mode, target_errors=100, max_bits=
         c = cnt[:len(points)]
         c.zero_()
         if n > 0:
-            ofdm.mc_sweep_points(seed, lo, n, n_sym, n_taps, snr[points], np.asarray(points, dtype=np.uint32), mode, c)
+            ofdm.mc_sweep_channel(seed, lo, n, n_sym, snr[points], mode, noise, snr_def, n_taps, np.asarray(points, dtype=np.uint32), c)
         if world > 1:
             allreduce_counter_tensor(c, group)              # on the device: NCCL over NVLink
         raw = c.cpu().numpy()
@@ -132,3 +134,20 @@ def ber_table(snr_db, counters):
         evm = np.sqrt(c.sum_err2 / c.sum_ref2) if c.sum_ref2 else float("nan")
         rows.append((float(s), int(c.bit_errors), int(c.bits), ber, 20 * np.log10(evm) if evm > 0 else -np.inf, int(c.frames_in_error)))
     return rows
+
+
+def qpsk_ber_awgn(snr_db, snr_def="esn0"):
+    """BER of this project's QPSK map over an AWGN channel with perfect channel knowledge: the textbook curve to lay the
+    measured one over.  snr_def "esn0" (Es/N0 per data subcarrier) or "ebn0" (Eb/N0 = Es/N0 / 2), as in binding.channel.
+
+    Each rail is decided alone with error probability p = Q(sqrt(Es/N0)).  The map (QPSK_Modulator, OFDM.c:415-433:
+    00 -> (+,+), 01 -> (-,+), 10 -> (-,-), 11 -> (+,-)) is not Gray coded: an I-rail error costs 1 bit, a Q-rail error 2 and
+    both together 1, so BER = (p (1-p) + 2 p (1-p) + p^2) / 2 = (3p - 2p^2) / 2.
+
+    The receiver does not know the channel: it estimates it from the two LTS halves, whose noise (half the variance of a data
+    bin's) goes into every equalised point.  The measured curve therefore lies to the right of this one."""
+    if snr_def not in ("esn0", "ebn0"):
+        raise ValueError("qpsk_ber_awgn needs snr_def 'esn0' or 'ebn0', not %r (the frame-power SNR depends on the frame)" % (snr_def,))
+    esn0 = 10.0 ** (np.asarray(snr_db, dtype=np.float64) / 10.0) * (2.0 if snr_def == "ebn0" else 1.0)
+    p = 0.5 * np.vectorize(math.erfc)(np.sqrt(esn0 / 2.0))  # Q(x) = erfc(x / sqrt(2)) / 2
+    return (3.0 * p - 2.0 * p * p) / 2.0

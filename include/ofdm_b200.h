@@ -161,6 +161,25 @@ int ofdm_awgn_inject(ofdm_ctx *ctx, const float *tx_dev, const float *g_dev, con
                      float *ota_dev, long n_frames, int n_sym, int mode);
 int ofdm_awgn_philox(ofdm_ctx *ctx, const float *tx_dev, const float *power_dev, float snr_db, uint32_t seed,
                      uint32_t stream, uint64_t frame0, float *ota_dev, long n_frames, int n_sym, int mode);
+
+/* ---- channels (no reference counterpart: the reference's channel is OFDM_NOISE_REAL_RAIL + OFDM_SNR_FRAME_POWER) ----
+ * noise:   OFDM_NOISE_REAL_RAIL  all of the noise power np on the I rail, y.re = x.re + sqrt(np) g0, y.im = x.im (SURVEY Q1);
+ *          OFDM_NOISE_COMPLEX    circular complex noise of total variance np, y = x + sqrt(np/2) (g0 + i g1).
+ * snr_def: OFDM_SNR_FRAME_POWER  np = P / (float)pow(10, snr_db/10), P the per-frame power of OFDM.c:637-643 (after the taps);
+ *          OFDM_SNR_ESN0         Es/N0 per data subcarrier: np = (float)(1 / (64 * 10^(snr_db/10))), the same for every frame;
+ *          OFDM_SNR_EBN0         Eb/N0, 2 bits per QPSK point: np = (float)(1 / (128 * 10^(snr_db/10))).
+ * n_taps:  0 = AWGN, 1..16 = the multipath channel of configs[4] below in front of the noise.
+ * g0 is the Philox domain-0 normal the real-rail channel draws for the sample, g1 the normal in the same slot of domain 4.
+ * EXACT: sigma_d = sqrt((double)np) (real rail) or sqrt(0.5 * (double)np) (complex), each noisy rail x + (float)(sigma_d * g);
+ * FAST: fmaf(sigma_f, g, x).  {OFDM_NOISE_REAL_RAIL, OFDM_SNR_FRAME_POWER, n} is the reference's channel and runs exactly the
+ * code of ofdm_awgn_philox / ofdm_mc_sweep_points_dev / ofdm_mc_sweep_until. */
+enum { OFDM_NOISE_REAL_RAIL = 0, OFDM_NOISE_COMPLEX = 1 };
+enum { OFDM_SNR_FRAME_POWER = 0, OFDM_SNR_ESN0 = 1, OFDM_SNR_EBN0 = 2 };
+typedef struct { int noise, snr_def, n_taps; } ofdm_channel;
+/* the channel on LTS||data frames, Philox draws as ofdm_awgn_philox; power_dev (nullable) is computed when snr_def needs it and
+ * ignored otherwise.  Chained with ofdm_rx_frames it gives per-bin dumps (e.g. constellations) under any channel. */
+int ofdm_awgn_philox_ex(ofdm_ctx *ctx, int noise, int snr_def, const float *tx_dev, const float *power_dev, float snr_db,
+                        uint32_t seed, uint32_t stream, uint64_t frame0, float *ota_dev, long n_frames, int n_sym, int mode);
 /* Receiver OFDM.c:1018-1165 on LTS||data frames: Channel_Estimation :830, CP strip :1024, fft :1037,
  * equalise :1046, demap :1061, AGC_Receiver :852, QPSK_Demodulator :873, EVM :1106-1150, BER :1154.
  * counters_dev (device, one ofdm_counters, accumulated into -- zero it first) may be NULL. */
@@ -239,6 +258,16 @@ int ofdm_mc_sweep_points_dev(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, long
 int ofdm_mc_sweep_until(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, int n_sym, int n_taps, const float *snr_db, int n_snr,
                         int mode, uint64_t target_errors, uint64_t max_bits, long round_frames, ofdm_counters *out_host,
                         int *rounds_out);
+/* The two above through any channel (ofdm_channel, see ofdm_awgn_philox_ex); ofdm_mc_sweep_points_dev and ofdm_mc_sweep_until are
+ * these with {OFDM_NOISE_REAL_RAIL, OFDM_SNR_FRAME_POWER, n_taps}.  Other channels run FAST two-symbol sweeps fused on chip
+ * (k_mc_quad) and everything else -- all of EXACT -- staged: Philox bits, transmitter, [taps], [frame power], then per point
+ * the channel into HBM and the verified receiver of ofdm_rx_frames.  Results depend only on (seed, global frame index, stream).
+ * A NULL or invalid channel returns OFDM_ERR_INVALID. */
+int ofdm_mc_sweep_channel_dev(ofdm_ctx *ctx, const ofdm_channel *ch, uint32_t seed, uint64_t frame0, long n_frames, int n_sym,
+                              const float *snr_db, const uint32_t *streams, int n_points, int mode, ofdm_counters *counters_dev);
+int ofdm_mc_sweep_channel_until(ofdm_ctx *ctx, const ofdm_channel *ch, uint32_t seed, uint64_t frame0, int n_sym, const float *snr_db,
+                                int n_snr, int mode, uint64_t target_errors, uint64_t max_bits, long round_frames,
+                                ofdm_counters *out_host, int *rounds_out);
 
 /* ---- multipath extension (BASELINE configs[4]; the reference's only channel is AWGN, OFDM.c:635-655) ----
  * y[n] = sum_l h[l] x[n-l] per frame, n_taps <= 16 (= CP length), applied between the transmitter and
