@@ -103,10 +103,10 @@ cudaError_t allow_smem(ofdm_ctx *ctx, K kernel, size_t bytes)
 // persistent launch geometry: resident blocks per SM (from the occupancy calculator) x SM count,
 // capped by the amount of work
 template <typename K>
-int grid_for(ofdm_ctx *ctx, K kernel, size_t dyn_smem, long work_items_per_block_iter, long work)
+int grid_for(ofdm_ctx *ctx, K kernel, size_t dyn_smem, long work_items_per_block_iter, long work, int threads = kThreads)
 {
     int per_sm = 1;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, dyn_smem) != cudaSuccess || per_sm < 1) per_sm = 1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, dyn_smem) != cudaSuccess || per_sm < 1) per_sm = 1;
     long full = (long)per_sm * ctx->sm_count;
     long need = (work + work_items_per_block_iter - 1) / work_items_per_block_iter;
     long g = need < full ? need : full;
@@ -1034,7 +1034,6 @@ int sweep_points(ofdm_ctx *ctx, const float *frames, const float *g, const float
             if (int st = ofdm_awgn_rx_inject(ctx, frames, g, power, bits, snr_db[i], n_frames, n_sym, mode, counters + i, nullptr)) return st;
         return OFDM_OK;
     }
-    const size_t smem = sweep_smem_bytes();
     const long max_frames = 1L << 30;                      // per launch: the per-lane totals are 32-bit
     for (int s0 = 0; s0 < n_snr; s0 += kMaxSnr) {
         SweepParams p;
@@ -1051,10 +1050,12 @@ int sweep_points(ofdm_ctx *ctx, const float *frames, const float *g, const float
             p.g = g + f0 * 320;
             p.power = power + f0;
             p.tx_bits = bits + f0 * 6;
-            auto launch = [&](auto k) -> int {
+            auto launch = [&](auto k) -> int {                          // the kernel's own block shape
+                constexpr int warps = kSweepWarps;
+                const size_t smem = sweep_smem_bytes(warps);
                 OFDM_CUDA(ctx, allow_smem(ctx, k, smem));
-                int grid = grid_for(ctx, k, smem, kWarpsPerBlock, p.n_frames);
-                k<<<grid, kThreads, smem, ctx->stream>>>(p);
+                const int grid = grid_for(ctx, k, smem, warps, p.n_frames, warps * 32);            // a warp works on one frame at a time
+                k<<<grid, warps * 32, smem, ctx->stream>>>(p);
                 return check_launch(ctx, "k_sweep_lin");
             };
             if (int st = mode == OFDM_MODE_EXACT ? launch(k_sweep_lin<kArithChecked>) : launch(k_sweep_lin<kArithFast>)) return st;

@@ -139,18 +139,17 @@ constexpr float kEvmGuard = 820.f;
 // THR_GIVEN: the caller supplies the decision threshold (rF carries it; rH2 unused) -- the sweep kernel evaluates it as a
 // polynomial in sigma per item instead of from |F|_1 and |G|_1 per point (ofdm_sweep.cuh) -- and has bounded |G|^2 < 1.6e14
 // for the whole frame from the window norms.
+// process_bin_spec_den takes |G|^2 = fma(G.x, G.x, G.y * G.y) and its approximate reciprocal from the caller, which may share
+// them between bins with the same estimate (the sweep kernel: both symbols of a subcarrier).
 template <int LEVEL, bool THR_GIVEN = false>
-__device__ __forceinline__ uint32_t process_bin_spec(float2 F, float2 G, float k, uint32_t txp, float rF, float rH2, float den_min4,
-                                                     float2 &e2, bool &doubt)
+__device__ __forceinline__ uint32_t process_bin_spec_den(float2 F, float2 G, float den, float inv, float k, uint32_t txp, float rF,
+                                                         float rH2, float den_min4, float2 &e2, bool &doubt)
 {
     const float a = F.x, b = F.y, c = G.x, d = G.y;
     // numerator F * conj(G) = (fma(a, c, b*d), fma(b, c, -(a*d))) in two packed instructions
     const float2 pt = __fmul2_rn(make_float2(d, d), make_float2(b, a));
     const float2 S = __ffma2_rn(make_float2(c, c), F, make_float2(pt.x, -pt.y));
     const float sr = S.x, si = S.y;
-    const float den = fmaf(c, c, d * d);
-    float inv;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(inv) : "f"(den));
     const uint32_t sq = txp << 31, sx = (txp ^ (txp >> 1)) << 31;          // IEEE sign bits of the tx Q / I rails
     const uint32_t kb = __float_as_uint(k);
     const uint32_t ei_ = (__float_as_uint(sr) ^ sx ^ kb) >> 31, eq_ = (__float_as_uint(si) ^ sq ^ kb) >> 31;
@@ -174,6 +173,15 @@ __device__ __forceinline__ uint32_t process_bin_spec(float2 F, float2 G, float k
     const float2 D = __ffma2_rn(U, make_float2(k, k), make_float2(__uint_as_float(0xBF3504F3u ^ sx), __uint_as_float(0xBF3504F3u ^ sq)));
     e2 = __ffma2_rn(D, D, e2);
     return ei_ | (eq_ << 8) | ((ei_ & eq_) << 16);
+}
+template <int LEVEL, bool THR_GIVEN = false>
+__device__ __forceinline__ uint32_t process_bin_spec(float2 F, float2 G, float k, uint32_t txp, float rF, float rH2, float den_min4,
+                                                     float2 &e2, bool &doubt)
+{
+    const float den = fmaf(G.x, G.x, G.y * G.y);
+    float inv;
+    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(inv) : "f"(den));
+    return process_bin_spec_den<LEVEL, THR_GIVEN>(F, G, den, inv, k, txp, rF, rH2, den_min4, e2, doubt);
 }
 __device__ __forceinline__ uint32_t process_bin_checked(float2 F, float2 G, float k, uint32_t txp, float rF, float rH2, float den_min4,
                                                         float2 &e2, bool &doubt)

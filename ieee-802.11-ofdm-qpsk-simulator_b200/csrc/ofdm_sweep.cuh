@@ -5,7 +5,8 @@
 // transform is linear, so   FFT(x + sigma g) = FFT(x) + sigma FFT(g):   a frame's four windows (LTS halves, two symbol
 // bodies) and the matching four windows of draws are transformed ONCE, and every SNR point then costs one packed
 // multiply-add per bin it needs -- F = X + sigma N for the lane's three data bins, G = (X_A + X_B) + sigma (N_A + N_B)
-// for their channel estimate (:848) -- followed by the decision stage.  The frame and its draws cross HBM once per
+// for their channel estimates (:848; two per lane: two of its bins are the two symbols of one subcarrier) -- followed by
+// the decision stage.  The frame and its draws cross HBM once per
 // sweep instead of once per SNR point (3100 B per frame instead of 21 x 3100 B), the SNR loop touches neither shared
 // memory nor the LSU, and the per-SNR totals live in registers of the lane that owns the SNR point (as in k_mc_philox).
 //
@@ -59,10 +60,50 @@ __device__ __forceinline__ float modulus_up(float2 z)
     return fmaf(r, 1.000004f, 2e-19f);
 }
 
+// Which bins a lane takes (tools/deal_search.py sweep).  Symbols 0 and 1 of a subcarrier share the channel estimate
+// G = A + B (:848), so each lane takes BOTH symbols of one "pair" bin -- items 0 and 1: one estimate, one |G|^2 and one
+// reciprocal per SNR point for the two -- and one "single" item (item 2) of the 16 other bins: lanes 0..7 of a half-warp
+// symbol 0, lanes 8..15 symbol 1 of the same 8 bins (as c_deal_bin).  The 16 pair bins of a half-warp are distinct mod 16, so
+// their loads from all four tiles are conflict-free; the single items cost one extra wavefront per frame, the least
+// possible (three of them fall on residue 2 mod 16 of the symbol tiles).
+__constant__ unsigned char c_sweep_pair[32] = { 1,  2,  5,  8, 11, 16, 19, 41, 44, 45, 46, 52, 54, 55, 58, 63,
+                                                3,  4, 10, 12, 17, 18, 22, 23, 25, 47, 48, 53, 56, 59, 61, 62};
+__constant__ unsigned char c_sweep_single[16] = { 6, 14, 15, 20, 26, 40, 49, 50,    9, 13, 24, 38, 39, 42, 51, 60};
+
+struct SweepItems {
+    int bin[2];                     // natural FFT bin of estimate 0 (items 0 and 1) and of estimate 1 (item 2)
+    int f_off[3];                   // where the item's bin sits in the symbol tiles fx[2..3]: sym*kWin + bin
+    float k4[3];                    // 1 / sc = 4 * 0.5 L[bin]
+    int word[3];                    // payload word of the frame holding the item's bit pair (sym*3 + d/16)
+    int shift[3];                   // position of the pair in that word
+};
+
+__device__ __forceinline__ SweepItems make_sweep_items(int lane)
+{
+    SweepItems c;
+    c.bin[0] = c_sweep_pair[lane];
+    c.bin[1] = c_sweep_single[(lane >> 4) * 8 + (lane & 7)];
+#pragma unroll
+    for (int t = 0; t < 3; ++t) {
+        const int bin = c.bin[t >> 1], sym = t == 2 ? (lane >> 3) & 1 : t;
+        const int d = c_tab.bin_data[bin];
+        c.f_off[t] = sym * kWin + bin;
+        c.k4[t] = 4.f * (0.5f * (float)c_tab.bin_lts[bin]);
+        c.word[t] = sym * 3 + (d >> 4);
+        c.shift[t] = 2 * (d & 15);
+    }
+    return c;
+}
+
+// Block shape: 2 blocks of 6 warps per SM, in both arithmetics.  168 registers hold three SNR points per pass (nine
+// independent item chains per warp) without spills, and 12 x 13.9 KB of shared memory fit.
+constexpr int kSweepWarps = 6;
+
 template <int ARITH>
-__global__ void __launch_bounds__(kThreads, 2) k_sweep_lin(SweepParams p)
+__global__ void __launch_bounds__(kSweepWarps * 32, 2) k_sweep_lin(SweepParams p)
 {
     constexpr int LEVEL = ARITH == kArithChecked ? 2 : 1;
+    constexpr int kWarps = kSweepWarps;
     extern __shared__ __align__(128) unsigned char s_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, grp = lane >> 3, u = lane & 7;
     const int warp_u = __shfl_sync(0xffffffffu, warp, 0);                  // same value, provably warp-uniform
@@ -70,15 +111,15 @@ __global__ void __launch_bounds__(kThreads, 2) k_sweep_lin(SweepParams p)
     SweepWarp &ws_u = reinterpret_cast<SweepWarp *>(s_raw)[warp_u];
     float2 *tile = ws.tile + grp * kGroupPitch;
     Tw<false> tw; tw.load(u);
-    const ItemConst ic = make_items(lane);
-    const float k4[3] = {4.f * ic.sc[0], 4.f * ic.sc[1], 4.f * ic.sc[2]};     // 1 / sc
+    const SweepItems ic = make_sweep_items(lane);
     constexpr int len = 320;
-    const long stride = (long)gridDim.x * kWarpsPerBlock;
-    const long f_first = (long)blockIdx.x * kWarpsPerBlock + warp_u;
+    const long stride = (long)gridDim.x * kWarps;
+    const long f_first = (long)blockIdx.x * kWarps + warp_u;
     const double q = (double)kQpsk;
     const double ref2_frame = 96.0 * (2.0 * q * q);
     const float inv_ref2 = (float)(1.0 / ref2_frame);
     constexpr uint32_t kBytes = 4 * 512 + 4 * 256;
+    constexpr int kStep = 3;                          // SNR points per pass of the loop below
 
     const uint32_t stage0 = tma::saddr(&ws_u.st[0]);
     const uint32_t bar0 = tma::saddr(&ws_u.bar[0]);
@@ -161,16 +202,20 @@ __global__ void __launch_bounds__(kThreads, 2) k_sweep_lin(SweepParams p)
             if (u == 0) { ws.norm[grp] = ok ? p.radius_scale * rx : inf; ws.norm[4 + grp] = ok ? p.radius_scale * rn : inf; }
         }
         __syncwarp();
-        // the lane's three data bins: everything the SNR loop needs, in registers
+        // the lane's three data bins and their two channel estimates: everything the SNR loop needs, in registers
         const float4 rX = *reinterpret_cast<const float4 *>(ws.norm), rN = *reinterpret_cast<const float4 *>(ws.norm + 4);
         const float rHX = rX.x + rX.y, rHN = rN.x + rN.y;                      // 2 r_H = r_A + r_B
-        float2 FX[3], FN[3], GX[3], GN[3];
-        float c0[3], c1[3], c2[3];
+        float2 FX[3], FN[3], GX[2], GN[2];
+        float c0[3], c1[3], c2[3], hcX[2], hcN[2];
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            const int bin = ic.bin[e];
+            GX[e] = cadd(ws.fx[0][bin], ws.fx[1][bin]);                        // A + B (:848), clean part
+            GN[e] = cadd(ws.fn[0][bin], ws.fn[1][bin]);                        //               noise part
+            if (LEVEL >= 2) { hcX[e] = modulus_up(GX[e]); hcN[e] = modulus_up(GN[e]); }
+        }
 #pragma unroll
         for (int t = 0; t < 3; ++t) {
-            const int bin = ic.bin[t];
-            GX[t] = cadd(ws.fx[0][bin], ws.fx[1][bin]);                        // A + B (:848), clean part
-            GN[t] = cadd(ws.fn[0][bin], ws.fn[1][bin]);                        //               noise part
             FX[t] = (&ws.fx[2][0])[ic.f_off[t]];
             FN[t] = (&ws.fn[2][0])[ic.f_off[t]];
             const bool sym0 = ic.f_off[t] < kWin;                              // the item's symbol
@@ -184,11 +229,11 @@ __global__ void __launch_bounds__(kThreads, 2) k_sweep_lin(SweepParams p)
             // square root, squares that underflow: windows below 1e-15 in norm are never speculated, so 2e-19 covers them).
             if (LEVEL >= 2) {
                 const float faX = modulus_up(FX[t]), faN = modulus_up(FN[t]);
-                const float hcX = modulus_up(GX[t]), hcN = modulus_up(GN[t]);
-                const float A0 = hcX + rHX, A1 = hcN + rHN;
-                c0[t] = fmaf(rFX, A0, fmaf(rHX, faX, 1.2e-7f * (faX * hcX)));
-                c1[t] = fmaf(rFX, A1, fmaf(rFN, A0, fmaf(rHX, faN, fmaf(rHN, faX, 1.2e-7f * fmaf(faX, hcN, faN * hcX)))));
-                c2[t] = fmaf(rFN, A1, fmaf(rHN, faN, 1.2e-7f * (faN * hcN)));
+                const float hX = hcX[t >> 1], hN = hcN[t >> 1];
+                const float A0 = hX + rHX, A1 = hN + rHN;
+                c0[t] = fmaf(rFX, A0, fmaf(rHX, faX, 1.2e-7f * (faX * hX)));
+                c1[t] = fmaf(rFX, A1, fmaf(rFN, A0, fmaf(rHX, faN, fmaf(rHN, faX, 1.2e-7f * fmaf(faX, hN, faN * hX)))));
+                c2[t] = fmaf(rFN, A1, fmaf(rHN, faN, 1.2e-7f * (faN * hN)));
             } else { c0[t] = c1[t] = c2[t] = 0.f; }
         }
         __syncwarp();                                         // everyone holds its items: fx / fn may be overwritten
@@ -196,41 +241,48 @@ __global__ void __launch_bounds__(kThreads, 2) k_sweep_lin(SweepParams p)
         // With S = F conj(G): negating F.x and G.y negates S.x alone, negating F.y and G.y negates S.y alone, so after
         //   F.x ^= (tx I-rail sign ^ sign sc),  F.y ^= (tx Q-rail sign ^ sign sc),  G.y ^= (tx I-rail sign ^ tx Q-rail sign)
         // every item looks as if (+1, +1)/sqrt(2) had been sent through sc = +1/2: a rail error is the sign bit of S, the error
-        // vector is 2 S / |G|^2 - (h, h), and |G|^2, the moduli and the thresholds are unchanged.  The replay reads global memory.
+        // vector is 2 S / |G|^2 - (h, h), and |G|^2, the moduli and the thresholds are unchanged.  Item 1 shares item 0's
+        // estimate: its G.y differs from item 0's by the sign g_rel, applied per point.  The replay reads global memory.
+        uint32_t gq[3];
 #pragma unroll
         for (int t = 0; t < 3; ++t) {
             const uint32_t tp = txw[t] >> ic.shift[t];
-            const uint32_t kb = __float_as_uint(k4[t]) & 0x80000000u;
-            const uint32_t fq = (tp << 31) ^ kb, fi = ((tp ^ (tp >> 1)) << 31) ^ kb, gq = (tp >> 1) << 31;
+            const uint32_t kb = __float_as_uint(ic.k4[t]) & 0x80000000u;
+            const uint32_t fq = (tp << 31) ^ kb, fi = ((tp ^ (tp >> 1)) << 31) ^ kb;
+            gq[t] = (tp >> 1) << 31;
             FX[t] = make_float2(__uint_as_float(__float_as_uint(FX[t].x) ^ fi), __uint_as_float(__float_as_uint(FX[t].y) ^ fq));
             FN[t] = make_float2(__uint_as_float(__float_as_uint(FN[t].x) ^ fi), __uint_as_float(__float_as_uint(FN[t].y) ^ fq));
-            GX[t].y = __uint_as_float(__float_as_uint(GX[t].y) ^ gq);
-            GN[t].y = __uint_as_float(__float_as_uint(GN[t].y) ^ gq);
         }
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            GX[e].y = __uint_as_float(__float_as_uint(GX[e].y) ^ gq[2 * e]);
+            GN[e].y = __uint_as_float(__float_as_uint(GN[e].y) ^ gq[2 * e]);
+        }
+        const uint32_t g_rel = gq[0] ^ gq[1];
         // the noise scale of every SNR point, (float)sqrt((double)(P / snr)) (:647, :651), one (two) per lane
         // (the double square root rounded to float is the correctly rounded float square root: 53 >= 2 * 24 + 2 bits, so the
         // second rounding cannot change the result -- no double arithmetic needed here; the replay takes sigma in double)
         float sig_lo = 0.f, sig_hi = 0.f;
         if (lane < p.n_snr) sig_lo = __fsqrt_rn(__fdiv_rn(P, p.snr_lin[lane]));
         if (p.n_snr > 32 && lane + 32 < p.n_snr) sig_hi = __fsqrt_rn(__fdiv_rn(P, p.snr_lin[lane + 32]));
-        // ... through shared memory (a free noise tile): one broadcast 64-bit load per pair of points in the loop
+        // ... through shared memory (a free noise tile): one broadcast load per pass in the loop.  Three points per pass sit
+        // in one 16-byte slot (points 3i..3i+2 at 4i..4i+2); the slots past n_snr hold 0.
+        auto sig_pos = [](int i) { return (i / 3) * 4 + i % 3; };
         float *sigs = reinterpret_cast<float *>(&ws.fn[1][0]);
-        sigs[lane] = sig_lo; sigs[lane + 32] = sig_hi;
-        if (lane < 2) sigs[64 + lane] = 0.f;
+        sigs[sig_pos(lane)] = sig_lo; sigs[sig_pos(lane + 32)] = sig_hi;
+        if (lane < 2) sigs[sig_pos(64 + lane)] = 0.f;
         __syncwarp();
 
         // ---- SNR loop OFDM.c:1202: one packed multiply-add per value, then the decision stage.  Per-point results
         // {packed rail errors, sum |e|^2} go through 64 words of shared memory (the noise tiles are free by now and the
         // replay does not touch them) so that the owner lanes book them once per frame instead of branching per point.
-        // The warp sums of a point (one REDUX for the packed counts, five dependent shuffles for sum |e|^2) are finished one
-        // iteration late, at the top of the next point's straight-line arithmetic, so that their latency is covered by it.
+        // The loop body has no data-dependent branch: each lane collects its doubtful points in a bit mask, and the warp
+        // resolves them after the loop (one vote per frame), patching their words before they are booked.
         uint2 *res = reinterpret_cast<uint2 *>(&ws.fn[0][0]);
-        // Two SNR points per iteration: six independent decision chains per lane instead of three (the kernel runs four warps per
-        // scheduler, so instruction-level parallelism inside a warp is what covers the rcp / multiply-add latencies).
         const float g2_limit = p.radius_scale * 1.58e6f;        // 8 rH2 / radius_scale (1 + 1e-4) < sqrt(1.6e14); infinite radius: never
         // one SNR point is prepared (noise scale, channel radius, guards) and then evaluated item by item, so that the loop body
-        // below can place the steps of the previous pair's warp reduction between the items
-        struct PointState { float sg, rH2, den_min4; float2 e2v; uint32_t pk; bool doubt; };
+        // below can place the steps of the previous pass's warp reduction between the items
+        struct PointState { float sg, rH2, den_min4; float2 e2v; uint32_t pk; bool doubt; float2 G; float den, inv; };
         auto point_begin = [&](float sg) {
             PointState q;
             q.sg = sg;
@@ -245,105 +297,118 @@ __global__ void __launch_bounds__(kThreads, 2) k_sweep_lin(SweepParams p)
         };
         auto point_item = [&](PointState &q, int t) {                                    // straight-line: no votes, no branches
             const float2 sg2 = make_float2(q.sg, q.sg);
+            if (t != 1) {                                     // items 0 and 2 form their estimate, item 1 uses item 0's
+                q.G = __ffma2_rn(sg2, GN[t >> 1], GX[t >> 1]);
+                q.den = fmaf(q.G.x, q.G.x, q.G.y * q.G.y);
+                asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(q.inv) : "f"(q.den));
+            }
+            const float2 G = t == 1 ? make_float2(q.G.x, __uint_as_float(__float_as_uint(q.G.y) ^ g_rel)) : q.G;
             const float2 F = __ffma2_rn(sg2, FN[t], FX[t]);
-            const float2 G = __ffma2_rn(sg2, GN[t], GX[t]);
             const float thr = fmaf(fmaf(c2[t], q.sg, c1[t]), q.sg, c0[t]);
-            q.pk += process_bin_spec<LEVEL, true>(F, G, 2.f, 0u, thr, q.rH2, q.den_min4, q.e2v, q.doubt);
+            q.pk += process_bin_spec_den<LEVEL, true>(F, G, q.den, q.inv, 2.f, 0u, thr, q.rH2, q.den_min4, q.e2v, q.doubt);
         };
-        auto resolve_point = [&](int si, float sg, uint32_t &pk, float &e2) {             // rare: a doubtful point (whole warp calls)
-            bool replay = true;
-            if (LEVEL >= 2) {
-                // The polynomial is an upper bound of the per-point threshold (triangle inequality): before paying for a replay,
-                // recheck the point with the threshold of its actual |F|, |G|.
-                const float4 qX = *reinterpret_cast<const float4 *>(ws.norm), qN = *reinterpret_cast<const float4 *>(ws.norm + 4);
-                const float2 sg2 = make_float2(sg, sg);
-                const float rH2 = fmaf(sg, rHN, rHX);
-                const float gd = p.evm_guard * rH2, den_min4 = gd * gd;
-                bool doubt2 = false;
-                float2 e2w = make_float2(0.f, 0.f);
-                uint32_t pk2 = 0;
+        // The warp sums of a pass (one REDUX per point for the packed counts, five dependent shuffle steps for the sums |e|^2)
+        // are finished one iteration late, on top of the next pass's nine independent item chains.
+        uint32_t pk_raw[kStep];                                 // the previous pass's per-lane packed counts and sums |e|^2
+        float e2_pend[kStep], red[kStep], red_in[kStep];
 #pragma unroll
-                for (int t = 0; t < 3; ++t) {
-                    const float2 F = __ffma2_rn(sg2, FN[t], FX[t]);
-                    const float2 G = __ffma2_rn(sg2, GN[t], GX[t]);
-                    const bool sym0 = ic.f_off[t] < kWin;
-                    const float rF = fmaf(sg, sym0 ? qN.z : qN.w, sym0 ? qX.z : qX.w);
-                    const float fa = modulus_up(F), hc = modulus_up(G);
-                    const float thr = fmaf(rF, hc + rH2, fmaf(rH2, fa, 1.2e-7f * (fa * hc)));
-                    pk2 += process_bin_spec<LEVEL, true>(F, G, 2.f, 0u, thr, rH2, den_min4, e2w, doubt2);
+        for (int j = 0; j < kStep; ++j) { pk_raw[j] = 0; e2_pend[j] = 0.f; }
+        auto red_issue = [&](int o) {
+#pragma unroll
+            for (int j = 0; j < kStep; ++j) red_in[j] = __shfl_xor_sync(0xffffffffu, red[j], o);
+        };
+        auto red_take = [&]() {
+#pragma unroll
+            for (int j = 0; j < kStep; ++j) red[j] += red_in[j];
+        };
+        uint64_t doubt_mask = 0;                                // the lane's doubtful points
+        for (int si = 0, sk = 0; si < p.n_snr; si += kStep, sk += 4) {
+            uint32_t pk_sum[kStep];
+#pragma unroll
+            for (int j = 0; j < kStep; ++j) { pk_sum[j] = __reduce_add_sync(0xffffffffu, pk_raw[j]); red[j] = e2_pend[j]; }   // the three 8-bit fields stay below 97
+            red_issue(16);
+            PointState q[kStep];
+            const float4 sp = *reinterpret_cast<const float4 *>(sigs + sk);
+            q[0] = point_begin(sp.x); q[1] = point_begin(sp.y); q[2] = point_begin(sp.z);
+            // item n of the pass, then the next shuffle step: offsets 8, 4, 2, 1 after the first four items
+#pragma unroll
+            for (int t = 0; t < 3; ++t) {
+#pragma unroll
+                for (int j = 0; j < kStep; ++j) {
+                    const int n = t * kStep + j;
+                    point_item(q[j], t);
+                    if (n < 4) { red_take(); red_issue(8 >> n); }
+                    else if (n == 4) red_take();
                 }
-                replay = __any_sync(0xffffffffu, doubt2);
-            }
-            if (replay) {                                     // not provably the reference's decisions / EVM: replay exactly
-                const double sigma_d = __dsqrt_rn((double)__fdiv_rn(P, p.snr_lin[si]));
-                const uint2 r = stream_frame_replay<kNoiseInject>(p.in + f * len, p.g + f * len, wb, sigma_d, 0u, 0u, 0ull,
-                                                                  ws.tile, &ws.fx[0][0], p.replayed);
-                pk = r.x; e2 = __uint_as_float(r.y);
-            }
-        };
-        // The warp sums of a pair (one REDUX each for the packed counts, five dependent shuffle steps for the two sums |e|^2,
-        // packed) are finished one iteration late: the REDUXes are issued at the top, the shuffle steps sit between the items of
-        // the next pair (a warp issues in order: a step placed right after the previous one would wait out its ~30 cycles).
-        uint32_t pk_raw0 = 0, pk_raw1 = 0;                      // the previous pair's per-lane packed counts
-        float2 e2_pend = make_float2(0.f, 0.f);
-        // measured: the pair pays for the verified decisions (4.13 -> 3.97 ms); the guarded-EVM-only loop is faster one point at a time
-        constexpr int kStep = LEVEL >= 2 ? 2 : 1;
-        float2 red = make_float2(0.f, 0.f), red_in = red;
-        // `after`: a sum of squares whose sign bit (never set) joins the shuffle's lane mask -- a data dependency that keeps the
-        // assembler from hoisting the whole shuffle chain to the top of the loop body.  Measured: spreading the steps pays in
-        // the one-point loop of the fast arithmetic (3.30 -> 3.19 ms) and costs in the two-point loop (3.79 -> 3.87 ms), where
-        // the hoisted chain leaves the scheduler more freedom for the six item chains.
-        constexpr bool kSpread = LEVEL < 2;
-        auto red_issue = [&](int o, float after) {
-            const int m = kSpread ? o | (int)(__float_as_uint(after) & 0x80000000u) : o;
-            red_in = make_float2(__shfl_xor_sync(0xffffffffu, red.x, m), __shfl_xor_sync(0xffffffffu, red.y, m));
-        };
-        auto red_take = [&]() { red = __fadd2_rn(red, red_in); };
-        for (int si = 0; si < p.n_snr; si += kStep) {
-            const uint32_t pk_sum0 = __reduce_add_sync(0xffffffffu, pk_raw0);            // one REDUX: the three 8-bit fields stay below 97
-            const uint32_t pk_sum1 = kStep == 2 ? __reduce_add_sync(0xffffffffu, pk_raw1) : 0u;
-            red = e2_pend;
-            red_issue(16, 0.f);
-            const bool two = kStep == 2 && si + 1 < p.n_snr;                             // warp-uniform
-            const int sj = two ? si + 1 : si;
-            float sg0, sg1;
-            if (kStep == 2) { const float2 sp = *reinterpret_cast<const float2 *>(sigs + si); sg0 = sp.x; sg1 = sp.y; }   // si even; 0 past the end
-            else { sg0 = sigs[si]; sg1 = 0.f; }
-            PointState q0 = point_begin(sg0), q1 = point_begin(sg1);
-            point_item(q0, 0); red_take(); red_issue(8, q0.e2v.x);
-            point_item(q0, 1); red_take(); red_issue(4, q0.e2v.x);
-            point_item(q0, 2); red_take(); red_issue(2, q0.e2v.x);
-            if (kStep == 2) {
-                point_item(q1, 0); red_take(); red_issue(1, q1.e2v.x);
-                point_item(q1, 1); red_take();
-            } else {
-                red_take(); red_issue(1, 0.f); red_take();
             }
             if (lane == 0 && si > 0) {
-                res[si - kStep] = make_uint2(pk_sum0, __float_as_uint(red.x));
-                if (kStep == 2) res[si - 1] = make_uint2(pk_sum1, __float_as_uint(red.y));
+#pragma unroll
+                for (int j = 0; j < kStep; ++j) res[si - kStep + j] = make_uint2(pk_sum[j], __float_as_uint(red[j]));
             }
-            if (kStep == 2) point_item(q1, 2);
-            uint32_t pk0 = q0.pk, pk1 = q1.pk;
-            float e20 = q0.e2v.x + q0.e2v.y, e21 = q1.e2v.x + q1.e2v.y;
-            if (__any_sync(0xffffffffu, q0.doubt || (kStep == 2 && q1.doubt))) {
-                if (__any_sync(0xffffffffu, q0.doubt)) resolve_point(si, sg0, pk0, e20);
-                if (two && __any_sync(0xffffffffu, q1.doubt)) resolve_point(sj, sg1, pk1, e21);
+            uint32_t bits = 0;
+#pragma unroll
+            for (int j = 0; j < kStep; ++j) {
+                pk_raw[j] = q[j].pk;
+                e2_pend[j] = q[j].e2v.x + q[j].e2v.y;
+                bits |= (uint32_t)q[j].doubt << j;
             }
-            pk_raw0 = pk0; pk_raw1 = pk1;
-            e2_pend = make_float2(e20, e21);
+            doubt_mask |= (uint64_t)bits << si;
         }
         {
-            const uint32_t pk_sum0 = __reduce_add_sync(0xffffffffu, pk_raw0);
-            const uint32_t pk_sum1 = kStep == 2 ? __reduce_add_sync(0xffffffffu, pk_raw1) : 0u;
-            float2 r = e2_pend;
+            const int last = (p.n_snr - 1) / kStep * kStep;                              // first point of the last pass
 #pragma unroll
-            for (int o = 16; o > 0; o >>= 1)
-                r = __fadd2_rn(r, make_float2(__shfl_xor_sync(0xffffffffu, r.x, o), __shfl_xor_sync(0xffffffffu, r.y, o)));
-            const int last = (p.n_snr - 1) & ~(kStep - 1);                               // first point of the last group
-            if (lane == 0) {
-                res[last] = make_uint2(pk_sum0, __float_as_uint(r.x));
-                if (last + 1 < p.n_snr) res[last + 1] = make_uint2(pk_sum1, __float_as_uint(r.y));
+            for (int j = 0; j < kStep; ++j) {
+                const uint32_t pk_sum = __reduce_add_sync(0xffffffffu, pk_raw[j]);
+                float r = e2_pend[j];
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) r += __shfl_xor_sync(0xffffffffu, r, o);
+                if (lane == 0) res[last + j] = make_uint2(pk_sum, __float_as_uint(r));   // up to res[65]: inside the tile
+            }
+        }
+        // ---- the doubtful points (rare): whole warp, one point at a time
+        {
+            if (p.n_snr < 64) doubt_mask &= (1ull << p.n_snr) - 1ull;                    // the points past the end of the last pass
+            uint64_t todo = __reduce_or_sync(0xffffffffu, (uint32_t)doubt_mask);
+            if (p.n_snr > 32) todo |= (uint64_t)__reduce_or_sync(0xffffffffu, (uint32_t)(doubt_mask >> 32)) << 32;
+            __syncwarp();                                                                // lane 0's words are written
+            while (todo != 0) {                                                          // warp-uniform
+                const int si = __ffsll((long long)todo) - 1;
+                todo &= todo - 1;
+                const float sg = sigs[sig_pos(si)];
+                bool replay = true;
+                if (LEVEL >= 2) {
+                    // The polynomial is an upper bound of the per-point threshold (triangle inequality): before paying for a
+                    // replay, recheck the point with the threshold of its actual |F|, |G|.
+                    const float4 qX = *reinterpret_cast<const float4 *>(ws.norm), qN = *reinterpret_cast<const float4 *>(ws.norm + 4);
+                    const float2 sg2 = make_float2(sg, sg);
+                    const float rH2 = fmaf(sg, rHN, rHX);
+                    const float gd = p.evm_guard * rH2, den_min4 = gd * gd;
+                    bool doubt2 = false;
+                    float2 e2w = make_float2(0.f, 0.f);
+                    float2 G;
+#pragma unroll
+                    for (int t = 0; t < 3; ++t) {
+                        if (t != 1) G = __ffma2_rn(sg2, GN[t >> 1], GX[t >> 1]);
+                        const float2 Gt = t == 1 ? make_float2(G.x, __uint_as_float(__float_as_uint(G.y) ^ g_rel)) : G;
+                        const float2 F = __ffma2_rn(sg2, FN[t], FX[t]);
+                        const bool sym0 = ic.f_off[t] < kWin;
+                        const float rF = fmaf(sg, sym0 ? qN.z : qN.w, sym0 ? qX.z : qX.w);
+                        const float fa = modulus_up(F), hc = modulus_up(Gt);
+                        const float thr = fmaf(rF, hc + rH2, fmaf(rH2, fa, 1.2e-7f * (fa * hc)));
+                        process_bin_spec<LEVEL, true>(F, Gt, 2.f, 0u, thr, rH2, den_min4, e2w, doubt2);
+                    }
+                    replay = __any_sync(0xffffffffu, doubt2);
+                }
+                if (replay) {                                 // not provably the reference's decisions / EVM: replay exactly
+                    const double sigma_d = __dsqrt_rn((double)__fdiv_rn(P, p.snr_lin[si]));
+                    const uint2 r = stream_frame_replay<kNoiseInject>(p.in + f * len, p.g + f * len, wb, sigma_d, 0u, 0u, 0ull,
+                                                                      ws.tile, &ws.fx[0][0], p.replayed);
+                    const uint32_t pk_sum = __reduce_add_sync(0xffffffffu, r.x);
+                    float e2 = __uint_as_float(r.y);
+#pragma unroll
+                    for (int o = 16; o > 0; o >>= 1) e2 += __shfl_xor_sync(0xffffffffu, e2, o);
+                    if (lane == 0) res[si] = make_uint2(pk_sum, __float_as_uint(e2));
+                }
             }
         }
         __syncwarp();
@@ -384,6 +449,6 @@ __global__ void __launch_bounds__(kThreads, 2) k_sweep_lin(SweepParams p)
     }
 }
 
-inline size_t sweep_smem_bytes() { return sizeof(SweepWarp) * kWarpsPerBlock; }
+inline size_t sweep_smem_bytes(int warps) { return sizeof(SweepWarp) * warps; }
 
 }  // namespace ofdm
