@@ -7,6 +7,7 @@
 #include <mutex>
 #include <new>
 #include <set>
+#include <type_traits>
 #include <utility>
 
 #include "ofdm_chain.cuh"
@@ -207,139 +208,91 @@ int launch_fft(ofdm_ctx *ctx, const float *in, float *out, long n)
     return check_launch(ctx, "k_fft64");
 }
 
-template <bool EXACT, int NOISE, bool DUMP>
-int launch_rx(ofdm_ctx *ctx, const RxParams &p)
+// persistent launch of a kernel that takes one params struct with n_frames: blocks of `warps` warps, a warp on `per_warp` frames
+// at a time
+template <typename K, typename P>
+int launch_persistent(ofdm_ctx *ctx, K k, int warps, int per_warp, size_t smem, const P &p, const char *name)
 {
-    auto k = k_rx_frames<EXACT, NOISE, DUMP>;
-    int grid = grid_for(ctx, k, 0, kWarpsPerBlock, p.n_frames);
-    k<<<grid, kThreads, 0, ctx->stream>>>(p);
-    return check_launch(ctx, "k_rx_frames");
+    if (smem) OFDM_CUDA(ctx, allow_smem(ctx, k, smem));
+    const int grid = grid_for(ctx, k, smem, (long)warps * per_warp, p.n_frames, warps * 32);
+    k<<<grid, warps * 32, smem, ctx->stream>>>(p);
+    return check_launch(ctx, name);
 }
 
-template <bool EXACT, int NOISE>
-int launch_rx_d(ofdm_ctx *ctx, bool dump, const RxParams &p)
+// runtime noise source / arithmetic -> template argument: f(std::integral_constant<int, value>)
+template <typename F>
+int with_noise(int noise, F f)
 {
-    return dump ? launch_rx<EXACT, NOISE, true>(ctx, p) : launch_rx<EXACT, NOISE, false>(ctx, p);
+    if (noise == kNoiseNone) return f(std::integral_constant<int, kNoiseNone>());
+    if (noise == kNoiseInject) return f(std::integral_constant<int, kNoiseInject>());
+    return f(std::integral_constant<int, kNoisePhilox>());
+}
+template <typename F>
+int with_arith(int arith, F f)
+{
+    if (arith == kArithFast) return f(std::integral_constant<int, kArithFast>());
+    if (arith == kArithChecked) return f(std::integral_constant<int, kArithChecked>());
+    return f(std::integral_constant<int, kArithExact>());
 }
 
-template <int ARITH, int NOISE>
-int launch_stream(ofdm_ctx *ctx, const RxParams &p)
+// EXACT speculates in fp32, verifies and replays exactly (kArithChecked) unless "exact_speculation" = 0
+int arith_of(const ofdm_ctx *ctx, int mode) { return mode != OFDM_MODE_EXACT ? kArithFast : ctx->checked ? kArithChecked : kArithExact; }
+
+enum { kRxQuad, kRxN, kRx2, kRxGeneric };
+
+// receiver family: the streaming kernels need no per-bin outputs and 16-byte aligned buffers (bulk copies); one frame per lane
+// group (k_stream_quad, ofdm_stream.cuh) for the speculating arithmetic, else one frame per warp -- the multi-pass kernel for
+// other frame shapes (or "general_stream" = 1), k_stream_rx2 for the default one
+int rx_family(const ofdm_ctx *ctx, int arith, int noise, const RxParams &p, bool dump)
 {
-    auto k = k_stream_rx2<ARITH, NOISE>;
-    const size_t smem = stream_smem_bytes<NOISE>();
-    OFDM_CUDA(ctx, allow_smem(ctx, k, smem));
-    int grid = grid_for(ctx, k, smem, kWarpsPerBlock, p.n_frames);
-    k<<<grid, kThreads, smem, ctx->stream>>>(p);
-    return check_launch(ctx, "k_stream_rx2");
+    const bool aligned = ((uintptr_t)p.in % 16 == 0) && (noise != kNoiseInject || (uintptr_t)p.g % 16 == 0);
+    if (dump || !aligned || ctx->force_generic) return kRxGeneric;
+    if (ctx->stream_layout == 0 && arith != kArithExact) return kRxQuad;
+    return p.n_sym != 2 || ctx->general_stream ? kRxN : kRx2;
 }
 
-template <int ARITH, int NOISE>
-int launch_stream_n(ofdm_ctx *ctx, const RxParams &p)
+// arithmetic policy of the streaming receivers: the all-exact kernels take the caller's params; the speculating ones get the
+// error radii (ofdm_chain.cuh: kRadius, kChanRadius) and the EVM guard (fast mode: tiny |H| bins are replayed exactly), except
+// fp32 with Philox noise, whose results are statistical: plain fp32 like the fused Monte-Carlo kernel
+RxParams rx_policy(const ofdm_ctx *ctx, int arith, int noise, RxParams q)
 {
-    auto k = k_stream_rxn<ARITH, NOISE>;
-    const size_t smem = stream_smem_bytes<NOISE>();
-    OFDM_CUDA(ctx, allow_smem(ctx, k, smem));
-    int grid = grid_for(ctx, k, smem, kWarpsPerBlock, p.n_frames);
-    k<<<grid, kThreads, smem, ctx->stream>>>(p);
-    return check_launch(ctx, "k_stream_rxn");
-}
-template <int ARITH, int NOISE, int WARPS, bool NSYM2 = false>
-int launch_stream_quad_w(ofdm_ctx *ctx, const RxParams &p)
-{
-    auto k = k_stream_quad<ARITH, NOISE, WARPS, NSYM2>;
-    const size_t smem = quad_smem_bytes<NOISE>(WARPS);
-    OFDM_CUDA(ctx, allow_smem(ctx, k, smem));
-    int per_sm = 1;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, WARPS * 32, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
-    const long full = (long)per_sm * ctx->sm_count, need = (p.n_frames + WARPS * 4 - 1) / (WARPS * 4);      // a warp works on four frames at a time
-    const long grid = need < full ? need : full;
-    k<<<(int)(grid < 1 ? 1 : grid), WARPS * 32, smem, ctx->stream>>>(p);
-    return check_launch(ctx, "k_stream_quad");
-}
-template <int ARITH, int NOISE>
-int launch_stream_quad(ofdm_ctx *ctx, const RxParams &p)
-{
-    if (ctx->stream_warps == 8) return launch_stream_quad_w<ARITH, NOISE, 8>(ctx, p);
-    // the default frame shape has its own build: unit w of a quad always in ring slot w ("general_stream" = 1 keeps the general one)
-    if (p.n_sym == 2 && !ctx->general_stream) return launch_stream_quad_w<ARITH, NOISE, 6, true>(ctx, p);
-    return launch_stream_quad_w<ARITH, NOISE, 6>(ctx, p);
-}
-// error radii of the speculating EXACT kernels (ofdm_chain.cuh: kRadius, kChanRadius)
-void set_radius(ofdm_ctx *ctx, RxParams &q)
-{
+    if (arith == kArithExact) return q;
     q.replayed = ctx->replayed_dev;
-    q.evm_guard = ctx->evm_guard;
+    q.evm_guard = arith == kArithFast && noise == kNoisePhilox ? 0.f : ctx->evm_guard;
     q.radius_scale = ctx->force_replay ? INFINITY : kRadius;
     q.radius_chan = ctx->force_replay ? INFINITY : kChanRadius * sqrtf((float)OFDM_FRAME_LEN(q.n_sym) * q.snr_lin) * 1.001f;
-}
-
-template <int NOISE>
-int launch_stream_n_mode(ofdm_ctx *ctx, int mode, const RxParams &p)
-{
-    if (mode == OFDM_MODE_EXACT && !ctx->checked) return launch_stream_n<kArithExact, NOISE>(ctx, p);
-    RxParams q = p;
-    set_radius(ctx, q);                 // fast mode keeps the EVM guard (tiny |H| bins are replayed exactly), exact mode verifies every decision
-    if (mode != OFDM_MODE_EXACT && NOISE == kNoisePhilox) q.evm_guard = 0.f;      // statistical results: plain fp32 (see launch_rx_any)
-    if (mode != OFDM_MODE_EXACT) return launch_stream_n<kArithFast, NOISE>(ctx, q);
-    return launch_stream_n<kArithChecked, NOISE>(ctx, q);
+    return q;
 }
 
 int launch_rx_any(ofdm_ctx *ctx, int mode, int noise, const RxParams &p)
 {
     const ofdm_rx_dump &d = p.dump;
     const bool dump = d.H || d.eq || d.sliced || d.bits || d.frame_bit_errors || d.frame_evm_lin;
-    // default frame shape without per-bin outputs: the TMA-staged streaming kernel (bulk copies need 16-byte alignment)
-    const bool aligned = ((uintptr_t)p.in % 16 == 0) && (noise != kNoiseInject || (uintptr_t)p.g % 16 == 0);
-    // speculating arithmetic, any frame shape: one frame per lane group (ofdm_stream.cuh)
-    if (!dump && aligned && !ctx->force_generic && ctx->stream_layout == 0 && (mode != OFDM_MODE_EXACT || ctx->checked)) {
-        RxParams q = p;
-        set_radius(ctx, q);             // exact mode verifies every decision; fast mode keeps the EVM guard (tiny |H| bins are replayed exactly)
-        if (mode == OFDM_MODE_EXACT) {
-            if (noise == kNoiseNone) return launch_stream_quad<kArithChecked, kNoiseNone>(ctx, q);
-            if (noise == kNoiseInject) return launch_stream_quad<kArithChecked, kNoiseInject>(ctx, q);
-            return launch_stream_quad<kArithChecked, kNoisePhilox>(ctx, q);
-        }
-        if (noise == kNoiseNone) return launch_stream_quad<kArithFast, kNoiseNone>(ctx, q);
-        if (noise == kNoiseInject) return launch_stream_quad<kArithFast, kNoiseInject>(ctx, q);
-        q.evm_guard = 0.f;              // Philox noise: statistical results, plain fp32 like the fused Monte-Carlo kernel
-        return launch_stream_quad<kArithFast, kNoisePhilox>(ctx, q);
-    }
-    // one frame per warp ("stream_layout" = 1, and the all-exact arithmetic): other frame shapes (or "general_stream" = 1) take
-    // the multi-pass streaming kernel
-    if (!dump && aligned && !ctx->force_generic && (p.n_sym != 2 || ctx->general_stream)) {
-        if (noise == kNoiseNone) return launch_stream_n_mode<kNoiseNone>(ctx, mode, p);
-        if (noise == kNoiseInject) return launch_stream_n_mode<kNoiseInject>(ctx, mode, p);
-        return launch_stream_n_mode<kNoisePhilox>(ctx, mode, p);
-    }
-    if (!dump && p.n_sym == 2 && aligned && !ctx->force_generic) {
-        if (mode == OFDM_MODE_EXACT) {
-            // fp32 speculation + verification + exact replay: same counts as the all-exact kernel (ofdm_chain.cuh)
-            if (ctx->checked) {
-                RxParams q = p;
-                set_radius(ctx, q);
-                if (noise == kNoiseNone) return launch_stream<kArithChecked, kNoiseNone>(ctx, q);
-                if (noise == kNoiseInject) return launch_stream<kArithChecked, kNoiseInject>(ctx, q);
-                return launch_stream<kArithChecked, kNoisePhilox>(ctx, q);
+    const int arith = arith_of(ctx, mode), family = rx_family(ctx, arith, noise, p, dump);
+    if (family == kRxGeneric)           // the generic kernel takes the caller's params in both modes
+        return with_noise(noise, [&](auto n) -> int {
+            constexpr int N = decltype(n)::value;
+            auto go = [&](auto k) { return launch_persistent(ctx, k, kWarpsPerBlock, 1, 0, p, "k_rx_frames"); };
+            if (mode == OFDM_MODE_EXACT) return dump ? go(k_rx_frames<true, N, true>) : go(k_rx_frames<true, N, false>);
+            return dump ? go(k_rx_frames<false, N, true>) : go(k_rx_frames<false, N, false>);
+        });
+    const RxParams q = rx_policy(ctx, arith, noise, p);
+    return with_noise(noise, [&](auto n) -> int {
+        return with_arith(arith, [&](auto a) -> int {
+            constexpr int N = decltype(n)::value, A = decltype(a)::value;
+            if constexpr (A != kArithExact) {
+                if (family == kRxQuad) {
+                    auto go = [&](auto k, int warps) { return launch_persistent(ctx, k, warps, 4, quad_smem_bytes<N>(warps), q, "k_stream_quad"); };
+                    if (ctx->stream_warps == 8) return go(k_stream_quad<A, N, 8>, 8);
+                    // the default frame shape has its own build: unit w of a quad always in ring slot w ("general_stream" = 1 keeps the general one)
+                    if (p.n_sym == 2 && !ctx->general_stream) return go(k_stream_quad<A, N, 6, true>, 6);
+                    return go(k_stream_quad<A, N, 6>, 6);
+                }
             }
-            if (noise == kNoiseNone) return launch_stream<kArithExact, kNoiseNone>(ctx, p);
-            if (noise == kNoiseInject) return launch_stream<kArithExact, kNoiseInject>(ctx, p);
-            return launch_stream<kArithExact, kNoisePhilox>(ctx, p);
-        }
-        RxParams q = p;
-        set_radius(ctx, q);             // the EVM guard of the fast kernels
-        if (noise == kNoiseNone) return launch_stream<kArithFast, kNoiseNone>(ctx, q);
-        if (noise == kNoiseInject) return launch_stream<kArithFast, kNoiseInject>(ctx, q);
-        q.evm_guard = 0.f;              // Philox noise: statistical results, plain fp32 like the fused Monte-Carlo kernel
-        return launch_stream<kArithFast, kNoisePhilox>(ctx, q);
-    }
-    if (mode == OFDM_MODE_EXACT) {
-        if (noise == kNoiseNone) return launch_rx_d<true, kNoiseNone>(ctx, dump, p);
-        if (noise == kNoiseInject) return launch_rx_d<true, kNoiseInject>(ctx, dump, p);
-        return launch_rx_d<true, kNoisePhilox>(ctx, dump, p);
-    }
-    if (noise == kNoiseNone) return launch_rx_d<false, kNoiseNone>(ctx, dump, p);
-    if (noise == kNoiseInject) return launch_rx_d<false, kNoiseInject>(ctx, dump, p);
-    return launch_rx_d<false, kNoisePhilox>(ctx, dump, p);
+            if (family == kRxN) return launch_persistent(ctx, k_stream_rxn<A, N>, kWarpsPerBlock, 1, stream_smem_bytes<N>(), q, "k_stream_rxn");
+            return launch_persistent(ctx, k_stream_rx2<A, N>, kWarpsPerBlock, 1, stream_smem_bytes<N>(), q, "k_stream_rx2");
+        });
+    });
 }
 
 int blocks_1d(long n) { return (int)((n + 255) / 256); }
@@ -1082,120 +1035,64 @@ int ofdm_random_bits(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, long n_frame
 }  // extern "C"
 
 namespace {
-// AWGN Monte-Carlo over a list of points; streams[i] (nullable: i) is the Philox noise stream of point i
-int mc_awgn_core(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, long n_frames, int n_sym, const float *snr_db, const uint32_t *streams,
-                 int n_snr, int mode, ofdm_counters *counters)
+// McParams of the sweep of one frame range over a list of points through channel ch; streams[i] (nullable: i) is the Philox
+// noise stream of point i.  The noise scale inv_sqrt_snr is 1 / sqrt(snr) for the reference channel, sigma / sqrt(P) for the
+// other frame-power ones and sigma itself for Es/N0 and Eb/N0 (kChFixedSigma), each in its own rounding.  Only the reference
+// channel's kernels speculate (error radii, replay counter).
+McParams mc_params(const ofdm_ctx *ctx, const ofdm_channel &ch, uint32_t seed, uint64_t frame0, long n_frames, const float *snr_db,
+                   const uint32_t *streams, int n_snr, ofdm_counters *counters)
 {
-    if (n_sym == 2) {
-        const size_t smem = mc_smem_bytes();
-        const long max_frames = 1L << 30;                  // per launch: the per-lane totals are 32-bit
-        for (long f0 = 0; f0 < n_frames; f0 += max_frames) {
-            McParams p;
-            memset(&p, 0, sizeof p);
-            p.seed = seed; p.frame0 = frame0 + (uint64_t)f0; p.n_frames = n_frames - f0 < max_frames ? n_frames - f0 : max_frames;
-            p.n_snr = n_snr; p.counters = counters;
-            for (int i = 0; i < n_snr; ++i) {
-                p.snr_lin[i] = snr_linear(snr_db[i]); p.inv_sqrt_snr[i] = (float)(1.0 / sqrt((double)p.snr_lin[i]));
-                p.stream[i] = streams ? streams[i] : (uint32_t)i;
-            }
-            p.radius_scale = ctx->force_replay ? INFINITY : kRadius;
-            p.replayed = ctx->replayed_dev;
-            p.evm_guard = ctx->evm_guard;
-            p.radius_chan = ctx->force_replay ? INFINITY : kChanRadius * sqrtf(320.f) * 1.001f;
-            auto launch = [&](auto k) -> int {
-                OFDM_CUDA(ctx, allow_smem(ctx, k, smem));
-                int grid = grid_for(ctx, k, smem, kWarpsPerBlock, p.n_frames);
-                k<<<grid, kThreads, smem, ctx->stream>>>(p);
-                return check_launch(ctx, "k_mc_philox");
-            };
-            // one frame per lane group (k_mc_quad, ofdm_mc_quad.cuh) for the speculating arithmetic; "stream_layout" = 1 and the
-            // all-exact arithmetic keep the one-frame-per-warp kernel
-            auto launch_quad = [&](auto k) -> int {
-                const size_t qsmem = mc_quad_smem_bytes();
-                OFDM_CUDA(ctx, allow_smem(ctx, k, qsmem));
-                int per_sm = 1;
-                if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, kMcQuadWarps * 32, qsmem) != cudaSuccess || per_sm < 1) per_sm = 1;
-                const long full = (long)per_sm * ctx->sm_count, need = (p.n_frames + kMcQuadWarps * 4 - 1) / (kMcQuadWarps * 4);
-                const long grid = need < full ? need : full;
-                k<<<(int)(grid < 1 ? 1 : grid), kMcQuadWarps * 32, qsmem, ctx->stream>>>(p);
-                return check_launch(ctx, "k_mc_quad");
-            };
-            int st;
-            const bool quad = ctx->stream_layout == 0;
-            if (mode != OFDM_MODE_EXACT) st = quad ? launch_quad(k_mc_quad<kArithFast>) : launch(k_mc_philox<kArithFast>);
-            else if (ctx->checked) st = quad ? launch_quad(k_mc_quad<kArithChecked>) : launch(k_mc_philox<kArithChecked>);
-            else st = launch(k_mc_philox<kArithExact>);
-            if (st) return st;
+    const bool reference = is_reference_channel(ch.noise, ch.snr_def), fixed = ch.snr_def != OFDM_SNR_FRAME_POWER;
+    const double rail_share = ch.noise == OFDM_NOISE_COMPLEX ? 0.5 : 1.0;      // complex noise: half of the noise power per rail
+    McParams p;
+    memset(&p, 0, sizeof p);
+    p.seed = seed; p.frame0 = frame0; p.n_frames = n_frames;
+    p.n_snr = n_snr; p.counters = counters; p.n_taps = ch.n_taps;
+    for (int i = 0; i < n_snr; ++i) {
+        if (fixed) p.inv_sqrt_snr[i] = (float)sqrt(rail_share * (double)fixed_noise_power(ch.snr_def, snr_db[i]));
+        else {
+            p.snr_lin[i] = snr_linear(snr_db[i]);
+            p.inv_sqrt_snr[i] = reference ? (float)(1.0 / sqrt((double)p.snr_lin[i])) : (float)sqrt(rail_share / (double)p.snr_lin[i]);
         }
-        return OFDM_OK;
+        p.stream[i] = streams ? streams[i] : (uint32_t)i;
     }
-    // other frame shapes: the same streams through the staged kernels, in chunks that bound the scratch memory (2 GiB of frames)
-    const int len = OFDM_FRAME_LEN(n_sym);
-    long chunk = (2L << 30) / ((long)len * 8);
-    if (chunk < 1024) chunk = 1024;
-    for (long f0 = 0; f0 < n_frames; f0 += chunk) {
-        const long n = n_frames - f0 < chunk ? n_frames - f0 : chunk;
-        void *bits = nullptr, *frames = nullptr, *power = nullptr;
-        if (int st = ensure_scratch(ctx, 4, (size_t)n * n_sym * 3 * sizeof(uint32_t), &bits)) return st;
-        if (int st = ensure_scratch(ctx, 1, (size_t)n * len * 2 * sizeof(float), &frames)) return st;
-        if (int st = ensure_scratch(ctx, 2, (size_t)n * sizeof(float), &power)) return st;
-        if (int st = ofdm_random_bits(ctx, seed, frame0 + (uint64_t)f0, n, n_sym, (uint32_t *)bits)) return st;
-        if (int st = ofdm_tx_frames(ctx, (const uint32_t *)bits, (float *)frames, (float *)power, n, n_sym, mode)) return st;
-        for (int i = 0; i < n_snr; ++i)
-            if (int st = ofdm_awgn_rx_philox(ctx, (const float *)frames, (const float *)power, (const uint32_t *)bits, snr_db[i], seed,
-                                             streams ? streams[i] : (uint32_t)i, frame0 + (uint64_t)f0, n, n_sym, mode, counters + i, nullptr))
-                return st;
+    if (reference) {
+        p.radius_scale = ctx->force_replay ? INFINITY : kRadius;
+        p.replayed = ctx->replayed_dev;
+        p.evm_guard = ctx->evm_guard;
+        p.radius_chan = ctx->force_replay ? INFINITY : kChanRadius * sqrtf(320.f) * 1.001f;
     }
-    return OFDM_OK;
+    return p;
 }
-int mc_multipath_core(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, long n_frames, int n_sym, int n_taps, const float *snr_db,
-                      const uint32_t *streams, int n_snr, int mode, ofdm_counters *counters);
 
-// Channels other than the reference's, fp32, two-symbol frames: k_mc_quad<fast, MP, CH>, the frame built once on chip and the
-// channel + receiver run per point from shared memory.  The noise scale goes through McParams::inv_sqrt_snr: sigma / sqrt(P)
-// for the frame-power definition, sigma itself for Es/N0 and Eb/N0 (kChFixedSigma).
-int mc_channel_fused(ofdm_ctx *ctx, const ofdm_channel &ch, uint32_t seed, uint64_t frame0, long n_frames, const float *snr_db,
-                     const uint32_t *streams, int n_snr, ofdm_counters *counters)
+// fused Monte-Carlo sweep of two-symbol frames, everything on chip: k_mc_quad works on four frames per warp in blocks of
+// kMcQuadWarps warps, k_mc_philox on one frame per warp.  One launch per 2^30 frames: the per-lane totals are 32-bit.
+template <typename K>
+int mc_fused(ofdm_ctx *ctx, K k, bool quad, const McParams &all)
 {
-    const bool cx = ch.noise == OFDM_NOISE_COMPLEX, fixed = ch.snr_def != OFDM_SNR_FRAME_POWER, mp = ch.n_taps > 0;
-    const double rail_share = cx ? 0.5 : 1.0;               // complex noise: half of the noise power per rail
-    const long max_frames = 1L << 30;                      // per launch: the per-lane totals are 32-bit
-    for (long f0 = 0; f0 < n_frames; f0 += max_frames) {
-        McParams p;
-        memset(&p, 0, sizeof p);
-        p.seed = seed; p.frame0 = frame0 + (uint64_t)f0; p.n_frames = n_frames - f0 < max_frames ? n_frames - f0 : max_frames;
-        p.n_snr = n_snr; p.counters = counters; p.n_taps = ch.n_taps;
-        for (int i = 0; i < n_snr; ++i) {
-            if (fixed) p.inv_sqrt_snr[i] = (float)sqrt(rail_share * (double)fixed_noise_power(ch.snr_def, snr_db[i]));
-            else { p.snr_lin[i] = snr_linear(snr_db[i]); p.inv_sqrt_snr[i] = (float)sqrt(rail_share / (double)p.snr_lin[i]); }
-            p.stream[i] = streams ? streams[i] : (uint32_t)i;
-        }
-        auto launch = [&](auto k) -> int {
-            const size_t smem = mp ? mc_quad_mp_smem_bytes() : mc_quad_smem_bytes();
-            OFDM_CUDA(ctx, allow_smem(ctx, k, smem));
-            int per_sm = 1;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, kMcQuadWarps * 32, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
-            const long full = (long)per_sm * ctx->sm_count, need = (p.n_frames + kMcQuadWarps * 4 - 1) / (kMcQuadWarps * 4);
-            const long grid = need < full ? need : full;
-            k<<<(int)(grid < 1 ? 1 : grid), kMcQuadWarps * 32, smem, ctx->stream>>>(p);
-            return check_launch(ctx, "k_mc_quad<channel>");
-        };
-        constexpr int C = kChComplex, F = kChFixedSigma;
-        int st;
-        if (mp) st = cx ? (fixed ? launch(k_mc_quad<kArithFast, true, C | F>) : launch(k_mc_quad<kArithFast, true, C>)) : launch(k_mc_quad<kArithFast, true, F>);
-        else st = cx ? (fixed ? launch(k_mc_quad<kArithFast, false, C | F>) : launch(k_mc_quad<kArithFast, false, C>)) : launch(k_mc_quad<kArithFast, false, F>);
+    const bool mp = all.n_taps > 0;
+    const size_t smem = quad ? (mp ? mc_quad_mp_smem_bytes() : mc_quad_smem_bytes()) : mc_smem_bytes(mp);
+    const long max_frames = 1L << 30;
+    for (long f0 = 0; f0 < all.n_frames; f0 += max_frames) {
+        McParams p = all;
+        p.frame0 = all.frame0 + (uint64_t)f0;
+        p.n_frames = all.n_frames - f0 < max_frames ? all.n_frames - f0 : max_frames;
+        const int st = quad ? launch_persistent(ctx, k, kMcQuadWarps, 4, smem, p, "k_mc_quad")
+                            : launch_persistent(ctx, k, kWarpsPerBlock, 1, smem, p, "k_mc_philox");
         if (st) return st;
     }
     return OFDM_OK;
 }
 
-// Every other shape and EXACT: frames staged in HBM per chunk -- Philox bits, transmitter, [taps], [frame power], then per point
-// the channel (k_awgn_channel) into an OTA buffer and the verified receiver of ofdm_rx_frames on it
-int mc_channel_staged(ofdm_ctx *ctx, const ofdm_channel &ch, uint32_t seed, uint64_t frame0, long n_frames, int n_sym, const float *snr_db,
-                      const uint32_t *streams, int n_snr, int mode, ofdm_counters *counters)
+// staged Monte-Carlo sweep, frames in HBM per chunk of at most 2 GiB: Philox bits, transmitter, [taps, frame power of the faded
+// frames], then per point the reference channel's fused channel + receiver (ofdm_awgn_rx_philox), or another channel
+// (k_awgn_channel) into an OTA buffer and the verified receiver of ofdm_rx_frames on it.  Without taps the frame power comes
+// from the transmitter (its LTS-prefix shortcut).
+int mc_staged(ofdm_ctx *ctx, const ofdm_channel &ch, uint32_t seed, uint64_t frame0, long n_frames, int n_sym, const float *snr_db,
+              const uint32_t *streams, int n_snr, int mode, ofdm_counters *counters)
 {
     const int len = OFDM_FRAME_LEN(n_sym);
-    const bool per_frame = ch.snr_def == OFDM_SNR_FRAME_POWER;
+    const bool reference = is_reference_channel(ch.noise, ch.snr_def), per_frame = ch.snr_def == OFDM_SNR_FRAME_POWER, mp = ch.n_taps > 0;
     long chunk = (2L << 30) / ((long)len * 8);
     if (chunk < 1024) chunk = 1024;
     for (long f0 = 0; f0 < n_frames; f0 += chunk) {
@@ -1204,20 +1101,26 @@ int mc_channel_staged(ofdm_ctx *ctx, const ofdm_channel &ch, uint32_t seed, uint
         void *bits = nullptr, *frames = nullptr, *power = nullptr, *faded = nullptr, *ota = nullptr;
         if (int st = ensure_scratch(ctx, 4, (size_t)n * n_sym * 3 * sizeof(uint32_t), &bits)) return st;
         if (int st = ensure_scratch(ctx, 1, frame_bytes, &frames)) return st;
-        if (int st = ensure_scratch(ctx, 6, frame_bytes, &ota)) return st;
+        if (mp) if (int st = ensure_scratch(ctx, 5, frame_bytes, &faded)) return st;
+        if (!reference) if (int st = ensure_scratch(ctx, 6, frame_bytes, &ota)) return st;
         if (per_frame) if (int st = ensure_scratch(ctx, 2, (size_t)n * sizeof(float), &power)) return st;
         const uint64_t fr0 = frame0 + (uint64_t)f0;
         if (int st = ofdm_random_bits(ctx, seed, fr0, n, n_sym, (uint32_t *)bits)) return st;
-        if (int st = ofdm_tx_frames(ctx, (const uint32_t *)bits, (float *)frames, ch.n_taps > 0 ? nullptr : (float *)power, n, n_sym, mode)) return st;
+        if (int st = ofdm_tx_frames(ctx, (const uint32_t *)bits, (float *)frames, mp ? nullptr : (float *)power, n, n_sym, mode)) return st;
         const float *air = (const float *)frames;
-        if (ch.n_taps > 0) {
-            if (int st = ensure_scratch(ctx, 5, frame_bytes, &faded)) return st;
+        if (mp) {
             if (int st = ofdm_multipath_philox(ctx, air, seed, fr0, ch.n_taps, (float *)faded, nullptr, n, n_sym)) return st;
             air = (const float *)faded;
             if (per_frame) if (int st = frame_power(ctx, air, (float *)power, n, len, mode)) return st;     // power of what goes on the air
         }
         for (int i = 0; i < n_snr; ++i) {
             const uint32_t stream = streams ? streams[i] : (uint32_t)i;
+            if (reference) {
+                if (int st = ofdm_awgn_rx_philox(ctx, air, (const float *)power, (const uint32_t *)bits, snr_db[i], seed, stream, fr0, n, n_sym,
+                                                 mode, counters + i, nullptr))
+                    return st;
+                continue;
+            }
             const int st = per_frame ? launch_awgn_channel(ctx, ch.noise, air, (const float *)power, snr_linear(snr_db[i]), 0.f, seed, stream, fr0,
                                                            (float *)ota, n, len, mode)
                                      : launch_awgn_channel(ctx, ch.noise, air, nullptr, 1.f, fixed_noise_power(ch.snr_def, snr_db[i]), seed, stream,
@@ -1239,7 +1142,8 @@ int ofdm_mc_sweep_philox_dev(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, long
     OFDM_REQUIRE(ctx, n_frames >= 0 && nsym_ok(n_sym) && mode_ok(mode) && n_snr >= 0 && n_snr <= kMaxSnr);
     if (n_frames == 0 || n_snr == 0) return OFDM_OK;
     OFDM_REQUIRE(ctx, snr_db != nullptr && counters != nullptr);
-    return mc_awgn_core(ctx, seed, frame0, n_frames, n_sym, snr_db, nullptr, n_snr, mode, counters);
+    const ofdm_channel ch = {OFDM_NOISE_REAL_RAIL, OFDM_SNR_FRAME_POWER, 0};
+    return ofdm_mc_sweep_channel_dev(ctx, &ch, seed, frame0, n_frames, n_sym, snr_db, nullptr, n_snr, mode, counters);
 }
 
 int ofdm_mc_sweep_points_dev(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, long n_frames, int n_sym, int n_taps, const float *snr_db,
@@ -1257,13 +1161,38 @@ int ofdm_mc_sweep_channel_dev(ofdm_ctx *ctx, const ofdm_channel *ch, uint32_t se
     OFDM_REQUIRE(ctx, n_frames >= 0 && nsym_ok(n_sym) && mode_ok(mode) && n_points >= 0 && n_points <= kMaxSnr);
     if (n_frames == 0 || n_points == 0) return OFDM_OK;
     OFDM_REQUIRE(ctx, snr_db != nullptr && counters != nullptr);
-    if (is_reference_channel(ch->noise, ch->snr_def)) {
-        if (ch->n_taps > 0) return mc_multipath_core(ctx, seed, frame0, n_frames, n_sym, ch->n_taps, snr_db, streams, n_points, mode, counters);
-        return mc_awgn_core(ctx, seed, frame0, n_frames, n_sym, snr_db, streams, n_points, mode, counters);
+    // Fused on chip (two-symbol frames only) or staged through HBM.  The reference channel without taps always fuses two-symbol
+    // frames.  With taps, "multipath_path" chooses (0 = auto); measured per 1 M frames x 21 SNR points: fast 14.8 ms fused vs
+    // 16.9 ms staged, exact 27.3 ms fused vs 20.0 ms staged (the fused kernel runs each frame's exact power chain on one lane, the
+    // staged path one chain per lane).  The other channels fuse only in fp32.
+    const bool reference = is_reference_channel(ch->noise, ch->snr_def), mp = ch->n_taps > 0, fast = mode != OFDM_MODE_EXACT;
+    bool fused = n_sym == 2;
+    if (!reference) fused = fused && fast && !ctx->force_generic;
+    else if (mp) fused = fused && !ctx->force_generic && (ctx->multipath_path == 2 || (ctx->multipath_path == 0 && fast));
+    if (!fused) return mc_staged(ctx, *ch, seed, frame0, n_frames, n_sym, snr_db, streams, n_points, mode, counters);
+    const McParams p = mc_params(ctx, *ch, seed, frame0, n_frames, snr_db, streams, n_points, counters);
+    auto quad = [&](auto k) { return mc_fused(ctx, k, true, p); };
+    if (!reference) {                   // k_mc_quad<fast, MP, CH>: the channel is a compile-time parameter
+        constexpr int C = kChComplex, F = kChFixedSigma;
+        const bool cx = ch->noise == OFDM_NOISE_COMPLEX, fixed = ch->snr_def != OFDM_SNR_FRAME_POWER;
+        auto go = [&](auto m) -> int {
+            constexpr bool M = decltype(m)::value;
+            return cx ? (fixed ? quad(k_mc_quad<kArithFast, M, C | F>) : quad(k_mc_quad<kArithFast, M, C>)) : quad(k_mc_quad<kArithFast, M, F>);
+        };
+        return mp ? go(std::true_type()) : go(std::false_type());
     }
-    if (mode != OFDM_MODE_EXACT && n_sym == 2 && !ctx->force_generic)
-        return mc_channel_fused(ctx, *ch, seed, frame0, n_frames, snr_db, streams, n_points, counters);
-    return mc_channel_staged(ctx, *ch, seed, frame0, n_frames, n_sym, snr_db, streams, n_points, mode, counters);
+    // one frame per lane group (k_mc_quad, ofdm_mc_quad.cuh) for the speculating arithmetic without taps and for fp32 with taps;
+    // "stream_layout" = 1 and the all-exact arithmetic keep the one-frame-per-warp kernel
+    return with_arith(arith_of(ctx, mode), [&](auto a) -> int {
+        constexpr int A = decltype(a)::value;
+        if constexpr (A == kArithFast) {
+            if (ctx->stream_layout == 0) return mp ? quad(k_mc_quad<A, true>) : quad(k_mc_quad<A>);
+        }
+        if constexpr (A == kArithChecked) {
+            if (ctx->stream_layout == 0 && !mp) return quad(k_mc_quad<A>);
+        }
+        return mp ? mc_fused(ctx, k_mc_philox<A, true>, false, p) : mc_fused(ctx, k_mc_philox<A>, false, p);
+    });
 }
 
 int ofdm_mc_sweep_until(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, int n_sym, int n_taps, const float *snr_db, int n_snr, int mode,
@@ -1373,86 +1302,10 @@ int ofdm_mc_sweep_multipath_dev(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, l
     OFDM_REQUIRE(ctx, n_frames >= 0 && nsym_ok(n_sym) && mode_ok(mode) && n_snr >= 0 && n_snr <= kMaxSnr && n_taps >= 1 && n_taps <= kMaxTaps);
     if (n_frames == 0 || n_snr == 0) return OFDM_OK;
     OFDM_REQUIRE(ctx, snr_db != nullptr && counters != nullptr);
-    return mc_multipath_core(ctx, seed, frame0, n_frames, n_sym, n_taps, snr_db, nullptr, n_snr, mode, counters);
+    const ofdm_channel ch = {OFDM_NOISE_REAL_RAIL, OFDM_SNR_FRAME_POWER, n_taps};
+    return ofdm_mc_sweep_channel_dev(ctx, &ch, seed, frame0, n_frames, n_sym, snr_db, nullptr, n_snr, mode, counters);
 }
 
-}  // extern "C"
-
-namespace {
-int mc_multipath_core(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, long n_frames, int n_sym, int n_taps, const float *snr_db,
-                      const uint32_t *streams, int n_snr, int mode, ofdm_counters *counters)
-{
-    // Measured per 1 M frames x 21 SNR points: fast 14.8 ms fused vs 16.9 ms staged; exact 27.3 ms fused vs 20.0 ms staged (the
-    // fused kernel runs each frame's exact power chain on one lane, the staged path one chain per lane).
-    const bool fused = ctx->multipath_path == 2 || (ctx->multipath_path == 0 && mode == OFDM_MODE_FAST);
-    if (n_sym == 2 && !ctx->force_generic && fused) {
-        // default frame shape: everything on chip (k_mc_philox<., true>), same totals as the staged path below
-        const size_t smem = mc_smem_bytes(true);
-        const long max_frames = 1L << 30;
-        for (long f0 = 0; f0 < n_frames; f0 += max_frames) {
-            McParams p;
-            memset(&p, 0, sizeof p);
-            p.seed = seed; p.frame0 = frame0 + (uint64_t)f0; p.n_frames = n_frames - f0 < max_frames ? n_frames - f0 : max_frames;
-            p.n_snr = n_snr; p.counters = counters; p.n_taps = n_taps;
-            for (int i = 0; i < n_snr; ++i) {
-                p.snr_lin[i] = snr_linear(snr_db[i]); p.inv_sqrt_snr[i] = (float)(1.0 / sqrt((double)p.snr_lin[i]));
-                p.stream[i] = streams ? streams[i] : (uint32_t)i;
-            }
-            p.radius_scale = ctx->force_replay ? INFINITY : kRadius;
-            p.replayed = ctx->replayed_dev;
-            p.evm_guard = ctx->evm_guard;
-            p.radius_chan = ctx->force_replay ? INFINITY : kChanRadius * sqrtf(320.f) * 1.001f;
-            auto launch = [&](auto k) -> int {
-                OFDM_CUDA(ctx, allow_smem(ctx, k, smem));
-                int grid = grid_for(ctx, k, smem, kWarpsPerBlock, p.n_frames);
-                k<<<grid, kThreads, smem, ctx->stream>>>(p);
-                return check_launch(ctx, "k_mc_philox<multipath>");
-            };
-            int st;
-            if (mode != OFDM_MODE_EXACT && ctx->stream_layout == 0) {           // one frame per lane group (k_mc_quad<fast, multipath>)
-                auto k = k_mc_quad<kArithFast, true>;
-                const size_t qsmem = mc_quad_mp_smem_bytes();
-                OFDM_CUDA(ctx, allow_smem(ctx, k, qsmem));
-                int per_sm = 1;
-                if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, kMcQuadWarps * 32, qsmem) != cudaSuccess || per_sm < 1) per_sm = 1;
-                const long full = (long)per_sm * ctx->sm_count, need = (p.n_frames + kMcQuadWarps * 4 - 1) / (kMcQuadWarps * 4);
-                const long grid = need < full ? need : full;
-                k<<<(int)(grid < 1 ? 1 : grid), kMcQuadWarps * 32, qsmem, ctx->stream>>>(p);
-                st = check_launch(ctx, "k_mc_quad<multipath>");
-            }
-            else if (mode != OFDM_MODE_EXACT) st = launch(k_mc_philox<kArithFast, true>);
-            else if (ctx->checked) st = launch(k_mc_philox<kArithChecked, true>);
-            else st = launch(k_mc_philox<kArithExact, true>);
-            if (st) return st;
-        }
-        return OFDM_OK;
-    }
-    // staged: frames in HBM once per chunk (two frame buffers of 2 GiB each)
-    const int len = OFDM_FRAME_LEN(n_sym);
-    long chunk = (2L << 30) / ((long)len * 8);
-    if (chunk < 1024) chunk = 1024;
-    for (long f0 = 0; f0 < n_frames; f0 += chunk) {
-        const long n = n_frames - f0 < chunk ? n_frames - f0 : chunk;
-        void *bits = nullptr, *frames = nullptr, *power = nullptr, *faded = nullptr;
-        if (int st = ensure_scratch(ctx, 4, (size_t)n * n_sym * 3 * sizeof(uint32_t), &bits)) return st;
-        if (int st = ensure_scratch(ctx, 1, (size_t)n * len * 2 * sizeof(float), &frames)) return st;
-        if (int st = ensure_scratch(ctx, 5, (size_t)n * len * 2 * sizeof(float), &faded)) return st;
-        if (int st = ensure_scratch(ctx, 2, (size_t)n * sizeof(float), &power)) return st;
-        const uint64_t fr0 = frame0 + (uint64_t)f0;
-        if (int st = ofdm_random_bits(ctx, seed, fr0, n, n_sym, (uint32_t *)bits)) return st;
-        if (int st = ofdm_tx_frames(ctx, (const uint32_t *)bits, (float *)frames, nullptr, n, n_sym, mode)) return st;
-        if (int st = ofdm_multipath_philox(ctx, (const float *)frames, seed, fr0, n_taps, (float *)faded, nullptr, n, n_sym)) return st;
-        if (int st = frame_power(ctx, (const float *)faded, (float *)power, n, len, mode)) return st;      // power of what goes on the air
-        for (int i = 0; i < n_snr; ++i)
-            if (int st = ofdm_awgn_rx_philox(ctx, (const float *)faded, (const float *)power, (const uint32_t *)bits, snr_db[i], seed,
-                                             streams ? streams[i] : (uint32_t)i, fr0, n, n_sym, mode, counters + i, nullptr))
-                return st;
-    }
-    return OFDM_OK;
-}
-}  // namespace
-
-extern "C" {
 
 // ------------------------------------------------------------------ pulse shaping (SURVEY 8(f) rank 1)
 int ofdm_rrc_tx(ofdm_ctx *ctx, const float *frames, float *out, long n_frames, int frame_len)

@@ -112,7 +112,7 @@ static void report_rate(const char *what, int n_gpus, long frames, int n_sym, in
 static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, const ofdm_channel *ch, const float *SNR, int n_snr, int mode,
                            ofdm_counters *totals, unsigned long long target_errors, unsigned long long max_bits, long round_frames, int round_reduce_host)
 {
-    const int n_taps = ch->n_taps, reference = ch->noise == OFDM_NOISE_REAL_RAIL && ch->snr_def == OFDM_SNR_FRAME_POWER;
+    const int n_taps = ch->n_taps;
     ofdm_ctx *ctxs[8] = {0};
     ofdm_ctx *ctx = NULL;
     void *cnt[8], *ints[8], *dbls[8];
@@ -131,9 +131,7 @@ static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, co
     NCHECK(ncclCommInitAll(comms, n_gpus, devs));
     for (int d = 0; d < n_gpus; ++d) {                      /* first use of a kernel on a device loads it: keep that out of the timing */
         ctx = ctxs[d];
-        if (!reference) CHECK(ofdm_mc_sweep_channel_dev(ctx, ch, seed, 0, 256, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)cnt[d]));
-        else if (n_taps > 0) CHECK(ofdm_mc_sweep_multipath_dev(ctx, seed, 0, 256, n_sym, n_taps, SNR, n_snr, mode, (ofdm_counters *)cnt[d]));
-        else CHECK(ofdm_mc_sweep_philox_dev(ctx, seed, 0, 256, n_sym, SNR, n_snr, mode, (ofdm_counters *)cnt[d]));
+        CHECK(ofdm_mc_sweep_channel_dev(ctx, ch, seed, 0, 256, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)cnt[d]));
         CHECK(ofdm_memset_dev(ctx, cnt[d], 0, sizeof(ofdm_counters) * (size_t)n_snr));
         CHECK(ofdm_counters_pack(ctx, (const ofdm_counters *)cnt[d], n_snr, (uint64_t *)ints[d], (double *)dbls[d]));
         CHECK(ofdm_ctx_sync(ctx));
@@ -219,9 +217,7 @@ static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, co
         long base = frames / n_gpus, rem = frames % n_gpus;
         long lo = d * base + (d < rem ? d : rem), n = base + (d < rem ? 1 : 0);
         ctx = ctxs[d];
-        if (!reference) CHECK(ofdm_mc_sweep_channel_dev(ctx, ch, seed, (uint64_t)lo, n, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)cnt[d]));
-        else if (n_taps > 0) CHECK(ofdm_mc_sweep_multipath_dev(ctx, seed, (uint64_t)lo, n, n_sym, n_taps, SNR, n_snr, mode, (ofdm_counters *)cnt[d]));
-        else CHECK(ofdm_mc_sweep_philox_dev(ctx, seed, (uint64_t)lo, n, n_sym, SNR, n_snr, mode, (ofdm_counters *)cnt[d]));
+        CHECK(ofdm_mc_sweep_channel_dev(ctx, ch, seed, (uint64_t)lo, n, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)cnt[d]));
         CHECK(ofdm_counters_pack(ctx, (const ofdm_counters *)cnt[d], n_snr, (uint64_t *)ints[d], (double *)dbls[d]));
     }
     NCHECK(ncclGroupStart());
@@ -373,7 +369,7 @@ int main(int argc, char **argv)
         const double dt = now_s() - t0;
         fprintf(stderr, "until-sweep: %d rounds of %ld frames, %llu frame-points x %d symbols on 1 GPU(s) in %.3f s = %.3e data symbols/s\n", rounds, round_frames,
                 fp, n_sym, dt, (double)fp * n_sym / dt);
-    } else if (frames > 1 && !reference_channel) {     /* another channel, with or without taps */
+    } else if (frames > 1) {                           /* Monte-Carlo sweep through the channel; --taps: configs[4]'s multipath taps */
         void *d_cnt = NULL;
         CHECK(ofdm_dev_alloc(ctx, &d_cnt, sizeof(ofdm_counters) * (size_t)n_snr));
         CHECK(ofdm_memset_dev(ctx, d_cnt, 0, sizeof(ofdm_counters) * (size_t)n_snr));
@@ -381,22 +377,8 @@ int main(int argc, char **argv)
         CHECK(ofdm_mc_sweep_channel_dev(ctx, &ch, seed, 0, frames, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)d_cnt));
         CHECK(ofdm_memcpy_d2h(ctx, totals, d_cnt, sizeof(ofdm_counters) * (size_t)n_snr));
         CHECK(ofdm_ctx_sync(ctx));
-        report_rate("channel sweep", 1, frames, n_sym, n_snr, now_s() - t0);
+        report_rate(!reference_channel ? "channel sweep" : n_taps > 0 ? "multipath sweep" : "sweep", 1, frames, n_sym, n_snr, now_s() - t0);
         ofdm_dev_free(ctx, d_cnt);
-    } else if (frames > 1 && n_taps > 0) {             /* configs[4]: per-frame random multipath taps */
-        void *d_cnt = NULL;
-        CHECK(ofdm_dev_alloc(ctx, &d_cnt, sizeof(ofdm_counters) * (size_t)n_snr));
-        CHECK(ofdm_memset_dev(ctx, d_cnt, 0, sizeof(ofdm_counters) * (size_t)n_snr));
-        const double t0 = now_s();
-        CHECK(ofdm_mc_sweep_multipath_dev(ctx, seed, 0, frames, n_sym, n_taps, SNR, n_snr, mode, (ofdm_counters *)d_cnt));
-        CHECK(ofdm_memcpy_d2h(ctx, totals, d_cnt, sizeof(ofdm_counters) * (size_t)n_snr));
-        CHECK(ofdm_ctx_sync(ctx));
-        report_rate("multipath sweep", 1, frames, n_sym, n_snr, now_s() - t0);
-        ofdm_dev_free(ctx, d_cnt);
-    } else if (frames > 1) {
-        const double t0 = now_s();
-        CHECK(ofdm_mc_sweep_philox(ctx, seed, 0, frames, n_sym, SNR, n_snr, mode, totals));
-        report_rate("sweep", 1, frames, n_sym, n_snr, now_s() - t0);
     } else {
         uint8_t *bits = NULL;
         CHECK(encode_message(message, &bits, &n_sym));

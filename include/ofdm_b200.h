@@ -114,7 +114,8 @@ int ofdm_ctx_sync(ofdm_ctx *ctx);
  *                            (default 16, the proven bound is 7; 2^28 = the reference's operations on every sample; same floats)
  *   "fused_sweep"       = 0  injected-noise sweeps launch one channel+receiver kernel per SNR point instead of the all-SNR
  *                            kernel (default 1; same totals)
- *   "multipath_path"    = 0  ofdm_mc_sweep_multipath_dev picks the faster of its two implementations per mode (default);
+ *   "multipath_path"    = 0  Monte-Carlo sweeps of the reference channel with taps (ofdm_mc_sweep_multipath_dev and the
+ *                            other sweeps given taps) pick the faster of their two implementations per mode (default);
  *                       = 1  frames staged in HBM (TX, fading, power, one receiver kernel per SNR point);
  *                       = 2  the fused on-chip kernel; both give the same totals */
 int ofdm_ctx_set_option(ofdm_ctx *ctx, const char *name, int value);
