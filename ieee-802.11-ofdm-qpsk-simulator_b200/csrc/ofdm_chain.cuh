@@ -189,6 +189,125 @@ __device__ __forceinline__ uint32_t process_bin_checked(float2 F, float2 G, floa
     return process_bin_spec<2>(F, G, k, txp, rF, rH2, den_min4, e2, doubt);
 }
 
+// ---- the exact replay: what turns "verified fp32" into the reference's counts --------------------------------------------
+// Where the replayed frame comes from.  n_sym(): its data symbols; window(n0): the lane group's 64 samples starting at frame
+// sample n0; draws(n0): their injected draws (kNoiseInject); words(sym, ...): the three payload words of data symbol sym.
+template <int NSYM = 0>             // NSYM > 0: the symbol count is known at compile time (no code for the passes after pass 0)
+struct GlobalFrame {                // the streaming and sweep kernels: frame, draws and payload words in HBM
+    const float2 *x; const float *g; const uint32_t *bits;
+    int n_sym_any;                  // NSYM == 0: the symbol count
+    __device__ int n_sym() const { return NSYM > 0 ? NSYM : n_sym_any; }
+    __device__ const float2 *window(int n0) const { return x + n0; }
+    __device__ const float *draws(int n0) const { return g + n0; }
+    __device__ void words(int sym, uint32_t, uint64_t, uint32_t (&w)[3]) const { w[0] = bits[3 * sym]; w[1] = bits[3 * sym + 1]; w[2] = bits[3 * sym + 2]; }
+};
+struct McFrame {                    // the Monte-Carlo kernels: a two-symbol frame built in shared memory, payload from Philox domain 1
+    const float2 *w;                // the lane group's window of pass 0: LTS half (s_ltsx) or symbol body (faded for multipath)
+    __device__ static constexpr int n_sym() { return 2; }
+    __device__ const float2 *window(int) const { return w; }
+    __device__ const float *draws(int) const { return nullptr; }
+    __device__ void words(int sym, uint32_t seed, uint64_t fr, uint32_t (&w)[3]) const
+    {
+        const uint4 b = Philox::run(make_uint4((uint32_t)fr, (uint32_t)(fr >> 32), (uint32_t)sym, kDomainBits), seed, 0u);
+        w[0] = b.x; w[1] = b.y; w[2] = b.z;
+    }
+};
+struct ReplayTotals {               // one lane's share of a replayed frame, not yet reduced over the warp
+    uint32_t i, q, both; float e2;
+    __device__ uint32_t packed() const { return i | (q << 8) | (both << 16); }      // two-symbol frames: at most 3 per lane
+};
+
+// One frame of any length in the reference's arithmetic (the rare path of the speculating kernels): the same draws, exact
+// channel, exact transform, exact decision stage.  Pass 0 = {LTS half 1, LTS half 2, symbol 0, symbol 1} with the 96 data bins
+// dealt out by make_items (all 32 lanes busy; the speculating kernels of two-symbol frames add their float terms in this order),
+// then four symbols per pass, each lane deciding the natural bins u + 8j of its group's symbol against the LTS kept in `lts`.
+// tile_w: the warp's transform tiles (kWarpTile); lts: [2][kWin].
+template <int NOISE, class Src>
+__device__ __noinline__ ReplayTotals frame_replay_exact(Src src, double sigma_d, uint32_t seed, uint32_t stream, uint64_t frame_id,
+                                                        float2 *tile_w, float2 *lts, unsigned long long *replayed)
+{
+    const int lane = threadIdx.x & 31, grp = lane >> 3, u = lane & 7;
+    const int n_sym = src.n_sym();
+    const int n_pass = 1 + (n_sym > 2 ? (n_sym + 1) / 4 : 0);
+    ReplayTotals t = {0u, 0u, 0u, 0.f};
+    for (int pass = 0; pass < n_pass; ++pass) {
+        const int sym = pass == 0 ? grp - 2 : 2 + (pass - 1) * 4 + grp;     // < 0: LTS half
+        const bool active = sym < n_sym;
+        const int n0 = sym < 0 ? 32 + 64 * grp : 176 + 80 * sym;           // Channel_Estimation :837-838, CP strip :1028
+        float z[8];
+        if (NOISE == kNoisePhilox && active) {
+            const int base = window_block_base(n0) + u;
+            float za[4], zb[4];
+            philox_normals4(seed, stream, frame_id, (uint32_t)base, kDomainNoise, za);
+            philox_normals4(seed, stream, frame_id, (uint32_t)(base + 8), kDomainNoise, zb);
+#pragma unroll
+            for (int m = 0; m < 4; ++m) { z[m] = za[m]; z[4 + m] = zb[m]; }
+        }
+        float2 v[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            const int m = slot_m<true>(i);
+            float2 sm = make_float2(0.f, 0.f);
+            if (active) {
+                sm = src.window(n0)[u + 8 * m];
+                if (NOISE == kNoiseInject) sm.x = add_noise<true>(sm.x, src.draws(n0)[u + 8 * m], sigma_d, 0.f);
+                if (NOISE == kNoisePhilox) sm.x = add_noise<true>(sm.x, z[m], sigma_d, 0.f);
+            }
+            v[i] = sm;
+        }
+        {                                   // the exact twiddles live only here (see below)
+            Tw<true> tw; tw.load(u);
+            fft64<true>(v, tw, tile_w + grp * kGroupPitch, u);
+        }
+        // The lane's bit pairs, two bits each, are fetched after the transform, whose registers are free by then.  The routine's
+        // register peak decides how much its callers spill around the call (-Xptxas -v).
+        const int isym = (lane >> 3) & 1;                                     // pass 0: the symbol of all three of the lane's items
+        uint32_t txp = 0;
+        if (pass == 0 ? isym < n_sym : active) {
+            uint32_t w[3];
+            src.words(pass == 0 ? isym : sym, seed, frame_id, w);
+            if (pass == 0) {
+                const ItemConst ic = make_items(lane);
+#pragma unroll
+                for (int k = 0; k < 3; ++k) {
+                    const int wi = ic.word[k] - 3 * isym;
+                    txp |= (((wi == 0 ? w[0] : wi == 1 ? w[1] : w[2]) >> ic.shift[k]) & 3u) << (2 * k);
+                }
+            } else {
+#pragma unroll
+                for (int j = 0; j < 8; ++j) txp |= bit_pair(w[0], w[1], w[2], c_tab.bin_data[u + 8 * j]) << (2 * j);
+            }
+        }
+        uint32_t pk = 0;
+        if (pass == 0) {                    // exchange: LTS groups publish A / B, data groups publish F
+            float2 *dst = grp < 2 ? lts + grp * kWin : tile_w + (grp - 2) * kWin;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) dst[u + 8 * j] = v[j];
+            __syncwarp();
+            const ItemConst ic = make_items(lane);
+#pragma unroll
+            for (int k = 0; k < 3; ++k) {
+                const float2 A = lts[ic.bin[k]], B = lts[kWin + ic.bin[k]];
+                const float2 Hh = make_float2(__fmul_rn(__fadd_rn(A.x, B.x), ic.sc[k]), __fmul_rn(__fadd_rn(A.y, B.y), ic.sc[k]));  // :848
+                pk += process_bin_hot<true>(tile_w[ic.f_off[k]], Hh, ic.sc[k], txp >> (2 * k), isym < n_sym, t.e2);
+            }
+        } else if (active) {
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                const int d = c_tab.bin_data[u + 8 * j];                       // < 0: null / pilot
+                const float sc = 0.5f * (float)c_tab.bin_lts[u + 8 * j];
+                const float2 A = lts[u + 8 * j], B = lts[kWin + u + 8 * j];
+                const float2 Hh = make_float2(__fmul_rn(__fadd_rn(A.x, B.x), sc), __fmul_rn(__fadd_rn(A.y, B.y), sc));      // :848
+                pk += process_bin_hot<true>(v[j], Hh, sc, txp >> (2 * j), d >= 0, t.e2);
+            }
+        }
+        t.i += pk & 0xFFu; t.q += (pk >> 8) & 0xFFu; t.both += pk >> 16;
+        __syncwarp();
+    }
+    if (lane == 0 && replayed != nullptr) atomicAdd(replayed, 1ull);
+    return t;
+}
+
 struct McParams {
     uint32_t seed;
     uint64_t frame0;
@@ -212,45 +331,6 @@ struct WarpShared {
     float2 body[2][kWin];           // the frame's two symbol bodies in time (skewed windows)
     uint2 res[kMaxSnr];             // per SNR point of the current frame: {packed rail errors, sum |e|^2}, booked once per frame
 };
-
-// Replay of one (frame, SNR point) of the Monte-Carlo kernel in the reference's arithmetic (rare path of kArithChecked):
-// the same Philox draws, exact channel, exact transform, exact decision stage.  txp3: the lane's three bit pairs,
-// two bits each.  Returns {packed rail errors, lane's sum |e|^2}, not yet reduced over the warp.
-__device__ __noinline__ uint2 mc_point_replay(const float2 *src, double sigma_d, uint32_t seed, uint32_t stream, uint64_t fr,
-                                              uint32_t txp3, float2 *ws_tile, float2 *ws_lts, unsigned long long *replayed)
-{
-    const int lane = threadIdx.x & 31, grp = lane >> 3, u = lane & 7;
-    Tw<true> tw; tw.load(u);
-    const ItemConst ic = make_items(lane);
-    const int blk_base = (grp < 2 ? 8 + 16 * grp : 44 + 20 * (grp - 2)) + u;
-    float za[4], zb[4];
-    philox_normals4(seed, stream, fr, (uint32_t)blk_base, kDomainNoise, za);
-    philox_normals4(seed, stream, fr, (uint32_t)(blk_base + 8), kDomainNoise, zb);
-    float2 r[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        const int m = slot_m<true>(i);
-        float2 s = src[u + 8 * m];
-        s.x = add_noise<true>(s.x, m < 4 ? za[m & 3] : zb[m & 3], sigma_d, 0.f);
-        r[i] = s;
-    }
-    fft64<true>(r, tw, ws_tile + grp * kGroupPitch, u);
-    float2 *dst = grp < 2 ? ws_lts + grp * kWin : ws_tile + (grp - 2) * kWin;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) dst[u + 8 * j] = r[j];
-    __syncwarp();
-    float e2 = 0.f;
-    uint32_t pk = 0;
-#pragma unroll
-    for (int t = 0; t < 3; ++t) {
-        const float2 A = ws_lts[ic.bin[t]], B = ws_lts[kWin + ic.bin[t]];
-        const float2 Hh = make_float2(__fmul_rn(__fadd_rn(A.x, B.x), ic.sc[t]), __fmul_rn(__fadd_rn(A.y, B.y), ic.sc[t]));
-        pk += item_eval<true>(ws_tile[ic.f_off[t]], Hh, ic.sc[t], (txp3 >> (2 * t)) & 3u, e2);
-    }
-    __syncwarp();
-    if (lane == 0 && replayed != nullptr) atomicAdd(replayed, 1ull);
-    return make_uint2(pk, __float_as_uint(e2));
-}
 
 // ARITH: kArithFast, kArithExact, or kArithChecked = exact transmitter, power and channel, receiver speculated in fp32
 // with verified decisions and exact replay (see above) -- the totals of kArithExact.
@@ -481,9 +561,8 @@ __global__ void __launch_bounds__(kThreads, 2) k_mc_philox(McParams p)
                 e2 = e2v.x + e2v.y;
                 __syncwarp();
                 if (__any_sync(0xffffffffu, doubt)) {             // not provably the reference's decisions / EVM: replay exactly
-                    const uint32_t txp3 = (txp[0] & 3u) | ((txp[1] & 3u) << 2) | ((txp[2] & 3u) << 4);
-                    const uint2 rr = mc_point_replay(src, sigma_d, p.seed, stream, fr, txp3, ws.tile, &ws.lts[0][0], p.replayed);
-                    pk = rr.x; e2 = __uint_as_float(rr.y);
+                    const ReplayTotals rr = frame_replay_exact<kNoisePhilox>(McFrame{src}, sigma_d, p.seed, stream, fr, ws.tile, &ws.lts[0][0], p.replayed);
+                    pk = rr.packed(); e2 = rr.e2;
                 }
             } else {
 #pragma unroll
@@ -734,53 +813,6 @@ template <bool WITH_DRAWS> struct alignas(16) StreamWarp {
     uint64_t bar[kStages];
     float radius[4];                // kArithChecked: error radius of each window's transform (see below)
 };
-// Replay of one frame in the reference's arithmetic (rare path of kArithChecked): samples straight from global
-// memory, exact channel, exact transform, exact decision stage.  Returns {packed rail errors, lane's sum |e|^2}.
-template <int NOISE>
-__device__ __noinline__ uint2 stream_frame_replay(const float2 *frame, const float *draws, const uint32_t *wb, double sigma_d,
-                                                  uint32_t seed, uint32_t stream, uint64_t frame_id, float2 *ws_tile, float2 *ws_lts,
-                                                  unsigned long long *replayed)
-{
-    const int lane = threadIdx.x & 31, grp = lane >> 3, u = lane & 7;
-    Tw<true> tw; tw.load(u);
-    const ItemConst ic = make_items(lane);
-    const int n0 = grp == 0 ? 32 : grp == 1 ? 96 : grp == 2 ? 176 : 256;
-    float z[8];
-    if (NOISE == kNoisePhilox) {                                  // the same draws as the speculated pass (window block layout)
-        const int blk_base = (grp < 2 ? 8 + 16 * grp : 44 + 20 * (grp - 2)) + u;
-        float za[4], zb[4];
-        philox_normals4(seed, stream, frame_id, (uint32_t)blk_base, kDomainNoise, za);
-        philox_normals4(seed, stream, frame_id, (uint32_t)(blk_base + 8), kDomainNoise, zb);
-#pragma unroll
-        for (int m = 0; m < 4; ++m) { z[m] = za[m]; z[4 + m] = zb[m]; }
-    }
-    float2 v[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        const int m = slot_m<true>(i), n = n0 + u + 8 * m;
-        float2 smp = frame[n];
-        if (NOISE == kNoiseInject) smp.x = add_noise<true>(smp.x, draws[n], sigma_d, 0.f);
-        if (NOISE == kNoisePhilox) smp.x = add_noise<true>(smp.x, z[m], sigma_d, 0.f);
-        v[i] = smp;
-    }
-    fft64<true>(v, tw, ws_tile + grp * kGroupPitch, u);
-    float2 *dst = grp < 2 ? ws_lts + grp * kWin : ws_tile + (grp - 2) * kWin;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) dst[u + 8 * j] = v[j];
-    __syncwarp();
-    float e2 = 0.f;
-    uint32_t pk = 0;
-#pragma unroll
-    for (int t = 0; t < 3; ++t) {
-        const float2 A = ws_lts[ic.bin[t]], B = ws_lts[kWin + ic.bin[t]];
-        const float2 Hh = make_float2(__fmul_rn(__fadd_rn(A.x, B.x), ic.sc[t]), __fmul_rn(__fadd_rn(A.y, B.y), ic.sc[t]));   // :848
-        pk += item_eval<true>(ws_tile[ic.f_off[t]], Hh, ic.sc[t], wb[ic.word[t]] >> ic.shift[t], e2);
-    }
-    __syncwarp();
-    if (lane == 0 && replayed != nullptr) atomicAdd(replayed, 1ull);
-    return make_uint2(pk, __float_as_uint(e2));
-}
-
 // resident blocks per SM the launch bounds ask for.  Round 1 ran the fp32 kernels without injected draws at three (80 registers);
 // with the EVM guard and its replay call they need more than 80 registers (spills made three blocks 2x slower than two).
 static_assert(sizeof(StreamStage<false>) % 16 == 0 && sizeof(StreamStage<true>) % 16 == 0 && sizeof(StreamWarp<false>) % 16 == 0, "stage alignment");
@@ -923,10 +955,9 @@ __global__ void __launch_bounds__(kThreads, stream_blocks_per_sm<ARITH, NOISE>()
                 f_e2 = e2v.x + e2v.y;
                 __syncwarp();
                 if (__any_sync(0xffffffffu, doubt)) {             // not provably the reference's decisions: replay exactly
-                    const uint2 r = stream_frame_replay<NOISE>(p.in + f * len, NOISE == kNoiseInject ? p.g + f * len : nullptr,
-                                                               p.tx_bits + f * 6, sigma_d, p.seed, p.stream, p.frame0 + (uint64_t)f,
-                                                               ws.tile, &ws.lts[0][0], p.replayed);
-                    pk = r.x; f_e2 = __uint_as_float(r.y);
+                    const GlobalFrame<2> fr = {p.in + f * len, NOISE == kNoiseInject ? p.g + f * len : nullptr, p.tx_bits + f * 6};
+                    const ReplayTotals r = frame_replay_exact<NOISE>(fr, sigma_d, p.seed, p.stream, p.frame0 + (uint64_t)f, ws.tile, &ws.lts[0][0], p.replayed);
+                    pk = r.packed(); f_e2 = r.e2;
                 }
             } else {
 #pragma unroll
@@ -982,93 +1013,7 @@ __global__ void __launch_bounds__(kThreads, stream_blocks_per_sm<ARITH, NOISE>()
 // The streaming receiver for any number of data symbols.  A frame is a sequence of passes through the same ring:
 // pass 0 = {LTS half 1, LTS half 2, symbol 0, symbol 1} exactly as k_stream_rx2, then four symbols per pass against the
 // channel estimate left in shared memory by pass 0, their 192 data bins dealt out six per lane.  kArithChecked marks a frame whose
-// decisions are not all provably the reference's and replays it whole (sweep_frame_replay) after its last pass.
-struct SweepLane {                  // per-lane constants for the natural bins u + 8j
-    uint32_t dlo, dhi;              // data index bytes (>= 0x80: null / pilot), j = 0..3 and 4..7
-    uint32_t lneg, lnul;            // bit j: L < 0, L == 0
-};
-__device__ __forceinline__ SweepLane make_sweep_lane(int u)
-{
-    SweepLane c = {0u, 0u, 0u, 0u};
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-        const uint32_t d = (uint32_t)(uint8_t)c_tab.bin_data[u + 8 * j];
-        if (j < 4) c.dlo |= d << (8 * j); else c.dhi |= d << (8 * (j - 4));
-        const int l = c_tab.bin_lts[u + 8 * j];
-        c.lneg |= (uint32_t)(l < 0) << j; c.lnul |= (uint32_t)(l == 0) << j;
-    }
-    return c;
-}
-struct SweepFrame {                 // one frame's inputs
-    const float2 *x; const float *g; const uint32_t *bits;
-    int n_sym; double sigma_d; uint32_t seed, stream; uint64_t frame_id;
-    unsigned long long *replayed;
-};
-struct SweepTotals { uint32_t i, q, both; float e2; };
-
-// One frame in the reference's arithmetic, samples straight from global memory (the replay of k_stream_rxn<kArithChecked>).
-template <int NOISE>
-__device__ __noinline__ SweepTotals sweep_frame_replay(SweepFrame fr, float2 *tile_w, float2 *lts /* [2][kWin] */)
-{
-    const int lane = threadIdx.x & 31, grp = lane >> 3, u = lane & 7;
-    float2 *tile = tile_w + grp * kGroupPitch;
-    Tw<true> tw; tw.load(u);
-    const SweepLane sl = make_sweep_lane(u);
-    const int n_sym = fr.n_sym;
-    const int n_pass = 1 + (n_sym > 2 ? (n_sym + 1) / 4 : 0);
-    SweepTotals t = {0u, 0u, 0u, 0.f};
-    unsigned long long *replayed = fr.replayed;
-    for (int pass = 0; pass < n_pass; ++pass) {
-        const int sym = pass == 0 ? grp - 2 : 2 + (pass - 1) * 4 + grp;     // < 0: LTS half
-        const bool active = sym < n_sym;
-        const int n0 = sym < 0 ? 32 + 64 * grp : 176 + 80 * sym;           // Channel_Estimation :837-838, CP strip :1028
-        float z[8];
-        if (NOISE == kNoisePhilox && active) {
-            const int base = window_block_base(n0) + u;
-            float za[4], zb[4];
-            philox_normals4(fr.seed, fr.stream, fr.frame_id, (uint32_t)base, kDomainNoise, za);
-            philox_normals4(fr.seed, fr.stream, fr.frame_id, (uint32_t)(base + 8), kDomainNoise, zb);
-#pragma unroll
-            for (int m = 0; m < 4; ++m) { z[m] = za[m]; z[4 + m] = zb[m]; }
-        }
-        float2 v[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            const int m = slot_m<true>(i);
-            float2 sm = make_float2(0.f, 0.f);
-            if (active) {
-                sm = fr.x[n0 + u + 8 * m];
-                if (NOISE == kNoiseInject) sm.x = add_noise<true>(sm.x, fr.g[n0 + u + 8 * m], fr.sigma_d, 0.f);
-                if (NOISE == kNoisePhilox) sm.x = add_noise<true>(sm.x, z[m], fr.sigma_d, 0.f);
-            }
-            v[i] = sm;
-        }
-        fft64<true>(v, tw, tile, u);
-        if (pass == 0 && grp < 2) {
-#pragma unroll
-            for (int j = 0; j < 8; ++j) lts[grp * kWin + u + 8 * j] = v[j];
-        }
-        __syncwarp();
-        if (sym >= 0 && active) {
-            const uint32_t *w = fr.bits + sym * 3;
-            const uint32_t w0 = w[0], w1 = w[1], w2 = w[2];
-            uint32_t pk = 0;
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                const uint32_t d = ((j < 4 ? sl.dlo : sl.dhi) >> (8 * (j & 3))) & 0xFFu;
-                const float sc = ((sl.lnul >> j) & 1u) ? 0.f : (((sl.lneg >> j) & 1u) ? -0.5f : 0.5f);
-                const float2 A = lts[u + 8 * j], B = lts[kWin + u + 8 * j];
-                const float2 Hh = make_float2(__fmul_rn(__fadd_rn(A.x, B.x), sc), __fmul_rn(__fadd_rn(A.y, B.y), sc));      // :848
-                pk += process_bin_hot<true>(v[j], Hh, sc, bit_pair(w0, w1, w2, (int)d), d < 0x80u, t.e2);
-            }
-            t.i += pk & 0xFFu; t.q += (pk >> 8) & 0xFFu; t.both += pk >> 16;
-        }
-        __syncwarp();
-    }
-    if (lane == 0 && replayed != nullptr) atomicAdd(replayed, 1ull);
-    return t;
-}
-
+// decisions are not all provably the reference's and replays it whole (frame_replay_exact) after its last pass.
 template <int ARITH, int NOISE>
 __global__ void __launch_bounds__(kThreads, 2) k_stream_rxn(RxParams p)
 {
@@ -1283,10 +1228,8 @@ __global__ void __launch_bounds__(kThreads, 2) k_stream_rxn(RxParams p)
             }
             if (SPEC) {
                 if (__any_sync(0xffffffffu, doubt)) {             // not provably the reference's decisions: replay the frame exactly
-                    SweepFrame fr;
-                    fr.x = p.in + f * len; fr.g = NOISE == kNoiseInject ? p.g + f * len : nullptr; fr.bits = fbits; fr.n_sym = n_sym;
-                    fr.sigma_d = sigma_d; fr.seed = p.seed; fr.stream = p.stream; fr.frame_id = p.frame0 + (uint64_t)f; fr.replayed = p.replayed;
-                    const SweepTotals t = sweep_frame_replay<NOISE>(fr, ws.tile, &ws.lts[0][0]);
+                    const GlobalFrame<> fr = {p.in + f * len, NOISE == kNoiseInject ? p.g + f * len : nullptr, fbits, n_sym};
+                    const ReplayTotals t = frame_replay_exact<NOISE>(fr, sigma_d, p.seed, p.stream, p.frame0 + (uint64_t)f, ws.tile, &ws.lts[0][0], p.replayed);
                     f_i = t.i; f_q = t.q; f_both = t.both; f_e2 = t.e2;
                 }
             }

@@ -12,7 +12,7 @@
 // Streams, draws and their assignment to samples are those of k_mc_philox (DESIGN.md "Philox streams"): the sweep's result
 // depends only on (seed, global frame index), not on which kernel, warp or lane group produced it.  kArithChecked = exact
 // transmitter, power and noise scale, receiver speculated in fp32 with every decision verified and doubtful (frame, point)s
-// replayed in the reference's arithmetic by the whole warp (mc_point_replay): the totals of the all-exact kernel.  The error
+// replayed in the reference's arithmetic by the whole warp (frame_replay_exact): the totals of the all-exact kernel.  The error
 // radii are those of k_stream_quad (halves added in time: 269 u S + 2 chan <= r_A + r_B).
 #pragma once
 #include "ofdm_stream.cuh"
@@ -326,21 +326,12 @@ __global__ void __launch_bounds__(kMcQuadWarps * 32, 2) k_mc_quad(McParams p)
                 while (dm != 0u) {                                // warp-uniform: the whole warp replays one (frame, point) at a time
                     const int g = (__ffs((int)dm) - 1) >> 3;
                     dm &= ~(0xFFu << (8 * g));
-                    const ItemConst ic = make_items(lane);
-                    const uint32_t wsrc[6] = {fw[0][0] ^ ql.flip0, fw[0][1] ^ ql.flip1, fw[0][2] ^ ql.flip2, fw[1][0] ^ ql.flip0, fw[1][1] ^ ql.flip1, fw[1][2] ^ ql.flip2};
-                    uint32_t txp3 = 0;
-#pragma unroll
-                    for (int k = 0; k < 6; ++k) {
-                        const uint32_t w = __shfl_sync(0xffffffffu, wsrc[k], 8 * g);
-#pragma unroll
-                        for (int t = 0; t < 3; ++t) if (ic.word[t] == k) txp3 |= ((w >> ic.shift[t]) & 3u) << (2 * t);
-                    }
                     const float Pg = __shfl_sync(0xffffffffu, P, 8 * g);
                     const double sigma_d = __dsqrt_rn((double)__fdiv_rn(Pg, p.snr_lin[si]));
-                    const float2 *src = grp < 2 ? s_ltsx + grp * kWin : ws.body[g] + (grp - 2) * kWin;
-                    const uint2 rr = mc_point_replay(src, sigma_d, p.seed, stream, p.frame0 + (uint64_t)(4 * qd + g), txp3, ws.tile, &ws.lts[0][0], p.replayed);
-                    const uint32_t tpk = __reduce_add_sync(0xffffffffu, rr.x);
-                    float te2 = __uint_as_float(rr.y);
+                    const McFrame fr = {grp < 2 ? s_ltsx + grp * kWin : ws.body[g] + (grp - 2) * kWin};
+                    const ReplayTotals rr = frame_replay_exact<kNoisePhilox>(fr, sigma_d, p.seed, stream, p.frame0 + (uint64_t)(4 * qd + g), ws.tile, &ws.lts[0][0], p.replayed);
+                    const uint32_t tpk = __reduce_add_sync(0xffffffffu, rr.packed());
+                    float te2 = rr.e2;
 #pragma unroll
                     for (int o = 16; o > 0; o >>= 1) te2 += __shfl_xor_sync(0xffffffffu, te2, o);
                     if (grp == g) { pk = u == 0 ? tpk : 0u; e2 = u == 0 ? te2 : 0.f; }

@@ -390,12 +390,9 @@ __global__ void __launch_bounds__(WARPS * 32, 2) k_stream_quad(RxParams p)
                 const int g = (__ffs((int)dm) - 1) >> 3;
                 dm &= ~(0xFFu << (8 * g));
                 const long fr_id = f0 + g;
-                SweepFrame fr;
-                fr.x = p.in + fr_id * len; fr.g = DRAWS ? p.g + fr_id * len : nullptr; fr.bits = p.tx_bits + fr_id * ((long)n_sym * 3);
-                fr.n_sym = n_sym;
-                fr.sigma_d = NOISE != kNoiseNone ? __dsqrt_rn((double)__fdiv_rn(p.power[fr_id], p.snr_lin)) : 0.0;
-                fr.seed = p.seed; fr.stream = p.stream; fr.frame_id = p.frame0 + (uint64_t)fr_id; fr.replayed = p.replayed;
-                const SweepTotals t = sweep_frame_replay<NOISE>(fr, ws.tile, &ws.lts[0][0]);
+                const GlobalFrame<NSYM2 ? 2 : 0> fr = {p.in + fr_id * len, DRAWS ? p.g + fr_id * len : nullptr, p.tx_bits + fr_id * ((long)n_sym * 3), n_sym};
+                const double sigma_d = NOISE != kNoiseNone ? __dsqrt_rn((double)__fdiv_rn(p.power[fr_id], p.snr_lin)) : 0.0;
+                const ReplayTotals t = frame_replay_exact<NOISE>(fr, sigma_d, p.seed, p.stream, p.frame0 + (uint64_t)fr_id, ws.tile, &ws.lts[0][0], p.replayed);
                 const uint32_t ti = __reduce_add_sync(0xffffffffu, t.i), tq = __reduce_add_sync(0xffffffffu, t.q);
                 const uint32_t tb = __reduce_add_sync(0xffffffffu, t.both);
                 float te2 = t.e2;

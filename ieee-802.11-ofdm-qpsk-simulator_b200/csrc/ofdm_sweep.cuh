@@ -12,7 +12,7 @@
 //
 // Exactness (OFDM_MODE_EXACT = kArithChecked) is the scheme of ofdm_chain.cuh: fp32 speculation, every rail decision
 // verified against a rigorous bound on |speculated - reference|, doubtful (frame, SNR point)s replayed in the
-// reference's arithmetic from global memory (stream_frame_replay).  The bound for this kernel, per bin of a window with
+// reference's arithmetic from global memory (frame_replay_exact, ofdm_chain.cuh).  The bound for this kernel, per bin of a window with
 // clean samples x, draws g and S = |x|_2 + sigma |g|_2 (u = 2^-24; |X_k| <= 8 |x|_2 by Cauchy-Schwarz):
 //   speculated  fl(X~ + sigma_f N~):  116 u |x|_2 + 116 u sigma |g|_2  (the two fp32 transforms, ofdm_chain.cuh)
 //                                     + 8 u sigma |g|_2  (sigma_f = fl32(sigma_d))  + 8 u S  (rounding of the multiply-add)
@@ -401,10 +401,10 @@ __global__ void __launch_bounds__(kSweepWarps * 32, 2) k_sweep_lin(SweepParams p
                 }
                 if (replay) {                                 // not provably the reference's decisions / EVM: replay exactly
                     const double sigma_d = __dsqrt_rn((double)__fdiv_rn(P, p.snr_lin[si]));
-                    const uint2 r = stream_frame_replay<kNoiseInject>(p.in + f * len, p.g + f * len, wb, sigma_d, 0u, 0u, 0ull,
-                                                                      ws.tile, &ws.fx[0][0], p.replayed);
-                    const uint32_t pk_sum = __reduce_add_sync(0xffffffffu, r.x);
-                    float e2 = __uint_as_float(r.y);
+                    const GlobalFrame<2> fr = {p.in + f * len, p.g + f * len, wb};
+                    const ReplayTotals r = frame_replay_exact<kNoiseInject>(fr, sigma_d, 0u, 0u, 0ull, ws.tile, &ws.fx[0][0], p.replayed);
+                    const uint32_t pk_sum = __reduce_add_sync(0xffffffffu, r.packed());
+                    float e2 = r.e2;
 #pragma unroll
                     for (int o = 16; o > 0; o >>= 1) e2 += __shfl_xor_sync(0xffffffffu, e2, o);
                     if (lane == 0) res[si] = make_uint2(pk_sum, __float_as_uint(e2));

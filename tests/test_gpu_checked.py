@@ -21,18 +21,34 @@ def knobs(ofdm):
     ofdm.set_option("exact_speculation", 1)
     ofdm.set_option("force_replay", 0)
     ofdm.set_option("force_generic_rx", 0)
+    ofdm.set_option("stream_layout", 0)
+    ofdm.set_option("multipath_path", 0)
+
+
+# name, arithmetic, exact_speculation, force_replay, force_generic_rx, stream_layout.  The forced replays run every caller of the
+# exact replay: one frame per lane group (k_stream_quad), one frame per warp (k_stream_rx2 / k_stream_rxn), and the fp32
+# kernels, whose EVM guard replays through the same routine.
+VARIANTS = (("checked", "exact", 1, 0, 0, 0), ("all_exact", "exact", 0, 0, 0, 0), ("replay_all", "exact", 1, 1, 0, 0),
+            ("replay_all_per_warp", "exact", 1, 1, 0, 1), ("fast_replay_all", "fast", 1, 1, 0, 0),
+            ("fast_replay_all_per_warp", "fast", 1, 1, 0, 1), ("generic", "exact", 0, 0, 1, 0))
 
 
 def run_variants(ofdm, pkg, fn):
-    """fn() -> Counters; returns {variant: (Counters, replayed frames)}"""
+    """fn(mode) -> Counters; returns {variant: (Counters, replayed frames)}.  Every forced variant replays every frame and
+    gives the all-exact kernel's integer totals."""
     out = {}
-    for name, spec, force, generic in (("checked", 1, 0, 0), ("all_exact", 0, 0, 0), ("replay_all", 1, 1, 0), ("generic", 0, 0, 1)):
+    for name, arith, spec, force, generic, layout in VARIANTS:
         ofdm.set_option("exact_speculation", spec)
         ofdm.set_option("force_replay", force)
         ofdm.set_option("force_generic_rx", generic)
+        ofdm.set_option("stream_layout", layout)
         ofdm.replayed_frames(reset=True)
-        c = fn()
+        c = fn(pkg.MODE_EXACT if arith == "exact" else pkg.MODE_FAST)
         out[name] = (c, ofdm.replayed_frames())
+    ofdm.set_option("stream_layout", 0)
+    for name, (c, replayed) in out.items():
+        if "replay_all" in name:
+            assert ints(c) == ints(out["all_exact"][0]) and replayed == c.frames, name
     return out
 
 
@@ -44,7 +60,7 @@ def test_counts_match_oracle_and_all_exact(knobs, pkg, port, snr):
     packed = ofdm.to_dev(pkg.pack_bits_host(bits).view(np.int32))
     gd = ofdm.to_dev(g)
     frames, power = ofdm.tx_frames(packed, n_sym, pkg.MODE_EXACT)
-    res = run_variants(ofdm, pkg, lambda: ofdm.awgn_rx_inject(frames, gd, packed, snr, n_sym, pkg.MODE_EXACT, power=power)[0])
+    res = run_variants(ofdm, pkg, lambda mode: ofdm.awgn_rx_inject(frames, gd, packed, snr, n_sym, mode, power=power)[0])
     acc = port.chain(bits, g, n_sym, snr)
     want = (acc.bit_errors, acc.bits, acc.frames_in_error, acc.rail_errors, acc.frames)
     for name, (c, _) in res.items():
@@ -68,7 +84,7 @@ def test_large_batch_low_snr(knobs, pkg):
     g = torch.randn((n, 320), dtype=torch.float32, device=ofdm.device, generator=gen)
     frames, power = ofdm.tx_frames(packed.view(n, 6), n_sym, pkg.MODE_EXACT)
     for snr in (0.0, 2.0):
-        res = run_variants(ofdm, pkg, lambda: ofdm.awgn_rx_inject(frames, g, packed, snr, n_sym, pkg.MODE_EXACT, power=power)[0])
+        res = run_variants(ofdm, pkg, lambda mode: ofdm.awgn_rx_inject(frames, g, packed, snr, n_sym, mode, power=power)[0])
         want = ints(res["all_exact"][0])
         assert ints(res["checked"][0]) == want and ints(res["replay_all"][0]) == want and ints(res["generic"][0]) == want
         assert 0 < res["checked"][1] < n // 10
@@ -95,7 +111,7 @@ def test_decisions_on_the_boundary(knobs, pkg, port, angle):
     ota = rotate_bodies(port.tx_frames(bits, n_sym), angle)
     want = port.rx_frames(ota, bits, n_sym)
     od = ofdm.to_dev(ota)
-    res = run_variants(ofdm, pkg, lambda: ofdm.rx_frames(od, packed, n_sym, pkg.MODE_EXACT)[0])
+    res = run_variants(ofdm, pkg, lambda mode: ofdm.rx_frames(od, packed, n_sym, mode)[0])
     for name, (c, _) in res.items():
         assert c.bit_errors == int(want["bit_errors"].sum()), name
         assert c.rail_errors == int(want["rail_errors"].sum()), name
@@ -128,7 +144,7 @@ def test_degenerate_frames(knobs, pkg, port):
     finite = [i for i in range(64) if i not in (7, 8)]
     packed = ofdm.to_dev(pkg.pack_bits_host(bits).view(np.int32))
     od = ofdm.to_dev(ota)
-    res = run_variants(ofdm, pkg, lambda: ofdm.rx_frames(od, packed, n_sym, pkg.MODE_EXACT)[0])
+    res = run_variants(ofdm, pkg, lambda mode: ofdm.rx_frames(od, packed, n_sym, mode)[0])
     want = ints(res["generic"][0])
     for name, (c, _) in res.items():
         assert ints(c) == want, name
@@ -194,7 +210,7 @@ def test_philox_noise_checked(knobs, pkg, snr):
     gen = torch.Generator(device=ofdm.device); gen.manual_seed(5)
     packed = torch.randint(-2**31, 2**31 - 1, (n * 6,), dtype=torch.int32, device=ofdm.device, generator=gen)
     frames, power = ofdm.tx_frames(packed, n_sym, pkg.MODE_EXACT)
-    res = run_variants(ofdm, pkg, lambda: ofdm.awgn_rx_philox(frames, packed, snr, 77, 3, 1000, n_sym, pkg.MODE_EXACT, power=power)[0])
+    res = run_variants(ofdm, pkg, lambda mode: ofdm.awgn_rx_philox(frames, packed, snr, 77, 3, 1000, n_sym, mode, power=power)[0])
     want = ints(res["all_exact"][0])
     for name, (c, _) in res.items():
         assert ints(c) == want, name
@@ -208,8 +224,13 @@ def test_multipath_sweep_checked(knobs, pkg):
     a = ofdm.mc_sweep_multipath(9, 0, 60_000, 2, 6, snr, pkg.MODE_EXACT)
     ofdm.set_option("exact_speculation", 0)
     b = ofdm.mc_sweep_multipath(9, 0, 60_000, 2, 6, snr, pkg.MODE_EXACT)
-    for x, y in zip(a, b):
-        assert ints(x) == ints(y)
+    # the fused verified kernel (k_mc_philox with taps) with every (frame, point) replayed
+    ofdm.set_option("exact_speculation", 1); ofdm.set_option("multipath_path", 2); ofdm.set_option("force_replay", 1)
+    ofdm.replayed_frames(reset=True)
+    c = ofdm.mc_sweep_multipath(9, 0, 60_000, 2, 6, snr, pkg.MODE_EXACT)
+    assert ofdm.replayed_frames() == 60_000 * len(snr)
+    for x, y, z in zip(a, b, c):
+        assert ints(x) == ints(y) == ints(z)
         assert abs(x.sum_err2 - y.sum_err2) <= 1e-5 * y.sum_err2
 
 
@@ -219,19 +240,22 @@ def test_monte_carlo_kernel_checked(knobs, pkg):
     snr = [float(s) for s in range(-2, 19, 2)]
     n = 150_000
     runs = {}
-    for name, spec, force in (("checked", 1, 0), ("all_exact", 0, 0), ("replay_all", 1, 1)):
-        ofdm.set_option("exact_speculation", spec); ofdm.set_option("force_replay", force)
+    # replay_all: k_mc_quad (one frame per lane group); replay_all_per_warp: k_mc_philox
+    for name, spec, force, layout in (("checked", 1, 0, 0), ("all_exact", 0, 0, 0), ("replay_all", 1, 1, 0), ("replay_all_per_warp", 1, 1, 1)):
+        ofdm.set_option("exact_speculation", spec); ofdm.set_option("force_replay", force); ofdm.set_option("stream_layout", layout)
         ofdm.replayed_frames(reset=True)
         runs[name] = (ofdm.mc_sweep_philox(2024, 5000, n, 2, snr, pkg.MODE_EXACT), ofdm.replayed_frames())
-    for x, y, z in zip(runs["checked"][0], runs["all_exact"][0], runs["replay_all"][0]):
-        assert ints(x) == ints(y) == ints(z)
+    ofdm.set_option("stream_layout", 0)
+    for x, y, z, w in zip(runs["checked"][0], runs["all_exact"][0], runs["replay_all"][0], runs["replay_all_per_warp"][0]):
+        assert ints(x) == ints(y) == ints(z) == ints(w)
         assert abs(x.sum_err2 - y.sum_err2) <= 1e-5 * y.sum_err2
         assert abs(z.sum_err2 - y.sum_err2) <= 1e-6 * y.sum_err2          # same per-bin arithmetic, the float terms of a frame added in another order
-    assert runs["replay_all"][1] == n * len(snr) and runs["all_exact"][1] == 0
+        assert abs(w.sum_err2 - y.sum_err2) <= 1e-6 * y.sum_err2
+    assert runs["replay_all"][1] == runs["replay_all_per_warp"][1] == n * len(snr) and runs["all_exact"][1] == 0
     assert 0 < runs["checked"][1] < n * len(snr) // 10
 
 
-@pytest.mark.parametrize("n_sym,snr", [(1, 1.0), (3, 5.0), (4, 0.0), (6, 2.0), (7, 9.0), (9, 3.0), (23, 4.0)])
+@pytest.mark.parametrize("n_sym,snr", [(1, 1.0), (3, 5.0), (4, 0.0), (5, 6.0), (6, 2.0), (7, 9.0), (9, 3.0), (23, 4.0)])
 def test_other_frame_shapes(knobs, pkg, port, n_sym, snr):
     """frames with n_sym != 2 stream through k_stream_rxn (pass 0 = LTS + two symbols, then four symbols per pass): speculation
     on / off / forced replay, the generic kernel and the oracle agree; fast mode agrees with the generic fast kernel"""
@@ -241,7 +265,7 @@ def test_other_frame_shapes(knobs, pkg, port, n_sym, snr):
     packed = ofdm.to_dev(pkg.pack_bits_host(bits).view(np.int32))
     gd = ofdm.to_dev(g)
     frames, power = ofdm.tx_frames(packed, n_sym, pkg.MODE_EXACT)
-    res = run_variants(ofdm, pkg, lambda: ofdm.awgn_rx_inject(frames, gd, packed, snr, n_sym, pkg.MODE_EXACT, power=power)[0])
+    res = run_variants(ofdm, pkg, lambda mode: ofdm.awgn_rx_inject(frames, gd, packed, snr, n_sym, mode, power=power)[0])
     acc = port.chain(bits, g, n_sym, snr)
     want = (acc.bit_errors, acc.bits, acc.frames_in_error, acc.rail_errors, acc.frames)
     for name, (c, _) in res.items():

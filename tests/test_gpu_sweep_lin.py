@@ -74,11 +74,16 @@ def test_every_point_replayed_and_all_exact(knobs, pkg):
         ofdm.set_option("fused_sweep", fused); ofdm.set_option("exact_speculation", spec); ofdm.set_option("force_replay", force)
         ofdm.replayed_frames(reset=True)
         runs[name] = (ofdm.sweep_inject_dev(packed, g, n, 2, snr, pkg.MODE_EXACT), ofdm.replayed_frames())
-    for a, b, c, d in zip(runs["fused"][0], runs["replay_all"][0], runs["all_exact"][0], runs["staged_checked"][0]):
-        assert ints(a) == ints(b) == ints(c) == ints(d)
+    # the fp32 sweep kernel's EVM-guard replay, forced for every point, on the same (exact) transmitter frames
+    ofdm.set_option("fused_sweep", 1); ofdm.set_option("exact_speculation", 1); ofdm.set_option("force_replay", 1)
+    frames, power = ofdm.tx_frames(packed, 2, pkg.MODE_EXACT)
+    ofdm.replayed_frames(reset=True)
+    runs["fast_replay_all"] = (ofdm.awgn_rx_inject_sweep(frames, g, packed, snr, 2, pkg.MODE_FAST, power=power), ofdm.replayed_frames())
+    for a, b, c, d, e in zip(runs["fused"][0], runs["replay_all"][0], runs["all_exact"][0], runs["staged_checked"][0], runs["fast_replay_all"][0]):
+        assert ints(a) == ints(b) == ints(c) == ints(d) == ints(e)
         assert abs(a.sum_err2 - c.sum_err2) <= 1e-6 * c.sum_err2 and abs(a.sum_evm_lin - c.sum_evm_lin) <= 1e-6 * c.sum_evm_lin
         assert abs(b.sum_err2 - c.sum_err2) <= 1e-7 * c.sum_err2           # the replay is the all-exact kernel's arithmetic (float partial sums grouped differently)
-    assert runs["replay_all"][1] == n * len(snr) and runs["all_exact"][1] == 0
+    assert runs["replay_all"][1] == runs["fast_replay_all"][1] == n * len(snr) and runs["all_exact"][1] == 0
     assert 0 < runs["fused"][1] < n * len(snr) // 10                       # speculation must pay
 
 
