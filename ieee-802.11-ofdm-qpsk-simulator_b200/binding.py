@@ -64,6 +64,31 @@ def channel(noise="real", snr_def="frame_power", n_taps=0):
     return Channel(NOISE[noise], SNR_DEF[snr_def], int(n_taps))
 
 
+class Code(C.Structure):
+    """ofdm_code"""
+    _fields_ = [("rate", C.c_int), ("decision", C.c_int)]
+
+
+# ofdm_code's enums under the names the Python methods take (DESIGN.md section 6.2)
+CODE = {"1/2": 1, "3/4": 2}
+DECISION = {"soft": 0, "hard": 1}
+DATA_BITS_PER_SYM = {"1/2": 48, "3/4": 72}
+
+
+def code(rate="1/2", decision="soft"):
+    """Code from names: rate "1/2" | "3/4", decision "soft" | "hard" (include/ofdm_b200.h)."""
+    if rate not in CODE:
+        raise ValueError("rate must be one of %s, not %r" % (sorted(CODE), rate))
+    if decision not in DECISION:
+        raise ValueError("decision must be one of %s, not %r" % (sorted(DECISION), decision))
+    return Code(CODE[rate], DECISION[decision])
+
+
+def info_bits(rate, n_sym):
+    """K_info: the information bits of a coded frame of n_sym OFDM symbols (the last 6 of n_sym * N_DBPS are the tail)."""
+    return n_sym * DATA_BITS_PER_SYM[rate] - 6
+
+
 class OfdmError(RuntimeError):
     pass
 
@@ -124,6 +149,11 @@ SIGNATURES = {
     "ofdm_mc_sweep_channel_until": (_I, [_VP, C.POINTER(Channel), _U32, _U64, _I, _VP, _I, _I, _U64, _U64, _L, C.POINTER(Counters),
                                          C.POINTER(_I)]),
     "ofdm_mc_sweep_philox": (_I, [_VP, _U32, _U64, _L, _I, _VP, _I, _I, C.POINTER(Counters)]),
+    "ofdm_conv_encode": (_I, [_VP, _I, _VP, _VP, _L, _I]),
+    "ofdm_viterbi_decode": (_I, [_VP, C.POINTER(Code), _VP, _VP, _VP, _VP, _L, _I, _VP]),
+    "ofdm_mc_sweep_coded_dev": (_I, [_VP, C.POINTER(Channel), C.POINTER(Code), _U32, _U64, _L, _I, _VP, _VP, _I, _I, _VP, _VP]),
+    "ofdm_mc_sweep_coded_until": (_I, [_VP, C.POINTER(Channel), C.POINTER(Code), _U32, _U64, _I, _VP, _I, _I, _U64, _U64, _L,
+                                       C.POINTER(Counters), C.POINTER(Counters), C.POINTER(_I)]),
     "ofdm_multipath_taps": (_I, [_VP, _VP, _VP, _I, _VP, _L, _I]),
     "ofdm_multipath_philox": (_I, [_VP, _VP, _U32, _U64, _I, _VP, _VP, _L, _I]),
     "ofdm_mc_sweep_multipath_dev": (_I, [_VP, _U32, _U64, _L, _I, _I, _VP, _I, _I, _VP]),
@@ -485,6 +515,49 @@ class Ofdm:
         self._check(self.lib.ofdm_mc_sweep_channel_until(self.h, C.byref(ch), seed, frame0, n_sym, snr.ctypes.data, len(snr), mode,
                                                          target_errors, max_bits, round_frames, out, C.byref(rounds)))
         return list(out), int(rounds.value)
+
+    # ---- the coded link (DESIGN.md section 6.2)
+    def conv_encode(self, info, n_sym, rate="1/2"):
+        """information words [n_frames * n_sym * 3] (int32) -> payload words of the same shape for tx_frames"""
+        n_frames = info.numel() // (3 * n_sym)
+        out = self.empty((n_frames * n_sym * 3,), self.torch.int32)
+        self._check(self.lib.ofdm_conv_encode(self.h, CODE[rate] if rate in CODE else -1, _ptr(info), _ptr(out), n_frames, n_sym))
+        return out
+
+    def viterbi_decode(self, H, eq, n_sym, rate="1/2", decision="soft", info=None, want_decoded=True):
+        """decode the receiver's H [n_frames, 64, 2] and eq [n_frames, n_sym * 48, 2] dumps; returns (coded Counters or None when
+        info is None, decoded words [n_frames * n_sym * 3] or None)"""
+        cd = code(rate, decision)
+        n_frames = H.shape[0]
+        cnt = self.new_counters() if info is not None else None
+        dec = self.zeros((n_frames * n_sym * 3,), self.torch.int32) if want_decoded else None
+        self._check(self.lib.ofdm_viterbi_decode(self.h, C.byref(cd), _ptr(H), _ptr(eq), _ptr(info), _ptr(dec), n_frames, n_sym, _ptr(cnt)))
+        return (self.read_counters(cnt)[0] if cnt is not None else None), dec
+
+    def mc_sweep_coded(self, seed, frame0, n_frames, n_sym, snr_db, mode, rate="1/2", decision="soft", noise="real", snr_def="frame_power",
+                       n_taps=0, streams=None, counters=None):
+        """Monte-Carlo sweep of the coded link through the channel (noise, snr_def, n_taps).  counters=None: returns host totals
+        (coded, raw); else counters is a pair of device tensors (coded, raw or None) accumulated into, and None is returned."""
+        ch, cd = channel(noise, snr_def, n_taps), code(rate, decision)
+        snr = np.ascontiguousarray(snr_db, dtype=np.float32)
+        st = None if streams is None else np.ascontiguousarray(streams, dtype=np.uint32)
+        coded, raw = counters if counters is not None else (self.new_counters(len(snr)), self.new_counters(len(snr)))
+        self._check(self.lib.ofdm_mc_sweep_coded_dev(self.h, C.byref(ch), C.byref(cd), seed, frame0, n_frames, n_sym, snr.ctypes.data,
+                                                     None if st is None else st.ctypes.data, len(snr), mode, _ptr(coded), _ptr(raw)))
+        if counters is not None:
+            return None
+        return self.read_counters(coded), self.read_counters(raw)
+
+    def mc_sweep_coded_until(self, seed, frame0, n_sym, snr_db, mode, rate="1/2", decision="soft", noise="real", snr_def="frame_power",
+                             n_taps=0, target_errors=100, max_bits=10 ** 9, round_frames=1 << 20):
+        """configs[3]'s stop rule on the coded counters, on one GPU: returns (coded host totals, raw host totals, rounds)"""
+        ch, cd = channel(noise, snr_def, n_taps), code(rate, decision)
+        snr = np.ascontiguousarray(snr_db, dtype=np.float32)
+        coded, raw = (Counters * len(snr))(), (Counters * len(snr))()
+        rounds = _I(0)
+        self._check(self.lib.ofdm_mc_sweep_coded_until(self.h, C.byref(ch), C.byref(cd), seed, frame0, n_sym, snr.ctypes.data, len(snr), mode,
+                                                       target_errors, max_bits, round_frames, coded, raw, C.byref(rounds)))
+        return list(coded), list(raw), int(rounds.value)
 
     def multipath_taps(self, tx, taps, n_sym):
         out = self.empty(tuple(tx.shape), self.torch.float32)

@@ -14,6 +14,7 @@
 #include "ofdm_stream.cuh"
 #include "ofdm_mc_quad.cuh"
 #include "ofdm_sweep.cuh"
+#include "ofdm_code.cuh"
 
 using namespace ofdm;
 
@@ -42,9 +43,10 @@ struct ofdm_ctx {
     float *sts_dev = nullptr;
     unsigned long long *replayed_dev = nullptr;  // frames / points the speculating kernels replayed exactly (this context)
     float lts_power_prefix = 0.0f;
-    // cached scratch (grown on demand, released with the context)
-    void *scratch[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    size_t scratch_bytes[7] = {0, 0, 0, 0, 0, 0, 0};
+    // cached scratch (grown on demand, released with the context); slots 7..10 belong to the coded link: payload words, H and
+    // eq dumps, k_viterbi's survivors in HBM
+    void *scratch[11] = {nullptr};
+    size_t scratch_bytes[11] = {0};
 };
 
 namespace {
@@ -332,11 +334,11 @@ bool snr_def_ok(int snr_def) { return snr_def >= OFDM_SNR_FRAME_POWER && snr_def
 bool is_reference_channel(int noise, int snr_def) { return noise == OFDM_NOISE_REAL_RAIL && snr_def == OFDM_SNR_FRAME_POWER; }
 
 // noise power of an Es/N0 or Eb/N0 point: a data bin carries X (|X| = 1) and, through the transmitter's 1/64 IFFT and the
-// receiver's unscaled FFT, noise of variance 64 np, so Es/N0 = 1 / (64 np); Eb/N0 = Es/N0 / 2 (two bits per QPSK point).
-// In double, rounded to float once.
-float fixed_noise_power(int snr_def, float snr_db)
+// receiver's unscaled FFT, noise of variance 64 np, so Es/N0 = 1 / (64 np); Eb/N0 = Es/N0 / bits, bits = the information bits
+// a QPSK point carries (2 uncoded, 2R behind a rate-R code; the 6 tail bits are not counted).  In double, rounded to float once.
+float fixed_noise_power(int snr_def, float snr_db, double bits = 2.0)
 {
-    const double per_point = snr_def == OFDM_SNR_EBN0 ? 128.0 : 64.0;
+    const double per_point = snr_def == OFDM_SNR_EBN0 ? 64.0 * bits : 64.0;
     return (float)(1.0 / (per_point * pow(10.0, (double)snr_db / 10.0)));
 }
 
@@ -354,6 +356,60 @@ int launch_awgn_channel(ofdm_ctx *ctx, int noise, const float *tx, const float *
     const bool cx = noise == OFDM_NOISE_COMPLEX;
     if (mode == OFDM_MODE_EXACT) return cx ? launch(k_awgn_channel<true, true>) : launch(k_awgn_channel<true, false>);
     return cx ? launch(k_awgn_channel<false, true>) : launch(k_awgn_channel<false, false>);
+}
+
+bool rate_ok(int rate) { return rate == OFDM_CODE_R12 || rate == OFDM_CODE_R34; }
+bool code_ok(const ofdm_code *code)
+{
+    return code != nullptr && rate_ok(code->rate) && (code->decision == OFDM_DECISION_SOFT || code->decision == OFDM_DECISION_HARD);
+}
+// information bits per QPSK point: 2 uncoded, 2R behind the code
+double info_bits_per_point(const ofdm_code *code) { return code == nullptr ? 2.0 : code->rate == OFDM_CODE_R12 ? 1.0 : 1.5; }
+
+int launch_conv_encode(ofdm_ctx *ctx, int rate, const uint32_t *info, uint32_t *payload, long n_frames, int n_sym)
+{
+    auto k = rate == OFDM_CODE_R12 ? k_conv_encode<kCodeR12> : k_conv_encode<kCodeR34>;
+    k<<<blocks_1d(n_frames * n_sym), 256, 0, ctx->stream>>>(info, payload, n_frames, n_sym);
+    return check_launch(ctx, "k_conv_encode");
+}
+
+// k_viterbi over n_frames frames: a block's survivors stay in shared memory up to kVitSmemMax (two-symbol frames: 6 KB at rate
+// 1/2, 9 KB at 3/4), longer frames keep them in a scratch buffer in HBM for a grid of at most two blocks per SM (the longest
+// frames: 288 KiB per warp).  Same code either way, so the same bits.  One launch per 2^20 frames: the per-lane totals are 32-bit.
+int launch_viterbi(ofdm_ctx *ctx, const ofdm_code &code, const float *H, const float *eq, const uint32_t *info, uint32_t *decoded,
+                   long n_frames, int n_sym, ofdm_counters *counters)
+{
+    const size_t per_warp = vit_surv_bytes(code.rate, n_sym);
+    const bool in_smem = per_warp * kVitWarps <= (size_t)kVitSmemMax;
+    const size_t smem = in_smem ? per_warp * kVitWarps : 0;
+    const long max_frames = 1L << 20;
+    auto go = [&](auto k) -> int {
+        if (in_smem) OFDM_CUDA(ctx, allow_smem(ctx, k, kVitSmemMax));
+        for (long f0 = 0; f0 < n_frames; f0 += max_frames) {
+            VitParams p;
+            memset(&p, 0, sizeof p);
+            p.n_frames = n_frames - f0 < max_frames ? n_frames - f0 : max_frames;
+            p.n_sym = n_sym;
+            p.H = reinterpret_cast<const float2 *>(H) + f0 * 64;
+            p.eq = reinterpret_cast<const float2 *>(eq) + f0 * n_sym * 48;
+            p.info = info ? info + f0 * n_sym * 3 : nullptr;
+            p.decoded = decoded ? decoded + f0 * n_sym * 3 : nullptr;
+            p.counters = counters;
+            int grid = grid_for(ctx, k, smem, kVitWarps, p.n_frames, kVitWarps * 32);
+            if (!in_smem) {
+                if (grid > 2 * ctx->sm_count) grid = 2 * ctx->sm_count;
+                void *buf = nullptr;
+                if (int st = ensure_scratch(ctx, 10, (size_t)grid * kVitWarps * per_warp, &buf)) return st;
+                p.surv_global = reinterpret_cast<uint2 *>(buf);
+            }
+            k<<<grid, kVitWarps * 32, smem, ctx->stream>>>(p);
+            if (int st = check_launch(ctx, "k_viterbi")) return st;
+        }
+        return OFDM_OK;
+    };
+    const bool hard = code.decision == OFDM_DECISION_HARD;
+    if (code.rate == OFDM_CODE_R12) return hard ? go(k_viterbi<kCodeR12, kDecisionHard>) : go(k_viterbi<kCodeR12, kDecisionSoft>);
+    return hard ? go(k_viterbi<kCodeR34, kDecisionHard>) : go(k_viterbi<kCodeR34, kDecisionSoft>);
 }
 
 
@@ -470,7 +526,7 @@ int ofdm_ctx_destroy(ofdm_ctx *ctx)
     if (!ctx) return OFDM_ERR_INVALID;
     cudaSetDevice(ctx->device);
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-    for (int i = 0; i < 7; ++i) if (ctx->scratch[i]) cudaFree(ctx->scratch[i]);
+    for (int i = 0; i < 11; ++i) if (ctx->scratch[i]) cudaFree(ctx->scratch[i]);
     if (ctx->sts_dev) cudaFree(ctx->sts_dev);
     if (ctx->replayed_dev) cudaFree(ctx->replayed_dev);
     if (ctx->copy_stream) {
@@ -1088,25 +1144,42 @@ int mc_fused(ofdm_ctx *ctx, K k, bool quad, const McParams &all)
 // frames], then per point the reference channel's fused channel + receiver (ofdm_awgn_rx_philox), or another channel
 // (k_awgn_channel) into an OTA buffer and the verified receiver of ofdm_rx_frames on it.  Without taps the frame power comes
 // from the transmitter (its LTS-prefix shortcut).
-int mc_staged(ofdm_ctx *ctx, const ofdm_channel &ch, uint32_t seed, uint64_t frame0, long n_frames, int n_sym, const float *snr_db,
-              const uint32_t *streams, int n_snr, int mode, ofdm_counters *counters)
+// With a code (nullable) the Philox bits are the information bits: k_conv_encode turns them into the payload the transmitter
+// sends, the receiver dumps H and eq of every point (its own counters go to raw, nullable) and k_viterbi decodes them and counts
+// the information-bit errors into counters.  Eb/N0 points then count information bits (fixed_noise_power).
+int mc_staged(ofdm_ctx *ctx, const ofdm_channel &ch, const ofdm_code *code, uint32_t seed, uint64_t frame0, long n_frames, int n_sym,
+              const float *snr_db, const uint32_t *streams, int n_snr, int mode, ofdm_counters *counters, ofdm_counters *raw)
 {
     const int len = OFDM_FRAME_LEN(n_sym);
     const bool reference = is_reference_channel(ch.noise, ch.snr_def), per_frame = ch.snr_def == OFDM_SNR_FRAME_POWER, mp = ch.n_taps > 0;
-    long chunk = (2L << 30) / ((long)len * 8);
+    const long dump_bytes = code ? (64L + 48L * n_sym) * 8 : 0;       // H and eq of a frame
+    long chunk = (2L << 30) / ((long)len * 8 + dump_bytes);
     if (chunk < 1024) chunk = 1024;
     for (long f0 = 0; f0 < n_frames; f0 += chunk) {
         const long n = n_frames - f0 < chunk ? n_frames - f0 : chunk;
-        const size_t frame_bytes = (size_t)n * len * 2 * sizeof(float);
-        void *bits = nullptr, *frames = nullptr, *power = nullptr, *faded = nullptr, *ota = nullptr;
-        if (int st = ensure_scratch(ctx, 4, (size_t)n * n_sym * 3 * sizeof(uint32_t), &bits)) return st;
+        const size_t frame_bytes = (size_t)n * len * 2 * sizeof(float), word_bytes = (size_t)n * n_sym * 3 * sizeof(uint32_t);
+        void *bits = nullptr, *frames = nullptr, *power = nullptr, *faded = nullptr, *ota = nullptr, *payload = nullptr;
+        ofdm_rx_dump dump;
+        memset(&dump, 0, sizeof dump);
+        if (int st = ensure_scratch(ctx, 4, word_bytes, &bits)) return st;
         if (int st = ensure_scratch(ctx, 1, frame_bytes, &frames)) return st;
         if (mp) if (int st = ensure_scratch(ctx, 5, frame_bytes, &faded)) return st;
         if (!reference) if (int st = ensure_scratch(ctx, 6, frame_bytes, &ota)) return st;
         if (per_frame) if (int st = ensure_scratch(ctx, 2, (size_t)n * sizeof(float), &power)) return st;
+        if (code) {
+            void *H = nullptr, *eq = nullptr;
+            if (int st = ensure_scratch(ctx, 7, word_bytes, &payload)) return st;
+            if (int st = ensure_scratch(ctx, 8, (size_t)n * 64 * 2 * sizeof(float), &H)) return st;
+            if (int st = ensure_scratch(ctx, 9, (size_t)n * n_sym * 48 * 2 * sizeof(float), &eq)) return st;
+            dump.H = (float *)H;
+            dump.eq = (float *)eq;
+        }
         const uint64_t fr0 = frame0 + (uint64_t)f0;
         if (int st = ofdm_random_bits(ctx, seed, fr0, n, n_sym, (uint32_t *)bits)) return st;
-        if (int st = ofdm_tx_frames(ctx, (const uint32_t *)bits, (float *)frames, mp ? nullptr : (float *)power, n, n_sym, mode)) return st;
+        if (code) if (int st = launch_conv_encode(ctx, code->rate, (const uint32_t *)bits, (uint32_t *)payload, n, n_sym)) return st;
+        const uint32_t *sent = (const uint32_t *)(code ? payload : bits);
+        const ofdm_rx_dump *dp = code ? &dump : nullptr;
+        if (int st = ofdm_tx_frames(ctx, sent, (float *)frames, mp ? nullptr : (float *)power, n, n_sym, mode)) return st;
         const float *air = (const float *)frames;
         if (mp) {
             if (int st = ofdm_multipath_philox(ctx, air, seed, fr0, ch.n_taps, (float *)faded, nullptr, n, n_sym)) return st;
@@ -1115,20 +1188,70 @@ int mc_staged(ofdm_ctx *ctx, const ofdm_channel &ch, uint32_t seed, uint64_t fra
         }
         for (int i = 0; i < n_snr; ++i) {
             const uint32_t stream = streams ? streams[i] : (uint32_t)i;
+            ofdm_counters *rx_cnt = code ? (raw ? raw + i : nullptr) : counters + i;
             if (reference) {
-                if (int st = ofdm_awgn_rx_philox(ctx, air, (const float *)power, (const uint32_t *)bits, snr_db[i], seed, stream, fr0, n, n_sym,
-                                                 mode, counters + i, nullptr))
+                if (int st = ofdm_awgn_rx_philox(ctx, air, (const float *)power, sent, snr_db[i], seed, stream, fr0, n, n_sym, mode, rx_cnt, dp))
                     return st;
-                continue;
+            } else {
+                const int st = per_frame ? launch_awgn_channel(ctx, ch.noise, air, (const float *)power, snr_linear(snr_db[i]), 0.f, seed, stream,
+                                                               fr0, (float *)ota, n, len, mode)
+                                         : launch_awgn_channel(ctx, ch.noise, air, nullptr, 1.f,
+                                                               fixed_noise_power(ch.snr_def, snr_db[i], info_bits_per_point(code)), seed, stream, fr0,
+                                                               (float *)ota, n, len, mode);
+                if (st) return st;
+                if (int st2 = ofdm_rx_frames(ctx, (const float *)ota, sent, n, n_sym, mode, rx_cnt, dp)) return st2;
             }
-            const int st = per_frame ? launch_awgn_channel(ctx, ch.noise, air, (const float *)power, snr_linear(snr_db[i]), 0.f, seed, stream, fr0,
-                                                           (float *)ota, n, len, mode)
-                                     : launch_awgn_channel(ctx, ch.noise, air, nullptr, 1.f, fixed_noise_power(ch.snr_def, snr_db[i]), seed, stream,
-                                                           fr0, (float *)ota, n, len, mode);
-            if (st) return st;
-            if (int st2 = ofdm_rx_frames(ctx, (const float *)ota, (const uint32_t *)bits, n, n_sym, mode, counters + i, nullptr)) return st2;
+            if (code)
+                if (int st = launch_viterbi(ctx, *code, dump.H, dump.eq, (const uint32_t *)bits, nullptr, n, n_sym, counters + i)) return st;
         }
     }
+    return OFDM_OK;
+}
+
+void add_counters(ofdm_counters &t, const ofdm_counters &q)
+{
+    t.bit_errors += q.bit_errors; t.bits += q.bits; t.frames_in_error += q.frames_in_error; t.rail_errors += q.rail_errors; t.frames += q.frames;
+    t.sum_err2 += q.sum_err2; t.sum_ref2 += q.sum_ref2; t.sum_evm_lin += q.sum_evm_lin;
+}
+
+// The stop rule of configs[3]: rounds of round_frames frames (global indices frame0 + r * round_frames ...) until every point has
+// >= target_errors bit errors or >= max_bits bits in out_host.  run_round(frame0, snr, streams, n_active, cnt, raw) accumulates
+// one round of the still-active points into the zeroed device counters cnt [n_active] and, when raw_host is given, raw
+// [n_active], which are summed into raw_host alongside.
+template <typename R>
+int until_rounds(ofdm_ctx *ctx, uint64_t frame0, const float *snr_db, int n_snr, uint64_t target_errors, uint64_t max_bits, long round_frames,
+                 ofdm_counters *out_host, ofdm_counters *raw_host, int *rounds_out, R run_round)
+{
+    if (rounds_out) *rounds_out = 0;
+    if (n_snr == 0) return OFDM_OK;
+    memset(out_host, 0, sizeof(ofdm_counters) * (size_t)n_snr);
+    if (raw_host) memset(raw_host, 0, sizeof(ofdm_counters) * (size_t)n_snr);
+    void *buf = nullptr;
+    if (int st = ensure_scratch(ctx, 3, sizeof(ofdm_counters) * 2 * (size_t)kMaxSnr, &buf)) return st;
+    ofdm_counters *cnt = (ofdm_counters *)buf, *raw = raw_host ? cnt + kMaxSnr : nullptr;
+    int active[kMaxSnr], n_active = n_snr, rounds = 0;
+    for (int i = 0; i < n_snr; ++i) active[i] = i;
+    ofdm_counters part[kMaxSnr], part_raw[kMaxSnr];
+    while (n_active > 0) {
+        float snr_a[kMaxSnr];
+        uint32_t stream_a[kMaxSnr];
+        for (int j = 0; j < n_active; ++j) { snr_a[j] = snr_db[active[j]]; stream_a[j] = (uint32_t)active[j]; }
+        OFDM_CUDA(ctx, cudaMemsetAsync(cnt, 0, sizeof(ofdm_counters) * (size_t)(raw ? 2 * kMaxSnr : n_active), ctx->stream));
+        if (int st = run_round(frame0 + (uint64_t)rounds * (uint64_t)round_frames, snr_a, stream_a, n_active, cnt, raw)) return st;
+        OFDM_CUDA(ctx, cudaMemcpyAsync(part, cnt, sizeof(ofdm_counters) * (size_t)n_active, cudaMemcpyDeviceToHost, ctx->stream));
+        if (raw) OFDM_CUDA(ctx, cudaMemcpyAsync(part_raw, raw, sizeof(ofdm_counters) * (size_t)n_active, cudaMemcpyDeviceToHost, ctx->stream));
+        OFDM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        int keep = 0;
+        for (int j = 0; j < n_active; ++j) {
+            ofdm_counters &t = out_host[active[j]];
+            add_counters(t, part[j]);
+            if (raw) add_counters(raw_host[active[j]], part_raw[j]);
+            if (t.bit_errors < target_errors && t.bits < max_bits) active[keep++] = active[j];   // the stop rule of configs[3]
+        }
+        n_active = keep;
+        ++rounds;
+    }
+    if (rounds_out) *rounds_out = rounds;
     return OFDM_OK;
 }
 }  // namespace
@@ -1169,7 +1292,7 @@ int ofdm_mc_sweep_channel_dev(ofdm_ctx *ctx, const ofdm_channel *ch, uint32_t se
     bool fused = n_sym == 2;
     if (!reference) fused = fused && fast && !ctx->force_generic;
     else if (mp) fused = fused && !ctx->force_generic && (ctx->multipath_path == 2 || (ctx->multipath_path == 0 && fast));
-    if (!fused) return mc_staged(ctx, *ch, seed, frame0, n_frames, n_sym, snr_db, streams, n_points, mode, counters);
+    if (!fused) return mc_staged(ctx, *ch, nullptr, seed, frame0, n_frames, n_sym, snr_db, streams, n_points, mode, counters, nullptr);
     const McParams p = mc_params(ctx, *ch, seed, frame0, n_frames, snr_db, streams, n_points, counters);
     auto quad = [&](auto k) { return mc_fused(ctx, k, true, p); };
     if (!reference) {                   // k_mc_quad<fast, MP, CH>: the channel is a compile-time parameter
@@ -1211,37 +1334,58 @@ int ofdm_mc_sweep_channel_until(ofdm_ctx *ctx, const ofdm_channel *ch, uint32_t 
     OFDM_REQUIRE(ctx, ch != nullptr && noise_ok(ch->noise) && snr_def_ok(ch->snr_def) && ch->n_taps >= 0 && ch->n_taps <= kMaxTaps);
     OFDM_REQUIRE(ctx, nsym_ok(n_sym) && mode_ok(mode) && n_snr >= 0 && n_snr <= kMaxSnr);
     OFDM_REQUIRE(ctx, round_frames >= 1 && max_bits >= 1 && (n_snr == 0 || (snr_db != nullptr && out_host != nullptr)));
-    if (rounds_out) *rounds_out = 0;
-    if (n_snr == 0) return OFDM_OK;
-    memset(out_host, 0, sizeof(ofdm_counters) * (size_t)n_snr);
-    void *cnt = nullptr;
-    if (int st = ensure_scratch(ctx, 3, sizeof(ofdm_counters) * (size_t)kMaxSnr, &cnt)) return st;
-    int active[kMaxSnr], n_active = n_snr, rounds = 0;
-    for (int i = 0; i < n_snr; ++i) active[i] = i;
-    ofdm_counters part[kMaxSnr];
-    while (n_active > 0) {
-        float snr_a[kMaxSnr];
-        uint32_t stream_a[kMaxSnr];
-        for (int j = 0; j < n_active; ++j) { snr_a[j] = snr_db[active[j]]; stream_a[j] = (uint32_t)active[j]; }
-        OFDM_CUDA(ctx, cudaMemsetAsync(cnt, 0, sizeof(ofdm_counters) * (size_t)n_active, ctx->stream));
-        if (int st = ofdm_mc_sweep_channel_dev(ctx, ch, seed, frame0 + (uint64_t)rounds * (uint64_t)round_frames, round_frames, n_sym, snr_a, stream_a,
-                                               n_active, mode, (ofdm_counters *)cnt))
-            return st;
-        OFDM_CUDA(ctx, cudaMemcpyAsync(part, cnt, sizeof(ofdm_counters) * (size_t)n_active, cudaMemcpyDeviceToHost, ctx->stream));
-        OFDM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        int keep = 0;
-        for (int j = 0; j < n_active; ++j) {
-            ofdm_counters &t = out_host[active[j]];
-            const ofdm_counters &q = part[j];
-            t.bit_errors += q.bit_errors; t.bits += q.bits; t.frames_in_error += q.frames_in_error; t.rail_errors += q.rail_errors; t.frames += q.frames;
-            t.sum_err2 += q.sum_err2; t.sum_ref2 += q.sum_ref2; t.sum_evm_lin += q.sum_evm_lin;
-            if (t.bit_errors < target_errors && t.bits < max_bits) active[keep++] = active[j];   // the stop rule of configs[3]
-        }
-        n_active = keep;
-        ++rounds;
-    }
-    if (rounds_out) *rounds_out = rounds;
-    return OFDM_OK;
+    return until_rounds(ctx, frame0, snr_db, n_snr, target_errors, max_bits, round_frames, out_host, nullptr, rounds_out,
+                        [&](uint64_t fr0, const float *snr, const uint32_t *streams, int n_points, ofdm_counters *cnt, ofdm_counters *) {
+                            return ofdm_mc_sweep_channel_dev(ctx, ch, seed, fr0, round_frames, n_sym, snr, streams, n_points, mode, cnt);
+                        });
+}
+
+// ------------------------------------------------------------------ the coded link (DESIGN.md section 6.2)
+int ofdm_conv_encode(ofdm_ctx *ctx, int rate, const uint32_t *info, uint32_t *payload, long n_frames, int n_sym)
+{
+    if (int st = bind(ctx)) return st;
+    OFDM_REQUIRE(ctx, rate_ok(rate) && n_frames >= 0 && nsym_ok(n_sym));
+    if (n_frames == 0) return OFDM_OK;
+    OFDM_REQUIRE(ctx, info != nullptr && payload != nullptr && (const void *)info != (const void *)payload);
+    return launch_conv_encode(ctx, rate, info, payload, n_frames, n_sym);
+}
+
+int ofdm_viterbi_decode(ofdm_ctx *ctx, const ofdm_code *code, const float *H, const float *eq, const uint32_t *info, uint32_t *decoded,
+                        long n_frames, int n_sym, ofdm_counters *counters)
+{
+    if (int st = bind(ctx)) return st;
+    OFDM_REQUIRE(ctx, code_ok(code) && n_frames >= 0 && nsym_ok(n_sym));
+    if (n_frames == 0) return OFDM_OK;
+    OFDM_REQUIRE(ctx, H != nullptr && eq != nullptr && (counters == nullptr || info != nullptr));
+    return launch_viterbi(ctx, *code, H, eq, info, decoded, n_frames, n_sym, counters);
+}
+
+int ofdm_mc_sweep_coded_dev(ofdm_ctx *ctx, const ofdm_channel *ch, const ofdm_code *code, uint32_t seed, uint64_t frame0, long n_frames,
+                            int n_sym, const float *snr_db, const uint32_t *streams, int n_points, int mode, ofdm_counters *coded,
+                            ofdm_counters *raw)
+{
+    if (int st = bind(ctx)) return st;
+    OFDM_REQUIRE(ctx, ch != nullptr && noise_ok(ch->noise) && snr_def_ok(ch->snr_def) && ch->n_taps >= 0 && ch->n_taps <= kMaxTaps);
+    OFDM_REQUIRE(ctx, code_ok(code));
+    OFDM_REQUIRE(ctx, n_frames >= 0 && nsym_ok(n_sym) && mode_ok(mode) && n_points >= 0 && n_points <= kMaxSnr);
+    if (n_frames == 0 || n_points == 0) return OFDM_OK;
+    OFDM_REQUIRE(ctx, snr_db != nullptr && coded != nullptr);
+    return mc_staged(ctx, *ch, code, seed, frame0, n_frames, n_sym, snr_db, streams, n_points, mode, coded, raw);
+}
+
+int ofdm_mc_sweep_coded_until(ofdm_ctx *ctx, const ofdm_channel *ch, const ofdm_code *code, uint32_t seed, uint64_t frame0, int n_sym,
+                              const float *snr_db, int n_snr, int mode, uint64_t target_errors, uint64_t max_bits, long round_frames,
+                              ofdm_counters *coded_host, ofdm_counters *raw_host, int *rounds_out)
+{
+    if (int st = bind(ctx)) return st;
+    OFDM_REQUIRE(ctx, ch != nullptr && noise_ok(ch->noise) && snr_def_ok(ch->snr_def) && ch->n_taps >= 0 && ch->n_taps <= kMaxTaps);
+    OFDM_REQUIRE(ctx, code_ok(code));
+    OFDM_REQUIRE(ctx, nsym_ok(n_sym) && mode_ok(mode) && n_snr >= 0 && n_snr <= kMaxSnr);
+    OFDM_REQUIRE(ctx, round_frames >= 1 && max_bits >= 1 && (n_snr == 0 || (snr_db != nullptr && coded_host != nullptr)));
+    return until_rounds(ctx, frame0, snr_db, n_snr, target_errors, max_bits, round_frames, coded_host, raw_host, rounds_out,
+                        [&](uint64_t fr0, const float *snr, const uint32_t *streams, int n_points, ofdm_counters *cnt, ofdm_counters *raw) {
+                            return ofdm_mc_sweep_coded_dev(ctx, ch, code, seed, fr0, round_frames, n_sym, snr, streams, n_points, mode, cnt, raw);
+                        });
 }
 
 int ofdm_mc_sweep_philox(ofdm_ctx *ctx, uint32_t seed, uint64_t frame0, long n_frames, int n_sym, const float *snr_db,

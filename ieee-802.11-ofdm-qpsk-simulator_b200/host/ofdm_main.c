@@ -30,6 +30,12 @@
  *       noise on the I rail only, SNR = measured frame power / noise power.  complex = circular complex noise, half of the noise
  *       power per rail; esn0 / ebn0 = Es/N0 per data subcarrier / Eb/N0, the SNR axis of textbook QPSK curves.  Not available
  *       with --message or --draws, whose channels are the reference's by definition;
+ *   --code 1/2|3/4 [--decision soft|hard] (with --frames N or --target-errors E, also with --taps, --noise, --snr-def and --gpus):
+ *       the coded link (ofdm_code, DESIGN.md section 6.2): the 802.11a convolutional code of that rate between the Philox bits and
+ *       the transmitter, a soft- (default) or hard-decision Viterbi decoder behind the receiver; --snr-def ebn0 then counts Eb per
+ *       information bit.  Output_BER.txt holds the decoded BER, a fifth file <outdir>/Output_PER.txt the packet error rate, and
+ *       the EVM files come from the receiver's own (raw) counters; the until rule stops on the decoded bit errors.  Not available
+ *       with --message or --draws;
  *   --gpus N: the frames of the Monte-Carlo sweep are sharded across N GPUs of this node by global frame index
  *       (one context per GPU, all driven from this thread) and the counters are summed with ONE NCCL all-reduce
  *       per buffer type (built with -DOFDM_WITH_NCCL; link -lnccl).
@@ -101,6 +107,15 @@ static void report_rate(const char *what, int n_gpus, long frames, int n_sym, in
             n_snr, n_gpus, seconds, (double)frames * n_sym * n_snr / seconds);
 }
 
+/* one Monte-Carlo call over a list of points: the channel sweep into cnt, or the coded link (coded counters into cnt [n_points],
+ * the receiver's raw counters into cnt + n_points) */
+static int run_points(ofdm_ctx *ctx, const ofdm_channel *ch, const ofdm_code *code, unsigned seed, uint64_t frame0, long n, int n_sym,
+                      const float *snr, const uint32_t *streams, int n_points, int mode, ofdm_counters *cnt)
+{
+    if (code) return ofdm_mc_sweep_coded_dev(ctx, ch, code, seed, frame0, n, n_sym, snr, streams, n_points, mode, cnt, cnt + n_points);
+    return ofdm_mc_sweep_channel_dev(ctx, ch, seed, frame0, n, n_sym, snr, streams, n_points, mode, cnt);
+}
+
 #ifdef OFDM_WITH_NCCL
 #define NCHECK(call)                                                                   \
     do {                                                                               \
@@ -108,11 +123,13 @@ static void report_rate(const char *what, int n_gpus, long frames, int n_sym, in
         if (r_ != ncclSuccess) { fprintf(stderr, "%s failed: %s\n", #call, ncclGetErrorString(r_)); return 1; } \
     } while (0)
 
-/* SURVEY 8(e): shard (frame range) across GPUs, counter-based RNG keyed on the global frame index, one all-reduce */
-static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, const ofdm_channel *ch, const float *SNR, int n_snr, int mode,
-                           ofdm_counters *totals, unsigned long long target_errors, unsigned long long max_bits, long round_frames, int round_reduce_host)
+/* SURVEY 8(e): shard (frame range) across GPUs, counter-based RNG keyed on the global frame index, one all-reduce.  With a code
+ * the counters of a call are the coded ones followed by the raw ones (2 n entries, reduced together); raw_totals receives the raw. */
+static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, const ofdm_channel *ch, const ofdm_code *code, const float *SNR,
+                           int n_snr, int mode, ofdm_counters *totals, ofdm_counters *raw_totals, unsigned long long target_errors,
+                           unsigned long long max_bits, long round_frames, int round_reduce_host)
 {
-    const int n_taps = ch->n_taps;
+    const int n_taps = ch->n_taps, per = code ? 2 : 1;
     ofdm_ctx *ctxs[8] = {0};
     ofdm_ctx *ctx = NULL;
     void *cnt[8], *ints[8], *dbls[8];
@@ -123,25 +140,25 @@ static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, co
         devs[d] = d;
         CHECK(ofdm_ctx_create(&ctxs[d], d));
         ctx = ctxs[d];
-        CHECK(ofdm_dev_alloc(ctx, &cnt[d], sizeof(ofdm_counters) * (size_t)n_snr));
-        CHECK(ofdm_dev_alloc(ctx, &ints[d], sizeof(uint64_t) * 5 * (size_t)n_snr));
-        CHECK(ofdm_dev_alloc(ctx, &dbls[d], sizeof(double) * 3 * (size_t)n_snr));
-        CHECK(ofdm_memset_dev(ctx, cnt[d], 0, sizeof(ofdm_counters) * (size_t)n_snr));
+        CHECK(ofdm_dev_alloc(ctx, &cnt[d], sizeof(ofdm_counters) * (size_t)(per * n_snr)));
+        CHECK(ofdm_dev_alloc(ctx, &ints[d], sizeof(uint64_t) * 5 * (size_t)(per * n_snr)));
+        CHECK(ofdm_dev_alloc(ctx, &dbls[d], sizeof(double) * 3 * (size_t)(per * n_snr)));
+        CHECK(ofdm_memset_dev(ctx, cnt[d], 0, sizeof(ofdm_counters) * (size_t)(per * n_snr)));
     }
     NCHECK(ncclCommInitAll(comms, n_gpus, devs));
     for (int d = 0; d < n_gpus; ++d) {                      /* first use of a kernel on a device loads it: keep that out of the timing */
         ctx = ctxs[d];
-        CHECK(ofdm_mc_sweep_channel_dev(ctx, ch, seed, 0, 256, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)cnt[d]));
-        CHECK(ofdm_memset_dev(ctx, cnt[d], 0, sizeof(ofdm_counters) * (size_t)n_snr));
-        CHECK(ofdm_counters_pack(ctx, (const ofdm_counters *)cnt[d], n_snr, (uint64_t *)ints[d], (double *)dbls[d]));
+        CHECK(run_points(ctx, ch, code, seed, 0, 256, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)cnt[d]));
+        CHECK(ofdm_memset_dev(ctx, cnt[d], 0, sizeof(ofdm_counters) * (size_t)(per * n_snr)));
+        CHECK(ofdm_counters_pack(ctx, (const ofdm_counters *)cnt[d], per * n_snr, (uint64_t *)ints[d], (double *)dbls[d]));
         CHECK(ofdm_ctx_sync(ctx));
     }
     /* ... and so does the first collective of a communicator (NCCL connects its peers lazily: ~0.1 s on 8 GPUs): one all-reduce
      * of the zeroed buffers before the clock starts */
     NCHECK(ncclGroupStart());
     for (int d = 0; d < n_gpus; ++d) {
-        NCHECK(ncclAllReduce(ints[d], ints[d], 5 * (size_t)n_snr, ncclUint64, ncclSum, comms[d], (cudaStream_t)ofdm_ctx_stream(ctxs[d])));
-        NCHECK(ncclAllReduce(dbls[d], dbls[d], 3 * (size_t)n_snr, ncclDouble, ncclSum, comms[d], (cudaStream_t)ofdm_ctx_stream(ctxs[d])));
+        NCHECK(ncclAllReduce(ints[d], ints[d], 5 * (size_t)(per * n_snr), ncclUint64, ncclSum, comms[d], (cudaStream_t)ofdm_ctx_stream(ctxs[d])));
+        NCHECK(ncclAllReduce(dbls[d], dbls[d], 3 * (size_t)(per * n_snr), ncclDouble, ncclSum, comms[d], (cudaStream_t)ofdm_ctx_stream(ctxs[d])));
     }
     NCHECK(ncclGroupEnd());
     for (int d = 0; d < n_gpus; ++d) { ctx = ctxs[d]; CHECK(ofdm_ctx_sync(ctx)); }
@@ -150,8 +167,9 @@ static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, co
          * slice of the round's frames; one all-reduce per buffer type per round; identical stop decisions everywhere */
         int active[64], n_active = n_snr, rounds = 0;
         unsigned long long done_frames = 0;
-        ofdm_counters part[64];
+        ofdm_counters part[128];
         memset(totals, 0, sizeof(ofdm_counters) * (size_t)n_snr);
+        if (code) memset(raw_totals, 0, sizeof(ofdm_counters) * (size_t)n_snr);
         for (int i = 0; i < n_snr; ++i) active[i] = i;
         const double t0 = now_s();
         while (n_active > 0) {
@@ -161,19 +179,19 @@ static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, co
                 long base = round_frames / n_gpus, rem = round_frames % n_gpus;
                 long lo = d * base + (d < rem ? d : rem), n = base + (d < rem ? 1 : 0);
                 ctx = ctxs[d];
-                CHECK(ofdm_memset_dev(ctx, cnt[d], 0, sizeof(ofdm_counters) * (size_t)n_active));
-                CHECK(ofdm_mc_sweep_channel_dev(ctx, ch, seed, (uint64_t)rounds * (uint64_t)round_frames + (uint64_t)lo, n, n_sym, snr_a, stream_a,
-                                                n_active, mode, (ofdm_counters *)cnt[d]));
-                if (!round_reduce_host) CHECK(ofdm_counters_pack(ctx, (const ofdm_counters *)cnt[d], n_active, (uint64_t *)ints[d], (double *)dbls[d]));
+                CHECK(ofdm_memset_dev(ctx, cnt[d], 0, sizeof(ofdm_counters) * (size_t)(per * n_active)));
+                CHECK(run_points(ctx, ch, code, seed, (uint64_t)rounds * (uint64_t)round_frames + (uint64_t)lo, n, n_sym, snr_a, stream_a, n_active,
+                                 mode, (ofdm_counters *)cnt[d]));
+                if (!round_reduce_host) CHECK(ofdm_counters_pack(ctx, (const ofdm_counters *)cnt[d], per * n_active, (uint64_t *)ints[d], (double *)dbls[d]));
             }
             if (round_reduce_host) {
                 /* one process drives every GPU: the round's partial counters (a few hundred bytes per GPU) can also be summed on the host */
-                static ofdm_counters per_gpu[8][64];
-                for (int d = 0; d < n_gpus; ++d) { ctx = ctxs[d]; CHECK(ofdm_memcpy_d2h(ctx, per_gpu[d], cnt[d], sizeof(ofdm_counters) * (size_t)n_active)); }
+                static ofdm_counters per_gpu[8][128];
+                for (int d = 0; d < n_gpus; ++d) { ctx = ctxs[d]; CHECK(ofdm_memcpy_d2h(ctx, per_gpu[d], cnt[d], sizeof(ofdm_counters) * (size_t)(per * n_active))); }
                 for (int d = 0; d < n_gpus; ++d) { ctx = ctxs[d]; CHECK(ofdm_ctx_sync(ctx)); }
                 memset(part, 0, sizeof part);
                 for (int d = 0; d < n_gpus; ++d)
-                    for (int j = 0; j < n_active; ++j) {
+                    for (int j = 0; j < per * n_active; ++j) {
                         part[j].bit_errors += per_gpu[d][j].bit_errors; part[j].bits += per_gpu[d][j].bits; part[j].frames_in_error += per_gpu[d][j].frames_in_error;
                         part[j].rail_errors += per_gpu[d][j].rail_errors; part[j].frames += per_gpu[d][j].frames;
                         part[j].sum_err2 += per_gpu[d][j].sum_err2; part[j].sum_ref2 += per_gpu[d][j].sum_ref2; part[j].sum_evm_lin += per_gpu[d][j].sum_evm_lin;
@@ -181,13 +199,13 @@ static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, co
             } else {
                 NCHECK(ncclGroupStart());
                 for (int d = 0; d < n_gpus; ++d) {
-                    NCHECK(ncclAllReduce(ints[d], ints[d], 5 * (size_t)n_active, ncclUint64, ncclSum, comms[d], (cudaStream_t)ofdm_ctx_stream(ctxs[d])));
-                    NCHECK(ncclAllReduce(dbls[d], dbls[d], 3 * (size_t)n_active, ncclDouble, ncclSum, comms[d], (cudaStream_t)ofdm_ctx_stream(ctxs[d])));
+                    NCHECK(ncclAllReduce(ints[d], ints[d], 5 * (size_t)(per * n_active), ncclUint64, ncclSum, comms[d], (cudaStream_t)ofdm_ctx_stream(ctxs[d])));
+                    NCHECK(ncclAllReduce(dbls[d], dbls[d], 3 * (size_t)(per * n_active), ncclDouble, ncclSum, comms[d], (cudaStream_t)ofdm_ctx_stream(ctxs[d])));
                 }
                 NCHECK(ncclGroupEnd());
                 ctx = ctxs[0];
-                CHECK(ofdm_counters_unpack(ctx, (ofdm_counters *)cnt[0], n_active, (const uint64_t *)ints[0], (const double *)dbls[0]));
-                CHECK(ofdm_memcpy_d2h(ctx, part, cnt[0], sizeof(ofdm_counters) * (size_t)n_active));
+                CHECK(ofdm_counters_unpack(ctx, (ofdm_counters *)cnt[0], per * n_active, (const uint64_t *)ints[0], (const double *)dbls[0]));
+                CHECK(ofdm_memcpy_d2h(ctx, part, cnt[0], sizeof(ofdm_counters) * (size_t)(per * n_active)));
                 for (int d = 0; d < n_gpus; ++d) { ctx = ctxs[d]; CHECK(ofdm_ctx_sync(ctx)); }
             }
             int keep = 0;
@@ -197,6 +215,13 @@ static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, co
                 t->rail_errors += part[j].rail_errors; t->frames += part[j].frames;
                 t->sum_err2 += part[j].sum_err2; t->sum_ref2 += part[j].sum_ref2; t->sum_evm_lin += part[j].sum_evm_lin;
                 done_frames += part[j].frames;
+                if (code) {
+                    ofdm_counters *r = &raw_totals[active[j]];
+                    const ofdm_counters *q = &part[n_active + j];
+                    r->bit_errors += q->bit_errors; r->bits += q->bits; r->frames_in_error += q->frames_in_error;
+                    r->rail_errors += q->rail_errors; r->frames += q->frames;
+                    r->sum_err2 += q->sum_err2; r->sum_ref2 += q->sum_ref2; r->sum_evm_lin += q->sum_evm_lin;
+                }
                 if (t->bit_errors < target_errors && t->bits < max_bits) active[keep++] = active[j];
             }
             n_active = keep;
@@ -217,23 +242,24 @@ static int sweep_multi_gpu(int n_gpus, unsigned seed, long frames, int n_sym, co
         long base = frames / n_gpus, rem = frames % n_gpus;
         long lo = d * base + (d < rem ? d : rem), n = base + (d < rem ? 1 : 0);
         ctx = ctxs[d];
-        CHECK(ofdm_mc_sweep_channel_dev(ctx, ch, seed, (uint64_t)lo, n, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)cnt[d]));
-        CHECK(ofdm_counters_pack(ctx, (const ofdm_counters *)cnt[d], n_snr, (uint64_t *)ints[d], (double *)dbls[d]));
+        CHECK(run_points(ctx, ch, code, seed, (uint64_t)lo, n, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)cnt[d]));
+        CHECK(ofdm_counters_pack(ctx, (const ofdm_counters *)cnt[d], per * n_snr, (uint64_t *)ints[d], (double *)dbls[d]));
     }
     NCHECK(ncclGroupStart());
     for (int d = 0; d < n_gpus; ++d) {
-        NCHECK(ncclAllReduce(ints[d], ints[d], 5 * (size_t)n_snr, ncclUint64, ncclSum, comms[d], (cudaStream_t)ofdm_ctx_stream(ctxs[d])));
-        NCHECK(ncclAllReduce(dbls[d], dbls[d], 3 * (size_t)n_snr, ncclDouble, ncclSum, comms[d], (cudaStream_t)ofdm_ctx_stream(ctxs[d])));
+        NCHECK(ncclAllReduce(ints[d], ints[d], 5 * (size_t)(per * n_snr), ncclUint64, ncclSum, comms[d], (cudaStream_t)ofdm_ctx_stream(ctxs[d])));
+        NCHECK(ncclAllReduce(dbls[d], dbls[d], 3 * (size_t)(per * n_snr), ncclDouble, ncclSum, comms[d], (cudaStream_t)ofdm_ctx_stream(ctxs[d])));
     }
     NCHECK(ncclGroupEnd());
     for (int d = 0; d < n_gpus; ++d) {
         ctx = ctxs[d];
-        CHECK(ofdm_counters_unpack(ctx, (ofdm_counters *)cnt[d], n_snr, (const uint64_t *)ints[d], (const double *)dbls[d]));
+        CHECK(ofdm_counters_unpack(ctx, (ofdm_counters *)cnt[d], per * n_snr, (const uint64_t *)ints[d], (const double *)dbls[d]));
     }
     ctx = ctxs[0];
     CHECK(ofdm_memcpy_d2h(ctx, totals, cnt[0], sizeof(ofdm_counters) * (size_t)n_snr));
+    if (code) CHECK(ofdm_memcpy_d2h(ctx, raw_totals, (ofdm_counters *)cnt[0] + n_snr, sizeof(ofdm_counters) * (size_t)n_snr));
     for (int d = 0; d < n_gpus; ++d) { ctx = ctxs[d]; CHECK(ofdm_ctx_sync(ctx)); }
-    report_rate(n_taps > 0 ? "multipath sweep" : "sweep", n_gpus, frames, n_sym, n_snr, now_s() - t0);
+    report_rate(code ? "coded sweep" : n_taps > 0 ? "multipath sweep" : "sweep", n_gpus, frames, n_sym, n_snr, now_s() - t0);
     for (int d = 0; d < n_gpus; ++d) {
         ncclCommDestroy(comms[d]);
         ofdm_dev_free(ctxs[d], cnt[d]); ofdm_dev_free(ctxs[d], ints[d]); ofdm_dev_free(ctxs[d], dbls[d]);
@@ -256,6 +282,9 @@ int main(int argc, char **argv)
     const char *draws_file = NULL, *bits_file = NULL;
     ofdm_channel ch = {OFDM_NOISE_REAL_RAIL, OFDM_SNR_FRAME_POWER, 0};
     int channel_set = 0;                 /* --noise / --snr-def given */
+    ofdm_code code_v = {0, OFDM_DECISION_SOFT};
+    const ofdm_code *code = NULL;        /* --code given */
+    int decision_set = 0;
     int round_reduce_host = 1;           /* until rule: per-round totals summed on the host (measured 8 GPUs, 13 rounds: 0.033 s against 0.294 s with two
                                             single-process NCCL group all-reduces per round, profiles/r2_c_driver_until_8gpu.txt) */
     for (int i = 1; i < argc; ++i) {
@@ -295,6 +324,16 @@ int main(int argc, char **argv)
             else if (!strcmp(v, "ebn0")) ch.snr_def = OFDM_SNR_EBN0;
             else { fprintf(stderr, "--snr-def must be frame_power, esn0 or ebn0\n"); return 2; }
             channel_set = 1;
+        } else if (!strcmp(a, "--code")) {
+            if (!strcmp(v, "1/2")) code_v.rate = OFDM_CODE_R12;
+            else if (!strcmp(v, "3/4")) code_v.rate = OFDM_CODE_R34;
+            else { fprintf(stderr, "--code must be 1/2 or 3/4\n"); return 2; }
+            code = &code_v;
+        } else if (!strcmp(a, "--decision")) {
+            if (!strcmp(v, "soft")) code_v.decision = OFDM_DECISION_SOFT;
+            else if (!strcmp(v, "hard")) code_v.decision = OFDM_DECISION_HARD;
+            else { fprintf(stderr, "--decision must be soft or hard\n"); return 2; }
+            decision_set = 1;
         }
         else { fprintf(stderr, "unknown option %s\n", a); return 2; }
         ++i;
@@ -307,18 +346,24 @@ int main(int argc, char **argv)
                         "--message and --draws run the reference's channel\n");
         return 2;
     }
+    if (decision_set && !code) { fprintf(stderr, "--decision needs --code\n"); return 2; }
+    if (code && (draws_file || (frames < 2 && target_errors == 0))) {
+        fprintf(stderr, "--code runs the coded link in the Monte-Carlo sweeps (--frames N > 1 or --target-errors E); not with --message or --draws\n");
+        return 2;
+    }
     ch.n_taps = n_taps;
     const int reference_channel = ch.noise == OFDM_NOISE_REAL_RAIL && ch.snr_def == OFDM_SNR_FRAME_POWER;
 
     ofdm_ctx *ctx = NULL;
-    float SNR[64], EVM_dB[64], EVM_AGC_dB[64], BER[64];
+    float SNR[64], EVM_dB[64], EVM_AGC_dB[64], BER[64], PER[64];
     for (int i = 0; i < n_snr; ++i) SNR[i] = snr_start + snr_step * (float)i;
-    ofdm_counters totals[64];
+    ofdm_counters totals[64], raw_totals[64];     /* with a code: totals = decoded (coded) counters, raw_totals = the receiver's */
 
     if (n_gpus > 1) {
 #ifdef OFDM_WITH_NCCL
         if (frames < 2 && target_errors == 0) { fprintf(stderr, "--gpus needs --frames N > 1 or --target-errors E\n"); return 2; }
-        int rc = sweep_multi_gpu(n_gpus, seed, frames, n_sym, &ch, SNR, n_snr, mode, totals, target_errors, max_bits, round_frames, round_reduce_host);
+        int rc = sweep_multi_gpu(n_gpus, seed, frames, n_sym, &ch, code, SNR, n_snr, mode, totals, raw_totals, target_errors, max_bits, round_frames,
+                                 round_reduce_host);
         if (rc) return rc;
 #else
         fprintf(stderr, "built without NCCL (make ofdm_sweep NCCL=1)\n");
@@ -363,7 +408,11 @@ int main(int argc, char **argv)
     } else if (target_errors > 0) {                    /* configs[3]: until >= E errors or the bit budget, one GPU */
         int rounds = 0;
         const double t0 = now_s();
-        CHECK(ofdm_mc_sweep_channel_until(ctx, &ch, seed, 0, n_sym, SNR, n_snr, mode, target_errors, max_bits, round_frames, totals, &rounds));
+        if (code)
+            CHECK(ofdm_mc_sweep_coded_until(ctx, &ch, code, seed, 0, n_sym, SNR, n_snr, mode, target_errors, max_bits, round_frames, totals, raw_totals,
+                                            &rounds));
+        else
+            CHECK(ofdm_mc_sweep_channel_until(ctx, &ch, seed, 0, n_sym, SNR, n_snr, mode, target_errors, max_bits, round_frames, totals, &rounds));
         unsigned long long fp = 0;
         for (int i = 0; i < n_snr; ++i) fp += totals[i].frames;
         const double dt = now_s() - t0;
@@ -371,13 +420,16 @@ int main(int argc, char **argv)
                 fp, n_sym, dt, (double)fp * n_sym / dt);
     } else if (frames > 1) {                           /* Monte-Carlo sweep through the channel; --taps: configs[4]'s multipath taps */
         void *d_cnt = NULL;
-        CHECK(ofdm_dev_alloc(ctx, &d_cnt, sizeof(ofdm_counters) * (size_t)n_snr));
-        CHECK(ofdm_memset_dev(ctx, d_cnt, 0, sizeof(ofdm_counters) * (size_t)n_snr));
+        const size_t n_cnt = (size_t)n_snr * (code ? 2 : 1);
+        CHECK(ofdm_dev_alloc(ctx, &d_cnt, sizeof(ofdm_counters) * n_cnt));
+        CHECK(ofdm_memset_dev(ctx, d_cnt, 0, sizeof(ofdm_counters) * n_cnt));
         const double t0 = now_s();
-        CHECK(ofdm_mc_sweep_channel_dev(ctx, &ch, seed, 0, frames, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)d_cnt));
+        CHECK(run_points(ctx, &ch, code, seed, 0, frames, n_sym, SNR, NULL, n_snr, mode, (ofdm_counters *)d_cnt));
         CHECK(ofdm_memcpy_d2h(ctx, totals, d_cnt, sizeof(ofdm_counters) * (size_t)n_snr));
+        if (code) CHECK(ofdm_memcpy_d2h(ctx, raw_totals, (ofdm_counters *)d_cnt + n_snr, sizeof(ofdm_counters) * (size_t)n_snr));
         CHECK(ofdm_ctx_sync(ctx));
-        report_rate(!reference_channel ? "channel sweep" : n_taps > 0 ? "multipath sweep" : "sweep", 1, frames, n_sym, n_snr, now_s() - t0);
+        report_rate(code ? "coded sweep" : !reference_channel ? "channel sweep" : n_taps > 0 ? "multipath sweep" : "sweep", 1, frames, n_sym, n_snr,
+                    now_s() - t0);
         ofdm_dev_free(ctx, d_cnt);
     } else {
         uint8_t *bits = NULL;
@@ -458,10 +510,17 @@ int main(int argc, char **argv)
         free(bits); free(words); free(rx_words); free(text);
     }
 
+    if (code)
+        fprintf(stderr, "code %s %s: Output_BER.txt = decoded information-bit BER, Output_PER.txt = packet error rate, EVM from the receiver\n",
+                code->rate == OFDM_CODE_R12 ? "1/2" : "3/4", code->decision == OFDM_DECISION_HARD ? "hard" : "soft");
     for (int i = 0; i < n_snr; ++i) {
         float Res[3];                                      /* EVM_dB, EVM_AGC_DB, BER  :1210 */
-        CHECK(ofdm_counters_finalize(&totals[i], Res));
+        CHECK(ofdm_counters_finalize(code ? &raw_totals[i] : &totals[i], Res));
         EVM_dB[i] = Res[0]; EVM_AGC_dB[i] = Res[1]; BER[i] = Res[2];
+        if (code) {
+            BER[i] = totals[i].bits ? (float)((double)totals[i].bit_errors / (double)totals[i].bits) : 0.f;
+            PER[i] = totals[i].frames ? (float)((double)totals[i].frames_in_error / (double)totals[i].frames) : 0.f;
+        }
         if (!quiet) printf("\nSNR %5.1f dB  EVM dB = %lf  EVM_AGC dB = %lf  BER = %le  (%llu frames)", SNR[i], Res[0], Res[1], Res[2],
                            (unsigned long long)totals[i].frames);
     }
@@ -470,6 +529,7 @@ int main(int argc, char **argv)
     snprintf(path, sizeof path, "%s/Output_EVM_AGC.txt", outdir);     CHECK(ofdm_write_float_array_to_file(EVM_dB, n_snr, path));
     snprintf(path, sizeof path, "%s/Output_EVM_AGC_DB.txt", outdir);  CHECK(ofdm_write_float_array_to_file(EVM_AGC_dB, n_snr, path));
     snprintf(path, sizeof path, "%s/Output_BER.txt", outdir);         CHECK(ofdm_write_float_array_to_file(BER, n_snr, path));
+    if (code) { snprintf(path, sizeof path, "%s/Output_PER.txt", outdir); CHECK(ofdm_write_float_array_to_file(PER, n_snr, path)); }
     if (!quiet) printf("\nCode Run Successful!\n");
     if (ctx) ofdm_ctx_destroy(ctx);
     return 0;

@@ -103,11 +103,12 @@ def until_loop(run_round, n_points, target_errors, max_bits, round_frames, rank=
 
 
 def mc_sweep_until(ofdm, seed, n_sym, snr_db, mode, target_errors=100, max_bits=10 ** 9, round_frames=1 << 22, n_taps=0, rank=0, world=1,
-                   group=None, frame0=0, noise="real", snr_def="frame_power"):
+                   group=None, frame0=0, noise="real", snr_def="frame_power", code=None, decision="soft"):
     """configs[3] as stated, on ``world`` GPUs: SNR points x frame ranges are sharded by rounds (every rank works on every
     still-active point, on its own slice of the round's frames -- so the slow high-SNR points use all GPUs), one all-reduce
-    of the counters per round.  ``noise`` / ``snr_def`` choose the channel (binding.channel; the default is the reference's).
-    Returns (list of global Counters, rounds) on every rank."""
+    of the counters per round.  ``noise`` / ``snr_def`` choose the channel (binding.channel; the default is the reference's);
+    ``code`` ("1/2" | "3/4", None = uncoded) runs the coded link with ``decision`` ("soft" | "hard") and stops on its
+    information-bit errors.  Returns (list of global Counters -- the coded ones with a code, rounds) on every rank."""
     import torch
     import torch.distributed as dist
     snr = np.asarray(snr_db, dtype=np.float32)
@@ -116,7 +117,10 @@ def mc_sweep_until(ofdm, seed, n_sym, snr_db, mode, target_errors=100, max_bits=
     def run_round(points, lo, n):
         c = cnt[:len(points)]
         c.zero_()
-        if n > 0:
+        if n > 0 and code is not None:
+            ofdm.mc_sweep_coded(seed, lo, n, n_sym, snr[points], mode, code, decision, noise, snr_def, n_taps, np.asarray(points, dtype=np.uint32),
+                                (c, None))
+        elif n > 0:
             ofdm.mc_sweep_channel(seed, lo, n, n_sym, snr[points], mode, noise, snr_def, n_taps, np.asarray(points, dtype=np.uint32), c)
         if world > 1:
             allreduce_counter_tensor(c, group)              # on the device: NCCL over NVLink

@@ -270,6 +270,37 @@ int ofdm_mc_sweep_channel_until(ofdm_ctx *ctx, const ofdm_channel *ch, uint32_t 
                                 int n_snr, int mode, uint64_t target_errors, uint64_t max_bits, long round_frames,
                                 ofdm_counters *out_host, int *rounds_out);
 
+/* ---- the coded link: the 802.11a convolutional code (IEEE 802.11a section 17.3.5.6; definitions in DESIGN.md section 6.2) ----
+ * K = 7, g0 = 133 (octal, output A), g1 = 171 (output B), rate 1/2 (48 data bits per OFDM symbol) or 3/4 (72: A0 B0 A1 B2 of every
+ * three input bits), per-symbol interleaver i = 6 (k mod 16) + floor(k / 16), and a precoding onto this project's QPSK map that sends
+ * coded bit c0 on the I rail and c1 on the Q rail as the 802.11a constellation (2c - 1)/sqrt(2).  A frame of n_sym symbols carries
+ * K_info = n_sym N_DBPS - 6 information bits -- bits 0 .. K_info-1 of its packed words -- and 6 zero tail bits.
+ * ofdm_conv_encode     information words [n_frames][n_sym*3] -> payload words [n_frames][n_sym*3] for ofdm_tx_frames.
+ * ofdm_viterbi_decode  maximum-likelihood decoding of whole frames from the receiver's H [n_frames][64][2] and eq
+ *                      [n_frames][n_sym*48][2] dumps: soft (L = |H|^2 eq per rail) or hard (L = +-1 by the slicer's rule) decisions.
+ *                      decoded_dev [n_frames][n_sym*3] (nullable) receives the decoded information bits (tail and pad bits 0);
+ *                      counters_dev (nullable; needs info_dev) accumulates the coded counters.
+ * Coded counters: bit_errors = information-bit errors, bits = K_info x frames, frames_in_error = packets with >= 1 such error
+ * (PER = frames_in_error / frames), rail_errors and the three sums 0.  Raw counters: the receiver's own against the payload words
+ * (rail_errors = coded-bit errors; the EVM sums keep their meaning).
+ * ofdm_mc_sweep_coded_dev / _until: ofdm_mc_sweep_channel_dev / _until with the code between the Philox bits and the transmitter
+ * and the decoder behind the receiver, always staged through HBM; an Eb/N0 point counts information bits (Es/N0 = Eb/N0 x 2R).
+ * raw (nullable) receives the raw counters; the until rule stops on the coded ones.  A NULL or invalid code or channel returns
+ * OFDM_ERR_INVALID. */
+enum { OFDM_CODE_R12 = 1, OFDM_CODE_R34 = 2 };
+enum { OFDM_DECISION_SOFT = 0, OFDM_DECISION_HARD = 1 };
+typedef struct { int rate, decision; } ofdm_code;
+int ofdm_conv_encode(ofdm_ctx *ctx, int rate, const uint32_t *info_dev, uint32_t *payload_dev, long n_frames, int n_sym);
+int ofdm_viterbi_decode(ofdm_ctx *ctx, const ofdm_code *code, const float *H_dev, const float *eq_dev,
+                        const uint32_t *info_dev /* nullable: count against it */, uint32_t *decoded_dev /* nullable */,
+                        long n_frames, int n_sym, ofdm_counters *counters_dev /* nullable */);
+int ofdm_mc_sweep_coded_dev(ofdm_ctx *ctx, const ofdm_channel *ch, const ofdm_code *code, uint32_t seed, uint64_t frame0,
+                            long n_frames, int n_sym, const float *snr_db, const uint32_t *streams, int n_points, int mode,
+                            ofdm_counters *coded_dev, ofdm_counters *raw_dev /* nullable */);
+int ofdm_mc_sweep_coded_until(ofdm_ctx *ctx, const ofdm_channel *ch, const ofdm_code *code, uint32_t seed, uint64_t frame0,
+                              int n_sym, const float *snr_db, int n_snr, int mode, uint64_t target_errors, uint64_t max_bits,
+                              long round_frames, ofdm_counters *coded_host, ofdm_counters *raw_host /* nullable */, int *rounds_out);
+
 /* ---- multipath extension (BASELINE configs[4]; the reference's only channel is AWGN, OFDM.c:635-655) ----
  * y[n] = sum_l h[l] x[n-l] per frame, n_taps <= 16 (= CP length), applied between the transmitter and
  * Transmission_Over_Air; the reference's own LTS estimate + one-tap equaliser (OFDM.c:830-850, 1046-1052) undo it.
